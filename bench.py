@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload encoder|model] [--mode ssl_encoder|ssl_all|downstream] [--patch 96|128] [--batch B]
-                    [--dtype bf16|fp32] [--dropout 0.1] [--checkpoint] [--frozen]
+                    [--dtype bf16|fp32] [--dropout 0.1] [--checkpoint] [--frozen] [--dump-outputs DIR]
 
 One "step" = forward + backward of the hot path over one batch of synthetic input.
   --workload encoder (default, BASELINE config[1]): the Swin encoder of SwinUNETR(feature_size=48) on 96^3 patches with
@@ -16,6 +16,9 @@ One "step" = forward + backward of the hot path over one batch of synthetic inpu
       12 prompted blocks), downstream (config[3]: frozen backbone, prompt-token-only gradients); --patch 128 = config[4].
 Metric: 3D patches / s, whole job.  Prints ONE JSON line (rank 0).  Under torchrun (N > 1) every rank processes its own
 batch shard (weak scaling: fixed per-GPU batch); gradients are all-reduced over NCCL once per step.
+--dump-outputs DIR: after the HBM-resident timed steps, rank 0 writes what the last of them returned to its caller (loss,
+every trainable parameter's gradient, the input's gradient where the input takes one) as DIR/<name>.npy, 64 MB at most.
+Weights, inputs and dropout seeds are seeded, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -27,6 +30,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -154,7 +158,9 @@ class EncoderWorkload:
             keep = {id(p) for st in self.model for _, p in st.named_parameters_bias_prompt_tokens()}
             for p in self.model.parameters():
                 p.requires_grad_(id(p) in keep)
-        self.params = [p for p in list(self.model.parameters()) + list(self.prompts.parameters()) if p.requires_grad]
+        named = list(self.model.named_parameters()) + [("prompts." + n, p) for n, p in self.prompts.named_parameters()]
+        self.named_params = [(n, p) for n, p in named if p.requires_grad]
+        self.params = [p for _, p in self.named_params]
         c0, _, d0 = self.specs[0]
         self.in_shape = (args.batch, c0, *d0)
         self.n_blocks = 6
@@ -190,7 +196,8 @@ class ModelWorkload:
         conf = pwa_b200.SwinUnetRConfig(training_mode=mode, use_encoder_prompting=enc_p, use_decoder_prompting=dec_p,
                                         use_checkpoint=use_checkpoint, attn_drop=args.dropout, proj_drop=args.dropout)
         self.model = pwa_b200.SwinUnetR(conf).to(dev).train()
-        self.params = [p for p in self.model.parameters() if p.requires_grad]
+        self.named_params = [(n, p) for n, p in self.model.named_parameters() if p.requires_grad]
+        self.params = [p for _, p in self.named_params]
         self.in_shape = (args.batch, 1, args.patch, args.patch, args.patch)
         self.autocast = args.dtype == "bf16"
         self.desc = (f"SwinUnetR(feature_size=48) {mode}, {args.patch}^3 single-channel patches, encoder"
@@ -315,6 +322,27 @@ def kernel_microbench(args, dev, dtype):
     return out, attn_launches
 
 
+DUMP_BYTES = 60 << 20                       # array data; the .npy headers fit in the rest of the 64 MB
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BYTES):
+    """Writes {name: tensor} as out_dir/<name>.npy in float32 (float64 stays float64).  Taken smallest first, an array is
+    written whole when it fits an even share of the budget still left; a larger one becomes a 1-D sample of that many
+    elements at sorted random flat indices from a fixed seed, so every run with the same shapes stores the same elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    left = budget
+    for i, (name, t) in enumerate(items):
+        t = t.detach().cpu()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        share = left // (len(items) - i) // t.element_size()
+        if t.numel() > share:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
+        left -= t.numel() * t.element_size()
+
+
 def run_ours(args):
     import torch.distributed as dist
     import pwa_b200
@@ -362,20 +390,25 @@ def run_ours(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}                                         # what the latest step handed back: its loss and input gradient
+
     def run_step(w, gr, x_src):
         if gr is not None:
             loss = gr(x_src)                          # copy into the static input (H2D or D2D) + one graph launch
             if world > 1:
                 gr.allreduce_flat()                   # ONE in-place NCCL all-reduce of the flat gradient buffer
+            last.update(loss=loss, input_grad=gr.input_grads[0])
         else:
             for p in w.params:
                 p.grad = None
-            loss = w.step(x_src.to(dev, non_blocking=True).clone().requires_grad_(args.workload == "encoder"))
+            x = x_src.to(dev, non_blocking=True).clone().requires_grad_(args.workload == "encoder")
+            loss = w.step(x)
             if world > 1:
                 grads = [p.grad for p in w.params if p.grad is not None]
                 flat = torch.cat([g.reshape(-1) for g in grads])
                 dist.all_reduce(flat)
                 flat.div_(world)
+            last.update(loss=loss, input_grad=x.grad)
         return loss
 
     def timed(w, gr, steps, warmup, count=False):
@@ -409,6 +442,13 @@ def run_ours(args):
         ms = timed(wl, graphed, args.steps, args.warmup, count=True)
     launches = KernelStats.launches
     KernelStats.reset(enabled=False)
+    if args.dump_outputs and rank == 0:
+        outs = {"loss": last["loss"]}
+        if last["input_grad"] is not None:
+            outs["input_grad"] = last["input_grad"]
+        for n, p in wl.named_params:                 # (a parameter the step never reaches has no gradient: zeros)
+            outs["grad." + n] = p.grad if p.grad is not None else torch.zeros_like(p)
+        dump_outputs(args.dump_outputs, outs)
 
     # ---- timed region 2: end to end through the public module API with host buffers ----
     feeder = InputPrefetcher(xdev[0], dev)
@@ -599,7 +639,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
-    steps, warmup = max(1, min(args.steps, 8)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, max(1, min(args.warmup, 1))
     cpu = cpu_baseline_sample(args, steps=steps, warmup=warmup, batch=1)
     line = {
         "impl": "reference", "metric": METRIC, "value": cpu["value"], "unit": UNIT, "n_gpus": args.gpus,
@@ -660,9 +700,15 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying a CUDA graph")
     ap.add_argument("--cuda-profiler-range", action="store_true",
                     help="bracket the HBM-resident timed region with cudaProfilerStart/Stop (for ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of the last HBM-resident timed step as DIR/<name>.npy (64 MB at most)")
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 5 if args.impl == "reference" else 20
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what --impl ours computes")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)

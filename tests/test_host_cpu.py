@@ -132,6 +132,41 @@ def test_bench_reference_arm_prints_the_contract_line():
         assert key in line, key
     assert line["cpu_baseline"]["kind"] == "port" and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["e2e"]["d2h_bytes_per_step"] == 0
+    assert line["steps"] == 1
+
+
+def test_bench_rejects_zero_steps():
+    import subprocess
+    import sys
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"],
+                         capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 2 and "--steps must be at least 1" in out.stderr
+    assert out.stdout == ""
+
+
+def test_bench_dump_outputs_budget_and_sample(tmp_path):
+    """bench.dump_outputs: arrays that fit an even share of the byte budget are written whole as float32 (float64 stays
+    float64), a larger one as the same sorted, seeded sample on every call, and the data stays within the budget."""
+    import bench
+    g = torch.Generator().manual_seed(3)
+    arrays = {"loss": torch.tensor(2.5), "small": torch.arange(10, dtype=torch.bfloat16),
+              "mid": torch.randn(2, 500, generator=g), "big": torch.randn(50, 100, generator=g, dtype=torch.float64)}
+    budget = 12000
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, budget=budget)
+    got = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in arrays}
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(f"{k}.npy" for k in arrays)
+    assert got["loss"].dtype == np.float32 and got["loss"].shape == () and got["loss"] == 2.5
+    assert got["small"].dtype == np.float32 and np.array_equal(got["small"], np.arange(10, dtype=np.float32))
+    assert got["mid"].dtype == np.float32 and np.array_equal(got["mid"], arrays["mid"].numpy())
+    big, full = got["big"], arrays["big"].numpy().reshape(-1)
+    assert big.dtype == np.float64 and big.ndim == 1 and 0 < big.size < full.size
+    pos = {v: i for i, v in enumerate(full)}
+    idx = np.array([pos[v] for v in big])
+    assert np.all(np.diff(idx) > 0)                                   # distinct elements, in flat order
+    assert sum(v.nbytes for v in got.values()) <= budget
+    for k in arrays:
+        assert np.array_equal(np.load(tmp_path / "b" / f"{k}.npy"), got[k])
 
 
 def test_token_split_picks_a_divisor_near_72():
