@@ -21,6 +21,8 @@
  *     libraries built with `make TIMELINE=1`.
  *   - re-entrant and thread-safe (no global mutable state besides one-time kernel attribute setup).
  *   - there is NO CPU fallback: device entry points fail with PWA_ERR_CUDA when no GPU is present.
+ *   - `dtype` is PWA_F32, PWA_BF16 or PWA_F16 wherever an entry point takes one; the two 16-bit types take the same paths
+ *     (tcgen05 kernels where the shape allows, the same envelope for both), fp32 runs on the CUDA-core kernels.
  */
 #ifndef PWA_H_
 #define PWA_H_
@@ -35,7 +37,9 @@ extern "C" {
 #define PWA_VERSION 100
 
 enum { PWA_OK = 0, PWA_ERR_ARG = -1, PWA_ERR_UNSUPPORTED = -2, PWA_ERR_CUDA = -3 };
-enum { PWA_F32 = 0, PWA_BF16 = 1 };
+/* Element type of the token tensors of an entry point's `dtype` argument.  Every kernel computes in fp32 (or accumulates in
+ * fp32 on the tensor cores) whatever the storage type; PWA_F16 is IEEE binary16 (torch.float16, torch.autocast's default). */
+enum { PWA_F32 = 0, PWA_BF16 = 1, PWA_F16 = 2 };
 
 /* Window geometry of one block call.  Filled by pwa_geometry(); plain ints so that it can be
  * mirrored by a ctypes.Structure. */
@@ -114,16 +118,17 @@ int pwa_gather_rows(const void* src_a, const void* src_b, void* dst, const int32
  * torch autograd in the reference): dW = dy^T x is computed as S batched slices of the token axis with fp32 partials. */
 int pwa_colsum_f32(const float* src, float* dst, int S, int64_t n, void* stream);
 
-/* dst[c] = sum over r < rows of x[r][c]: x [rows][C] bf16 or fp32 (dtype = PWA_BF16 / PWA_F32), dst [C] fp32, both on the
+/* dst[c] = sum over r < rows of x[r][c]: x [rows][C] bf16, fp16 or fp32 (dtype), dst [C] fp32, both on the
  * DEVICE; dst is zeroed by the call.  The bias gradient of the q|k|v projection (window_attention.py:28-30: nn.Linear with
  * bias; torch autograd sums the packed dq|dk|dv rows over all tokens there).  C must be a multiple of the elements per
- * 16 bytes (8 / 4) and at most 512 such vectors; x 16-byte aligned.  fp32 atomics: the sum order is not fixed. */
+ * 16 bytes (8 for bf16 / fp16, 4 for fp32) and at most 512 such vectors; x 16-byte aligned.  fp32 atomics: the sum order is not fixed. */
 int pwa_colsum_rows(const void* x, float* dst, int64_t rows, int C, int dtype, void* stream);
 
 /* y[i] = keep(i) ? x[i] / keep_rate : 0 for i < n, keep(i) a counter-based hash of the two uint32 words at seed_dev (DEVICE
  * memory) and i; rate in steps of 1/256.  Replaces nn.Dropout(proj_drop) after the attention output projection
  * (window_attention.py:33,60).  The same call on dy is the backward.  No generator state is involved, so an activation-
  * checkpointed block recomputes the same mask and a captured CUDA graph gets fresh masks whenever the seed words change.
+ * The mask depends only on the seed words and i, not on dtype (fp32, bf16 or fp16 with fp32 math).
  * x == y is allowed; both 16-byte aligned. */
 int pwa_dropout(const void* x, void* y, int64_t n, float p_drop, const void* seed_dev, int dtype, void* stream);
 
@@ -165,7 +170,11 @@ typedef struct pwa_attn_shape {
  * shift mask).  out [B][P][N][C]; lse fp32 [B][P][h][N] (natural-log sum-exp of the masked logits).
  * logits = (q.k^T*scale + bias) * mask ; softmax ; dropout ; @ v   (window_attention.py:49-58),
  * queries = the N content tokens only (prompt rows are cut by swin_block.py:222-225).
- * impl: 0 = auto, 1 = fp32 CUDA-core kernel, 2 = bf16 tcgen05/TMEM kernel. */
+ * dtype PWA_F32 / PWA_BF16 / PWA_F16 for q, k, v, kp, vp, out.
+ * impl: 0 = auto, 1 = fp32-math CUDA-core kernel (any dtype), 2 = tcgen05/TMEM kernel (bf16 or fp16; fp32 accumulation).
+ * The fp16 tcgen05 forward keeps each row's largest probability a normal fp16 number (DESIGN.md §4(b)): it scales the
+ * probabilities by 2^10 before rounding them and takes the exact-row-maximum sweep when the norm bound is loose by more
+ * than 24 binades (bf16: 80). */
 int pwa_attn_fwd(const void* q, const void* k, const void* v, const void* kp, const void* vp,
                  const float* th, const float* tw, const float* td, const float* tok,
                  const uint8_t* ids, void* out, float* lse, const pwa_attn_shape* s, int dtype,
@@ -173,7 +182,8 @@ int pwa_attn_fwd(const void* q, const void* k, const void* v, const void* kp, co
 
 /* ---- (c) backward ----------------------------------------------------------------------------- */
 
-/* Inputs as pwa_attn_fwd plus out, lse, dout [B][P][N][C].  Outputs: dq,dk,dv [B][P][N][C] (dtype);
+/* Inputs as pwa_attn_fwd plus out, lse, dout [B][P][N][C].  Outputs: dq,dk,dv [B][P][N][C] (dtype: fp32, bf16 or fp16;
+ * in fp16 a gradient that overflows becomes inf, and a non-finite dout stays non-finite in every gradient it reaches);
  * dkp,dvp fp32 [B][I][C], summed over the P windows of each sample; dth,dtw,dtd,dtok fp32, summed
  * over batch and windows.  The fp32 accumulators are zeroed by this call (cudaMemsetAsync on
  * `stream`).  delta fp32 [B][P][h][N] is caller-provided scratch. */
@@ -225,7 +235,7 @@ int pwa_ln_bwd2(const void* dy, const void* x, const float* gamma, const float* 
                 const void* dres, void* dx, float* dgamma, float* dbeta, float* dres_colsum, float* dx_colsum,
                 int64_t rows, int C, int dtype, void* stream);
 
-/* ---- token-domain GEMM with fused LayerNorm / residual / dropout prologue (tcgen05, bf16) ------------------------------- */
+/* ---- token-domain GEMM with fused LayerNorm / residual / dropout prologue (tcgen05, bf16 or fp16) ---------------------- */
 
 /* s = dropout(x) (+ res) ; z = LayerNorm(s) * gamma + beta (gamma == NULL: z = s) ; y = z @ W^T (+ bias).
  * x, res, sum_out, ln_out [T][C] bf16; W [Cout][C] bf16 row-major; bias [Cout] bf16 or NULL; y [T][Cout] bf16; mean, rstd fp32
@@ -234,13 +244,19 @@ int pwa_ln_bwd2(const void* dy, const void* x, const float* gamma, const float* 
  * One pass over the tokens for what the reference runs as LayerNorm + Linear (+ Dropout + add) modules: swin_block.py:216 +
  * window_attention.py:42-44 (attn_norm + to_q|to_k|to_v as one [C -> 3C] projection), window_attention.py:60 +
  * swin_block.py:222-227 (proj_drop, residual add, mlp_norm, the single-Linear MLP).  C % 16 == 0, 16 <= C <= 192,
- * Cout % 16 == 0 (pwa_token_gemm_supported). */
+ * Cout % 16 == 0 (pwa_token_gemm_supported).
+ * pwa_token_gemm_fwd_dt takes the element type of x, res, sum_out, ln_out, W, bias and y: PWA_BF16 or PWA_F16 (fp32 LayerNorm
+ * math and fp32 accumulation either way); pwa_token_gemm_fwd is its PWA_BF16 call. */
 int pwa_token_gemm_supported(int C, int Cout);
 int pwa_token_gemm_fwd(const void* x, const void* res, const float* gamma, const float* beta, const void* W, const void* bias,
                        void* sum_out, void* ln_out, void* y, float* mean, float* rstd, int64_t T, int C, int Cout, float eps,
                        float p_drop, const void* seed_dev, void* stream);
+int pwa_token_gemm_fwd_dt(const void* x, const void* res, const float* gamma, const float* beta, const void* W, const void* bias,
+                          void* sum_out, void* ln_out, void* y, float* mean, float* rstd, int64_t T, int C, int Cout, float eps,
+                          float p_drop, const void* seed_dev, int dtype, void* stream);
 
-/* 1 iff the bf16 tcgen05 kernel supports this shape (else impl=0 falls back to the fp32-math kernel). */
+/* 1 iff the tcgen05 kernels (forward and backward) support this shape and dtype (PWA_BF16 or PWA_F16: the same shapes for
+ * both; else impl=0 runs the fp32-math kernel). */
 int pwa_attn_tc_supported(const pwa_attn_shape* s, int dtype);
 
 /* Window attention with DENSE position-bias / mask tensors: the literal argument form of the reference's
@@ -252,7 +268,7 @@ int pwa_attn_tc_supported(const pwa_attn_shape* s, int dtype);
  * element (b,p,h,i,j) at b*stride[0] + p*stride[1] + h*stride[2] + i*stride[3] + j (j contiguous; stride 0 = broadcast).
  * dbias (or NULL): fp32 buffer with bias's strides, ZEROED by the caller; the gradient is accumulated with atomics.
  * p_drop in steps of 1/256 with the generator of pwa_attn_fwd (nq rows per window-head); seed_dev = two uint32 words on
- * the device.  fp32 arithmetic, fp32 / bf16 I/O; head dims 3, 6, 8, 12, 16, 24, 32, 48. */
+ * the device.  fp32 arithmetic, fp32 / bf16 / fp16 I/O; head dims 3, 6, 8, 12, 16, 24, 32, 48. */
 typedef struct pwa_dense_attn {
   int32_t B, P, heads, dh, nq, nk;
   int32_t ld_q, ld_k, ld_v;

@@ -11,7 +11,7 @@ import os
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libpwa_b200.so")
 
-PWA_F32, PWA_BF16 = 0, 1
+PWA_F32, PWA_BF16, PWA_F16 = 0, 1, 2
 
 
 class PwaGeom(C.Structure):
@@ -78,6 +78,8 @@ def _load():
     lib.pwa_token_gemm_supported.restype = i32
     lib.pwa_token_gemm_fwd.argtypes = [vp] * 11 + [C.c_int64, i32, i32, C.c_float, C.c_float, vp, vp]
     lib.pwa_token_gemm_fwd.restype = i32
+    lib.pwa_token_gemm_fwd_dt.argtypes = [vp] * 11 + [C.c_int64, i32, i32, C.c_float, C.c_float, vp, i32, vp]
+    lib.pwa_token_gemm_fwd_dt.restype = i32
     if hasattr(lib, "pwa_debug_fwd_timeline"):          # debug builds only (make TIMELINE=1, include/pwa_debug.h)
         lib.pwa_debug_fwd_timeline.argtypes = [vp, i32]
         lib.pwa_debug_fwd_timeline.restype = i32
@@ -106,7 +108,7 @@ def _load():
 lib = _load()
 
 EXPORTED_SYMBOLS = ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
-                    "pwa_partition", "pwa_reverse", "pwa_reverse_add", "pwa_gather_rows", "pwa_colsum_f32", "pwa_colsum_rows", "pwa_dropout", "pwa_dropout_colsum", "pwa_token_gemm_supported", "pwa_token_gemm_fwd", "pwa_attn_fwd", "pwa_attn_bwd", "pwa_attn_tc_supported", "pwa_attn_dense_fwd", "pwa_attn_dense_bwd",
+                    "pwa_partition", "pwa_reverse", "pwa_reverse_add", "pwa_gather_rows", "pwa_colsum_f32", "pwa_colsum_rows", "pwa_dropout", "pwa_dropout_colsum", "pwa_token_gemm_supported", "pwa_token_gemm_fwd", "pwa_token_gemm_fwd_dt", "pwa_attn_fwd", "pwa_attn_bwd", "pwa_attn_tc_supported", "pwa_attn_dense_fwd", "pwa_attn_dense_bwd",
                     "pwa_ln_fwd", "pwa_ln_bwd", "pwa_ln_bwd2", "pwa_bias_tables_fwd", "pwa_bias_tables_bwd")
 
 

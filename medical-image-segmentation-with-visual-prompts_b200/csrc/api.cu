@@ -74,7 +74,7 @@ extern "C" int pwa_attn_fwd(const void* q, const void* k, const void* v, const v
   if (rc != PWA_OK) return rc;
   PWA_CHECK_ARG(q && k && v && th && tw && td && out && lse, "pwa_attn_fwd: null pointer");
   PWA_CHECK_ARG(p.I == 0 || (kp && vp && tok), "pwa_attn_fwd: prompt tensors missing for I=%d", p.I);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_attn_fwd: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_attn_fwd: bad dtype %d", dtype);
   p.q = q; p.k = k; p.v = v; p.kp = kp; p.vp = vp;
   p.th = th; p.tw = tw; p.td = td; p.tok = tok; p.ids = ids;
   p.out = out; p.lse = lse;
@@ -94,9 +94,10 @@ extern "C" int pwa_attn_fwd(const void* q, const void* k, const void* v, const v
     return PWA_ERR_UNSUPPORTED;
   }
   if (impl == 2 || (impl == 0 && tc_ok)) {
-    // PWA_FWD_WS=0 (test infrastructure): the round-1 kernel (four 128-thread CTAs per SM) for A/B measurements
+    // PWA_FWD_WS=0 (test infrastructure): the round-1 kernel (four 128-thread CTAs per SM) for A/B measurements -- bf16
+    // only: fp16 always runs the warp-specialised kernel (tc_ok implies that it takes the shape)
     static const int use_ws = getenv("PWA_FWD_WS") ? atoi(getenv("PWA_FWD_WS")) : 1;
-    if (use_ws && attn_ws_supported(p, dtype)) return attn_ws_forward(p, st);
+    if ((use_ws || dtype == PWA_F16) && attn_ws_supported(p, dtype)) return attn_ws_forward(p, dtype, st);
     return attn_tc_forward(p, st);
   }
   return attn_f32_forward(p, dtype, st);
@@ -113,7 +114,7 @@ extern "C" int pwa_attn_bwd(const void* q, const void* k, const void* v, const v
   PWA_CHECK_ARG(q && k && v && th && tw && td && out && lse && dout && dq && dk && dv && dth && dtw && dtd && delta,
                 "pwa_attn_bwd: null pointer");
   PWA_CHECK_ARG(p.I == 0 || (kp && vp && tok && dkp && dvp && dtok), "pwa_attn_bwd: prompt tensors missing for I=%d", p.I);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_attn_bwd: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_attn_bwd: bad dtype %d", dtype);
   p.q = q; p.k = k; p.v = v; p.kp = kp; p.vp = vp;
   p.th = th; p.tw = tw; p.td = td; p.tok = tok; p.ids = ids;
   p.out = const_cast<void*>(out); p.lse = const_cast<float*>(lse); p.dout = dout;
@@ -134,6 +135,6 @@ extern "C" int pwa_attn_bwd(const void* q, const void* k, const void* v, const v
     set_error("pwa_attn_bwd: tcgen05 kernel does not support this shape/dtype");
     return PWA_ERR_UNSUPPORTED;
   }
-  if (impl == 2 || (impl == 0 && tc_ok)) return attn_tc_backward(p, st);
+  if (impl == 2 || (impl == 0 && tc_ok)) return attn_tc_backward(p, dtype, st);
   return attn_f32_backward(p, dtype, st);
 }

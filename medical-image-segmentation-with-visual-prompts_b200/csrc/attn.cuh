@@ -127,12 +127,13 @@ __device__ __forceinline__ uint32_t drop_transpose_tile(uint32_t x, int lane) {
 int attn_f32_forward(const AttnParams& p, int dtype, cudaStream_t st);
 int attn_f32_backward(const AttnParams& p, int dtype, cudaStream_t st);
 
-// bf16 tcgen05 / TMEM kernels (attn_tc.cu)
+// tcgen05 / TMEM kernels.  attn_tc_supported: bf16 -> the round-1 forward's envelope (attn_tc.cu, bf16 only); fp16 -> the
+// shapes that BOTH the warp-specialised forward and the backward take (the round-1 forward never runs fp16)
 bool attn_tc_supported(const AttnParams& p, int dtype);
-int attn_tc_forward(const AttnParams& p, cudaStream_t st);
+int attn_tc_forward(const AttnParams& p, cudaStream_t st);                 // bf16 only
 bool attn_ws_supported(const AttnParams& p, int dtype);       // attn_tc_ws.cu: warp-specialised forward
-int attn_ws_forward(const AttnParams& p, cudaStream_t st);
+int attn_ws_forward(const AttnParams& p, int dtype, cudaStream_t st);     // bf16 or fp16
 bool attn_tc_bwd_supported(const AttnParams& p, int dtype);   // attn_tc_bwd.cu
-int attn_tc_backward(const AttnParams& p, cudaStream_t st);
+int attn_tc_backward(const AttnParams& p, int dtype, cudaStream_t st);    // bf16 or fp16
 
 }  // namespace pwa

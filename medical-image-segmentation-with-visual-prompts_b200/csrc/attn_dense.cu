@@ -7,7 +7,7 @@
 //     logits[i][j] = (scale * q_i . k_j + bias[b, p, h, i, j]) * mask[b, p, h, i, j]      (mask multiplicative, BEFORE softmax)
 //     out_i        = dropout(softmax_j(logits)) @ v
 // Every row of q is a query (prompt rows included, as in the reference; n_q and n_k are free).  fp32 arithmetic on the
-// CUDA cores, fp32 or bf16 I/O; one CTA = one (sample, window, head) with the head's K / V (or Q / dO) slices in shared
+// CUDA cores, fp32, bf16 or fp16 I/O; one CTA = one (sample, window, head) with the head's K / V (or Q / dO) slices in shared
 // memory, one thread per query row (forward, dQ + dbias) or per key (dK / dV): the layout of attn_f32.cu, with global
 // reads of the dense tensors in place of table lookups.  Broadcast dimensions are strides of 0; the bias gradient is
 // accumulated with fp32 atomics into a buffer of the bias's own (broadcast) shape.
@@ -312,22 +312,24 @@ using namespace pwa;
 extern "C" int pwa_attn_dense_fwd(const void* q, const void* k, const void* v, const float* bias, const float* mask, void* out,
                                   float* lse, const pwa_dense_attn* s, int dtype, void* stream) {
   PWA_CHECK_ARG(q && k && v && out && lse, "pwa_attn_dense_fwd: null pointer");
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_attn_dense_fwd: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_attn_dense_fwd: bad dtype %d", dtype);
   DenseParams p{};
   if (int rc = fill_params(p, s, bias, mask, "pwa_attn_dense_fwd")) return rc;
   p.q = q; p.k = k; p.v = v; p.o = out; p.lse = lse;
-  return dtype == PWA_F32 ? dense_fwd_t<float>(p, s->dh, (cudaStream_t)stream) : dense_fwd_t<__nv_bfloat16>(p, s->dh, (cudaStream_t)stream);
+  cudaStream_t st = (cudaStream_t)stream;
+  return dtype == PWA_F32 ? dense_fwd_t<float>(p, s->dh, st) : dtype == PWA_BF16 ? dense_fwd_t<__nv_bfloat16>(p, s->dh, st) : dense_fwd_t<__half>(p, s->dh, st);
 }
 
 extern "C" int pwa_attn_dense_bwd(const void* q, const void* k, const void* v, const float* bias, const float* mask, const void* out,
                                   const float* lse, const void* dout, void* dq, void* dk, void* dv, float* dbias, float* delta,
                                   const pwa_dense_attn* s, int dtype, void* stream) {
   PWA_CHECK_ARG(q && k && v && out && lse && dout && dq && dk && dv && delta, "pwa_attn_dense_bwd: null pointer");
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_attn_dense_bwd: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_attn_dense_bwd: bad dtype %d", dtype);
   PWA_CHECK_ARG(dbias == nullptr || bias != nullptr, "pwa_attn_dense_bwd: dbias without bias");
   DenseParams p{};
   if (int rc = fill_params(p, s, bias, mask, "pwa_attn_dense_bwd")) return rc;
   p.q = q; p.k = k; p.v = v; p.out = out; p.lse = const_cast<float*>(lse); p.dout = dout;
   p.dq = dq; p.dk = dk; p.dv = dv; p.dbias = dbias; p.delta = delta;
-  return dtype == PWA_F32 ? dense_bwd_t<float>(p, s->dh, (cudaStream_t)stream) : dense_bwd_t<__nv_bfloat16>(p, s->dh, (cudaStream_t)stream);
+  cudaStream_t st = (cudaStream_t)stream;
+  return dtype == PWA_F32 ? dense_bwd_t<float>(p, s->dh, st) : dtype == PWA_BF16 ? dense_bwd_t<__nv_bfloat16>(p, s->dh, st) : dense_bwd_t<__half>(p, s->dh, st);
 }

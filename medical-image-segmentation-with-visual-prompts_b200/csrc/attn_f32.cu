@@ -438,12 +438,12 @@ template <typename T> static int bwd_t(const AttnParams& p, int dh, cudaStream_t
 
 int attn_f32_forward(const AttnParams& p, int dtype, cudaStream_t st) {
   const int dh = p.C / p.heads;
-  return dtype == PWA_F32 ? fwd_t<float>(p, dh, st) : fwd_t<__nv_bfloat16>(p, dh, st);
+  return dtype == PWA_F32 ? fwd_t<float>(p, dh, st) : dtype == PWA_BF16 ? fwd_t<__nv_bfloat16>(p, dh, st) : fwd_t<__half>(p, dh, st);
 }
 
 int attn_f32_backward(const AttnParams& p, int dtype, cudaStream_t st) {
   const int dh = p.C / p.heads;
-  return dtype == PWA_F32 ? bwd_t<float>(p, dh, st) : bwd_t<__nv_bfloat16>(p, dh, st);
+  return dtype == PWA_F32 ? bwd_t<float>(p, dh, st) : dtype == PWA_BF16 ? bwd_t<__nv_bfloat16>(p, dh, st) : bwd_t<__half>(p, dh, st);
 }
 
 }  // namespace pwa

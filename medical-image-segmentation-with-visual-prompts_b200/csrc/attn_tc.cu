@@ -640,6 +640,7 @@ int launch_tc(const AttnParams& p, cudaStream_t st) {
 }  // namespace
 
 bool attn_tc_supported(const AttnParams& p, int dtype) {
+  if (dtype == PWA_F16) return attn_ws_supported(p, PWA_BF16) && attn_tc_bwd_supported(p, PWA_BF16);
   if (dtype != PWA_BF16) return false;
   if (p.N != kN) return false;                                   // two 128-row tiles / two 128-key content blocks
   if (p.wd > 4 || p.wh + p.ww > 16) return false;                // one-hot bias columns must fit the layout

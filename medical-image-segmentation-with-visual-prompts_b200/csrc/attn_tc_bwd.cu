@@ -1,4 +1,4 @@
-// (c) backward of the fused prompted window attention on tcgen05 tensor cores + TMEM, bf16 I/O.
+// (c) backward of the fused prompted window attention on tcgen05 tensor cores + TMEM, bf16 or fp16 I/O.
 //
 // One persistent CTA per SM (800 threads, all 512 TMEM columns) = one fixed head, walking over (sample, window)
 // pairs.  Everything is computed in the TRANSPOSED orientation: the 128 TMEM lanes are KEYS (one key block:
@@ -118,8 +118,8 @@ __host__ __device__ inline BwdSmem bwd_layout(int KS, int DHP, int NKT, int wh, 
   return s;
 }
 
-template <int DH>
-__device__ __forceinline__ void load_row_b(const __nv_bfloat16* src, __nv_bfloat16 (&dst)[DH]) {
+template <int DH, typename E>
+__device__ __forceinline__ void load_row_b(const E* src, E (&dst)[DH]) {
   if constexpr (DH % 4 == 0) {
     const uint2* s2 = reinterpret_cast<const uint2*>(src);
     uint2* d2 = reinterpret_cast<uint2*>(dst);
@@ -131,35 +131,35 @@ __device__ __forceinline__ void load_row_b(const __nv_bfloat16* src, __nv_bfloat
   }
 }
 
-template <int DH>
-__device__ __forceinline__ void store_row_b(__nv_bfloat16* dst, const float* v, float mul) {
+template <int DH, typename E>
+__device__ __forceinline__ void store_row_b(E* dst, const float* v, float mul) {
   if constexpr (DH % 4 == 0) {
 #pragma unroll
     for (int d = 0; d < DH; d += 4) {
       uint2 w;
-      w.x = pack_bf16(v[d] * mul, v[d + 1] * mul);
-      w.y = pack_bf16(v[d + 2] * mul, v[d + 3] * mul);
+      w.x = pack2t<E>(v[d] * mul, v[d + 1] * mul);
+      w.y = pack2t<E>(v[d + 2] * mul, v[d + 3] * mul);
       *reinterpret_cast<uint2*>(dst + d) = w;
     }
   } else {
 #pragma unroll
-    for (int d = 0; d < DH; ++d) dst[d] = __float2bfloat16(v[d] * mul);
+    for (int d = 0; d < DH; ++d) dst[d] = from_f32<E>(v[d] * mul);
   }
 }
 
 // [real DH | up to 4 extra columns | zero pad] -> NCH chunks of 8 columns, chunk c of row r at base + c*stride + r*16
-template <int DH, int NCH>
-__device__ __forceinline__ void store_chunks_b(uint8_t* base, uint32_t chunk_stride, int row, const __nv_bfloat16 (&real)[DH],
-                                               __nv_bfloat16 x0, __nv_bfloat16 x1, __nv_bfloat16 x2, __nv_bfloat16 x3) {
-  const __nv_bfloat16 zero = __float2bfloat16(0.f);
+template <int DH, int NCH, typename E>
+__device__ __forceinline__ void store_chunks_b(uint8_t* base, uint32_t chunk_stride, int row, const E (&real)[DH],
+                                               E x0, E x1, E x2, E x3) {
+  const E zero = from_f32<E>(0.f);
 #pragma unroll
   for (int c = 0; c < NCH; ++c) {
-    __align__(16) __nv_bfloat16 tmp[8];
+    __align__(16) E tmp[8];
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int col = c * 8 + e;
       const int x = col - DH;
-      __nv_bfloat16 v = zero;
+      E v = zero;
       if (col < DH) v = real[col < DH ? col : 0];
       else if (x == 0) v = x0;
       else if (x == 1) v = x1;
@@ -192,7 +192,10 @@ enum {
 // DROP: attention dropout (window_attention.py:57) with the mask of csrc/attn.cuh.  P^T feeds dV dropped (one AND on
 // the packed pairs, after the shift mask; the inverse keep rate is applied when dV is drained), dP^T is masked and
 // scaled before delta is subtracted (so delta cannot ride in the dP^T MMA: FOLD is off).
-template <int DH, bool MASKED, bool DROP>
+// E: element type of the token tensors and of the MMA operands (bf16 or fp16).  P^T uses the exact log-sum-exp (P <= 1), so
+// fp16's range matters only for g = P (dP - delta), delta and the stored gradients: under a large loss scale they overflow to
+// inf (NaN where inf meets inf), never to a finite value, and a non-finite dout stays non-finite -- GradScaler sees it.
+template <int DH, bool MASKED, bool DROP, typename E>
 // (72 registers is the hard cap: 25 warps spread 7/6/6/6 over the four sub-partitions of 16 384 registers each, and
 //  7 warps x 32 x 80 does not fit -- a __maxnreg__(80) build fails to launch)
 __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p) {
@@ -231,7 +234,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
   const uint32_t seed1 = DROP ? (p.drop_seed ? p.drop_seed[1] : p.seed_host[1]) : 0u;
   const DropThresh& dth = p.drop_planes;          // constant bank (filled by the dispatcher)
   const float keep_scale = DROP ? p.inv_keep : 1.f;
-  const __nv_bfloat16 one = __float2bfloat16(1.f), zero = __float2bfloat16(0.f);
+  const E one = from_f32<E>(1.f), zero = from_f32<E>(0.f);
 
   // ---- once per CTA: zero everything the MMAs may touch beyond the staged rows, window-independent operands ----
   for (uint32_t i = tid; i < L.total / 16; i += kThreadsB) reinterpret_cast<uint4*>(smem)[i] = make_uint4(0, 0, 0, 0);
@@ -240,7 +243,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
     const int iw = (n / p.wd) % p.ww, ih = n / (p.wd * p.ww);
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-      __align__(16) __nv_bfloat16 tmp[8];
+      __align__(16) E tmp[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int col = c * 8 + e;
@@ -260,7 +263,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
     const int jw = (j / p.wd) % p.ww, jh = j / (p.wd * p.ww);
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-      __align__(16) __nv_bfloat16 tmp[8];
+      __align__(16) E tmp[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int col = c * 8 + e;
@@ -271,7 +274,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
         } else if (col < p.wh) {
           v = gtok_s[j - kN];
         }
-        tmp[e] = __float2bfloat16(v * inv_scale);
+        tmp[e] = from_f32<E>(v * inv_scale);
       }
       *reinterpret_cast<uint4*>(Ka + c * (NKR * 16) + j * 16) = *reinterpret_cast<const uint4*>(tmp);
     }
@@ -349,7 +352,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
       const uint8_t* opnd = smem + L.opnd0 + ob * L.opnd_bytes;
       const float* lse2_s = reinterpret_cast<const float*>(opnd + L.lse2);
       const float* delta_s = reinterpret_cast<const float*>(opnd + L.delta);
-      const __nv_bfloat16* wp_s = reinterpret_cast<const __nv_bfloat16*>(opnd + L.wp);
+      const E* wp_s = reinterpret_cast<const E*>(opnd + L.wp);
       const uint32_t* rs_s = reinterpret_cast<const uint32_t*>(opnd + L.rs);
       const uint32_t* sel_s = reinterpret_cast<const uint32_t*>(opnd + L.sel);
       const uint8_t* ids_s = opnd + L.ids;
@@ -420,10 +423,10 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
                   gv[e] = pv[e] * (FOLD ? dpe : dpe + nd[e]);
                 }
               }
-              pk[q4 * 2] = pack_bf16(pv[0], pv[1]);
-              pk[q4 * 2 + 1] = pack_bf16(pv[2], pv[3]);
-              gk[q4 * 2] = pack_bf16(gv[0], gv[1]);
-              gk[q4 * 2 + 1] = pack_bf16(gv[2], gv[3]);
+              pk[q4 * 2] = pack2t<E>(pv[0], pv[1]);
+              pk[q4 * 2 + 1] = pack2t<E>(pv[2], pv[3]);
+              gk[q4 * 2] = pack2t<E>(gv[0], gv[1]);
+              gk[q4 * 2 + 1] = pack2t<E>(gv[2], gv[3]);
             }
             if (do_mask) {
               const uint4 s4 = *reinterpret_cast<const uint4*>(sel_s + id_slot(cid) * (kN / 4) + r0 / 4 + h * 4);
@@ -472,11 +475,11 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
     // round 1 measured as "one thread issues a tcgen05.mma only every ~100-200 clk").
     {
       const uint32_t tmem = __shfl_sync(0xffffffffu, tmem_base_s, 0);
-      const uint32_t idescT = make_idesc_bf16(128, 64, 0, 0);       // S^T, dP^T : A K-major, B K-major, N = 64 rows
-      const uint32_t idescDV = make_idesc_bf16(128, DHP, 0, 1);     // dV  : A tmem, B = dO MN-major
-      const uint32_t idescDK = make_idesc_bf16(128, DKC, 0, 1);     // dK' : A tmem, B = Q' MN-major
-      const uint32_t idescAUG = make_idesc_bf16(128, 16, 0, 1);     // dKaug
-      const uint32_t idescDQ = make_idesc_bf16(128, DKC, 1, 1);     // dQ' : A = g smem MN-major, B = K' MN-major
+      const uint32_t idescT = make_idesc<E>(128, 64, 0, 0);       // S^T, dP^T : A K-major, B K-major, N = 64 rows
+      const uint32_t idescDV = make_idesc<E>(128, DHP, 0, 1);     // dV  : A tmem, B = dO MN-major
+      const uint32_t idescDK = make_idesc<E>(128, DKC, 0, 1);     // dK' : A tmem, B = Q' MN-major
+      const uint32_t idescAUG = make_idesc<E>(128, 16, 0, 1);     // dKaug
+      const uint32_t idescDQ = make_idesc<E>(128, DKC, 1, 1);     // dQ' : A = g smem MN-major, B = K' MN-major
       const int role = __shfl_sync(0xffffffffu, warp - kIssue0, 0); // 0 S, 1 V, 2 K, 3 A, 4 Q
       int it = 0;
       for (int bw = bw0; bw < n_pairs; bw += stride, ++it) {
@@ -629,7 +632,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
       uint8_t* dOs = opnd + L.dO;
       float* lse2_s = reinterpret_cast<float*>(opnd + L.lse2);
       float* delta_s = reinterpret_cast<float*>(opnd + L.delta);
-      __nv_bfloat16* wp_s = reinterpret_cast<__nv_bfloat16*>(opnd + L.wp);
+      E* wp_s = reinterpret_cast<E*>(opnd + L.wp);
       uint32_t* rs_s = reinterpret_cast<uint32_t*>(opnd + L.rs);
       uint32_t* sel_s = reinterpret_cast<uint32_t*>(opnd + L.sel);
       uint8_t* ids_s = opnd + L.ids;
@@ -656,24 +659,25 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
         if (!(all || part == qi)) continue;
         const int n = pt + qi * kProd;
         const size_t goff = ((size_t)bw * kN + n) * p.C + head * DH;
-        __nv_bfloat16 row[DH], drow[DH], orow[DH];
-        load_row_b<DH>((const __nv_bfloat16*)p.q + ((size_t)bw * kN + n) * p.ldq + head * DH, row);
-        load_row_b<DH>((const __nv_bfloat16*)p.dout + goff, drow);
-        load_row_b<DH>((const __nv_bfloat16*)p.out + goff, orow);
+        E row[DH], drow[DH], orow[DH];
+        load_row_b<DH>((const E*)p.q + ((size_t)bw * kN + n) * p.ldq + head * DH, row);
+        load_row_b<DH>((const E*)p.dout + goff, drow);
+        load_row_b<DH>((const E*)p.out + goff, orow);
         const float l2 = p.lse[((size_t)bw * p.heads + head) * kN + n] * 1.4426950408889634f;
         const int id_ = n % p.wd;
         store_chunks_b<DH, KS * 2>(Qs, kN * 16, n, row, id_ == 0 ? one : zero, id_ == 1 ? one : zero, id_ == 2 ? one : zero,
                                    id_ == 3 ? one : zero);
         float dl = 0.f;
 #pragma unroll
-        for (int d = 0; d < DH; ++d) dl = fmaf(__bfloat162float(drow[d]), __bfloat162float(orow[d]), dl);
-        // dO' = [dO | -delta (bf16 hi, lo)]: with V' = [V | 1 1] the dP^T MMA yields dP - delta directly
-        const __nv_bfloat16 dhi = __float2bfloat16(-dl);
-        const __nv_bfloat16 dlo = __float2bfloat16(-dl - __bfloat162float(dhi));
+        for (int d = 0; d < DH; ++d) dl = fmaf(to_f32(drow[d]), to_f32(orow[d]), dl);
+        // dO' = [dO | -delta (hi, lo in E)]: with V' = [V | 1 1] the dP^T MMA yields dP - delta directly.  (fp16: a delta
+        // beyond 65504 gives hi = +-inf, lo = -+inf and NaN in dP - delta: non-finite, as the fp32 value would make dq)
+        const E dhi = from_f32<E>(-dl);
+        const E dlo = from_f32<E>(-dl - to_f32(dhi));
         store_chunks_b<DH, DHP / 8>(dOs, kN * 16, n, drow, FOLD ? dhi : zero, FOLD ? dlo : zero, zero, zero);
         delta_s[n] = -dl;                                          // (the compute warps add it)
         lse2_s[n] = l2;
-        wp_s[n] = __float2bfloat16(fast_exp2(-l2));
+        wp_s[n] = from_f32<E>(fast_exp2(-l2));
       }
       for (int ki = 0; ki < 3; ++ki) {                             // key rows: K', V'
         if (!(all || (part == 2 && ki < 2) || (part == 3 && ki == 2))) continue;
@@ -681,14 +685,14 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
         if (j >= NKT) continue;
         const bool content = j < kN;
         const size_t off = content ? ((size_t)bw * kN + j) * p.ldq + head * DH : ((size_t)b * p.I + (j - kN)) * p.ldp + head * DH;
-        __nv_bfloat16 row[DH], vrow[DH];
-        load_row_b<DH>((const __nv_bfloat16*)(content ? p.k : p.kp) + off, row);
-        load_row_b<DH>((const __nv_bfloat16*)(content ? p.v : p.vp) + off, vrow);
+        E row[DH], vrow[DH];
+        load_row_b<DH>((const E*)(content ? p.k : p.kp) + off, row);
+        load_row_b<DH>((const E*)(content ? p.v : p.vp) + off, vrow);
         const int jd = j % p.wd;
-        __nv_bfloat16 ex[4];
+        E ex[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u)
-          ex[u] = (content && u < p.wd) ? __float2bfloat16(__ldg(&p.td[(head * p.wd + u) * p.wd + jd]) * inv_scale) : zero;
+          ex[u] = (content && u < p.wd) ? from_f32<E>(__ldg(&p.td[(head * p.wd + u) * p.wd + jd]) * inv_scale) : zero;
         store_chunks_b<DH, KS * 2>(Ks, NKR * 16, j, row, ex[0], ex[1], ex[2], ex[3]);
         store_chunks_b<DH, DHP / 8>(Vs, NKR * 16, j, vrow, FOLD ? one : zero, FOLD ? one : zero, zero, zero);
       }
@@ -729,7 +733,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
       auto put_dv = [&](const float (&dv)[DHP]) {
         if (!key_ok) return;
         if (kb < 2) {
-          store_row_b<DH>((__nv_bfloat16*)p.dv + ((size_t)bw * kN + key) * p.ldq + head * DH, dv, keep_scale);
+          store_row_b<DH>((E*)p.dv + ((size_t)bw * kN + key) * p.ldq + head * DH, dv, keep_scale);
         } else if constexpr (kRegPrompt) {
 #pragma unroll
           for (int d = 0; d < DH; ++d) accp_v[d] = fmaf(dv[d], keep_scale, accp_v[d]);
@@ -742,7 +746,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
       auto put_dk = [&](const float (&dk)[DKC]) {
         if (!key_ok) return;
         if (kb < 2) {
-          store_row_b<DH>((__nv_bfloat16*)p.dk + ((size_t)bw * kN + key) * p.ldq + head * DH, dk, p.scale);
+          store_row_b<DH>((E*)p.dk + ((size_t)bw * kN + key) * p.ldq + head * DH, dk, p.scale);
 #pragma unroll
           for (int uu = 0; uu < 4; ++uu) acc_d[kb][uu] += dk[DH + uu];   // d K'[DH+u] = sum_rows(id==u) g = dTd[u][jd]
         } else if constexpr (kRegPrompt) {
@@ -797,14 +801,14 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
           for (int d = 0; d < 16; ++d) dq[mt][c * 16 + d] = __uint_as_float(o[d]);
         }
         if constexpr (2 * DKC > 64)      // large heads: one tile at a time (registers)
-          store_row_b<DH>((__nv_bfloat16*)p.dq + ((size_t)bw * kN + mt * 128 + lane_row) * p.ldq + head * DH, dq[mt], p.scale);
+          store_row_b<DH>((E*)p.dq + ((size_t)bw * kN + mt * 128 + lane_row) * p.ldq + head * DH, dq[mt], p.scale);
       }
       tc_fence_before();
       mbar_arrive(&bar[bDqFree]);
       if constexpr (2 * DKC <= 64) {
 #pragma unroll
         for (int mt = 0; mt < 2; ++mt)
-          store_row_b<DH>((__nv_bfloat16*)p.dq + ((size_t)bw * kN + mt * 128 + lane_row) * p.ldq + head * DH, dq[mt], p.scale);
+          store_row_b<DH>((E*)p.dq + ((size_t)bw * kN + mt * 128 + lane_row) * p.ldq + head * DH, dq[mt], p.scale);
       }
       STAMP(4);
     };
@@ -936,7 +940,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
   if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-template <int DH>
+template <int DH, typename E>
 int launch_bwd_tc(const AttnParams& p, cudaStream_t st) {
   constexpr int DHP = BCfg<DH>::DHP, KS = BCfg<DH>::KS;
   const int NKT = kN + p.I;
@@ -947,8 +951,8 @@ int launch_bwd_tc(const AttnParams& p, cudaStream_t st) {
   if (grid < p.heads) grid = p.heads;
   const int need = p.B * p.P * p.heads;
   if (grid > need) grid = need;
-  auto kern = p.drop_thresh ? (p.ids ? attn_bwd_tc_kernel<DH, true, true> : attn_bwd_tc_kernel<DH, false, true>)
-                            : (p.ids ? attn_bwd_tc_kernel<DH, true, false> : attn_bwd_tc_kernel<DH, false, false>);
+  auto kern = p.drop_thresh ? (p.ids ? attn_bwd_tc_kernel<DH, true, true, E> : attn_bwd_tc_kernel<DH, false, true, E>)
+                            : (p.ids ? attn_bwd_tc_kernel<DH, true, false, E> : attn_bwd_tc_kernel<DH, false, false, E>);
   PWA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, kThreadsB, smem, st>>>(p);
   PWA_CUDA_OK(cudaGetLastError());
@@ -965,16 +969,21 @@ bool attn_tc_bwd_supported(const AttnParams& p, int dtype) {
   return bwd_layout(KS, DHP, kN + p.I, p.wh, p.ww, p.wd, p.I, true).total <= 224 * 1024;
 }
 
-int attn_tc_backward(const AttnParams& p, cudaStream_t st) {
+template <typename E>
+static int backward_t(const AttnParams& p, cudaStream_t st) {
   switch (p.C / p.heads) {
-    case 3: return launch_bwd_tc<3>(p, st);
-    case 6: return launch_bwd_tc<6>(p, st);
-    case 12: return launch_bwd_tc<12>(p, st);
-    case 24: return launch_bwd_tc<24>(p, st);
-    case 48: return launch_bwd_tc<48>(p, st);
+    case 3: return launch_bwd_tc<3, E>(p, st);
+    case 6: return launch_bwd_tc<6, E>(p, st);
+    case 12: return launch_bwd_tc<12, E>(p, st);
+    case 24: return launch_bwd_tc<24, E>(p, st);
+    case 48: return launch_bwd_tc<48, E>(p, st);
   }
   set_error("tcgen05 attention backward: head_dim %d not instantiated", p.C / p.heads);
   return PWA_ERR_UNSUPPORTED;
+}
+
+int attn_tc_backward(const AttnParams& p, int dtype, cudaStream_t st) {
+  return dtype == PWA_F16 ? backward_t<__half>(p, st) : backward_t<__nv_bfloat16>(p, st);
 }
 
 }  // namespace pwa

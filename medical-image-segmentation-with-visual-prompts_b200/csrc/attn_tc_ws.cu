@@ -1,4 +1,4 @@
-// (b) fused prompted window attention forward, warp-specialised (tcgen05 + TMEM, bf16 I/O) -- round-2 kernel.
+// (b) fused prompted window attention forward, warp-specialised (tcgen05 + TMEM, bf16 or fp16 I/O) -- round-2 kernel.
 //
 // One persistent CTA per SM (768 threads = 24 warps, 6 per scheduler) = one fixed head, walking (sample, window) pairs.
 // The softmax of this path is bound by the MUFU pipe (one ex2 per logit, 16 / clk / SM), so everything else is taken off
@@ -24,6 +24,8 @@
 // rare fallback), no online rescaling, relative-position bias folded into the QK^T MMA through one-hot / table columns,
 // multiplicative pre-softmax shift mask (window_attention.py:49-58), ones column of V for the softmax denominator,
 // bit-sliced dropout keep words (csrc/attn.cuh).  TMEM: per group 3 x 64 columns of S / P plus 1-2 O accumulators.
+#include <type_traits>
+
 #include "attn.cuh"
 #include "tc_common.cuh"
 
@@ -123,21 +125,44 @@ __device__ __forceinline__ uint32_t hadd2_bf16(uint32_t a, uint32_t b) {
   asm("add.rn.bf16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
   return d;
 }
+__device__ __forceinline__ uint32_t hadd2_f16(uint32_t a, uint32_t b) {
+  uint32_t d;
+  asm("add.rn.f16x2 %0, %1, %2;" : "=r"(d) : "r"(a), "r"(b));
+  return d;
+}
+template <typename T> __device__ __forceinline__ uint32_t hadd2t(uint32_t a, uint32_t b) {
+  return std::is_same<T, __half>::value ? hadd2_f16(a, b) : hadd2_bf16(a, b);
+}
+
+// Stabiliser of the element type.  P = exp2(S c - mb) with mb an upper bound of the row's logits (norm bound, or the exact
+// row maximum after the sweep) is rounded to T before the PV MMA.  bf16 has fp32's exponent range: a row whose largest P
+// is 2^-80 still normalises.  fp16 flushes below 2^-24 (normal from 2^-14), so the fp16 kernel forms P = exp2(S c - mb + 10)
+// (largest P <= 2^10: a 32-key partial sum of the dropout denominator stays <= 2^15 < 65504) and sweeps for the exact row
+// maximum as soon as the bound may sit more than 24 binades above it: the row's largest P is then >= 2^(10 - 24) = 2^-14,
+// a normal fp16 number, and whatever still flushes lies below the rounding error of that largest term.
+template <typename T> struct WsStab {
+  static constexpr float shift = 0.f, max_gap = 2.f * kMaxBoundW;
+};
+template <> struct WsStab<__half> {
+  static constexpr float shift = 10.f, max_gap = 24.f;
+};
 // Dropout on the 16 packed pairs of a 32-key chunk + the chunk's share of the softmax denominator (the undropped values,
 // after the shift mask).  The ALU pipe (shifts, logic, PRMT) is what saturates in the dropout variants (ncu: 64 % busy next
 // to 25 % on the FMA pipe), so the sum is formed where it is cheapest there: four pairs are first added as packed bf16 on
 // the FMA pipe (HADD2.BF16; partial sums of <= 4 probabilities, 2^-9 relative each, averaging out over the row's 40
 // groups) and only every fourth pair is unpacked into the fp32 accumulators.
-template <int G = 0>
+template <typename T, int G = 0>
 __device__ __forceinline__ void drop_apply16w(uint32_t (&pk)[16], uint32_t kw, float& s0, float& s1) {
   if constexpr (G < 16) {
-    const uint32_t part = hadd2_bf16(hadd2_bf16(pk[G], pk[G + 1]), hadd2_bf16(pk[G + 2], pk[G + 3]));
-    fadd2w(s0, s1, __uint_as_float(part << 16), __uint_as_float(part & 0xffff0000u));
+    const uint32_t part = hadd2t<T>(hadd2t<T>(pk[G], pk[G + 1]), hadd2t<T>(pk[G + 2], pk[G + 3]));
+    float f0, f1;
+    unpack2t<T>(part, f0, f1);
+    fadd2w(s0, s1, f0, f1);
     pk[G] &= drop_pair_mask<G>(kw);
     pk[G + 1] &= drop_pair_mask<G + 1>(kw);
     pk[G + 2] &= drop_pair_mask<G + 2>(kw);
     pk[G + 3] &= drop_pair_mask<G + 3>(kw);
-    drop_apply16w<G + 4>(pk, kw, s0, s1);
+    drop_apply16w<T, G + 4>(pk, kw, s0, s1);
   }
 }
 
@@ -188,8 +213,8 @@ __host__ __device__ inline WsSmem ws_layout(int KS, int DHP, int NKT, bool maske
   return s;
 }
 
-template <int DH>
-__device__ __forceinline__ void load_row_w(const __nv_bfloat16* src, __nv_bfloat16 (&dst)[DH]) {
+template <int DH, typename T>
+__device__ __forceinline__ void load_row_w(const T* src, T (&dst)[DH]) {
   if constexpr (DH % 4 == 0) {
     const uint2* s2 = reinterpret_cast<const uint2*>(src);
     uint2* d2 = reinterpret_cast<uint2*>(dst);
@@ -200,28 +225,28 @@ __device__ __forceinline__ void load_row_w(const __nv_bfloat16* src, __nv_bfloat
     for (int i = 0; i < DH; ++i) dst[i] = src[i];
   }
 }
-template <int DH>
-__device__ __forceinline__ float sumsq_w(const __nv_bfloat16 (&r)[DH]) {
+template <int DH, typename T>
+__device__ __forceinline__ float sumsq_w(const T (&r)[DH]) {
   float s = 0.f;
 #pragma unroll
   for (int i = 0; i < DH; ++i) {
-    const float v = __bfloat162float(r[i]);
+    const float v = to_f32(r[i]);
     s = fmaf(v, v, s);
   }
   return s;
 }
 // staged K-dim layout of one head: [real DH | up to 4 extra columns | zero pad] -> KS k-steps of 16
-template <int DH, int KS>
-__device__ __forceinline__ void store_chunks_w(uint8_t* base, uint32_t chunk_stride, int row, const __nv_bfloat16 (&real)[DH],
-                                               const __nv_bfloat16 (&extra)[4], int n_extra) {
+template <int DH, int KS, typename T>
+__device__ __forceinline__ void store_chunks_w(uint8_t* base, uint32_t chunk_stride, int row, const T (&real)[DH],
+                                               const T (&extra)[4], int n_extra) {
 #pragma unroll
   for (int c = 0; c < KS * 2; ++c) {
-    __align__(16) __nv_bfloat16 tmp[8];
+    __align__(16) T tmp[8];
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int col = c * 8 + e;
       const int x = col - DH;
-      __nv_bfloat16 v = __float2bfloat16(0.f);
+      T v = from_f32<T>(0.f);
       if (col < DH) v = real[col < DH ? col : 0];
       else if (x < 4 && x < n_extra) v = extra[x & 3];
       tmp[e] = v;
@@ -248,7 +273,7 @@ __device__ __forceinline__ void stage_sync() { asm volatile("bar.sync 1, %0;" ::
 // S buffer it would skip a phase between two waits, which a parity wait cannot tell apart; unit % 6 is always the same set
 enum { bOpFull = 0, bOpFree = 3, bSFull = 6, bPReady = 18, bOFull = 24, bOFree = 28, bLsum = 32, kNumBarsW = 38 };
 
-template <int DH, bool MASKED, bool DROP>
+template <int DH, bool MASKED, bool DROP, typename T>
 __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p) {
   constexpr int DHP = WCfg<DH>::DHP, NDC = WCfg<DH>::NDC, KS = WCfg<DH>::KS, NOB = WCfg<DH>::NOB, GC = WCfg<DH>::GC;
   extern __shared__ __align__(128) uint8_t smem[];
@@ -267,7 +292,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
   const int head = blockIdx.x % p.heads;
   const float inv_scale = 1.f / p.scale;
   const float c2 = p.scale * 1.4426950408889634f;          // logits -> log2 domain
-  const __nv_bfloat16 one = __float2bfloat16(1.f), zero = __float2bfloat16(0.f);
+  const T one = from_f32<T>(1.f), zero = from_f32<T>(0.f);
   const int n_units = (NKT + kUK - 1) / kUK;
   const int last_nk = NKT - kUK * (n_units - 1);            // 64 or 32
   const int n_pairs = p.B * p.P;
@@ -295,7 +320,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
     const int id_ = n % p.wd, iw = (n / p.wd) % p.ww, ih = n / (p.wd * p.ww);
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-      __align__(16) __nv_bfloat16 tmp[8];
+      __align__(16) T tmp[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int col = c * 8 + e;
@@ -315,7 +340,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
     const int jw = (j / p.wd) % p.ww, jh = j / (p.wd * p.ww);
 #pragma unroll
     for (int c = 0; c < 2; ++c) {
-      __align__(16) __nv_bfloat16 tmp[8];
+      __align__(16) T tmp[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) {
         const int col = c * 8 + e;
@@ -326,7 +351,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
         } else if (col < p.wh) {
           v = tok_s[j - kN];
         }
-        tmp[e] = __float2bfloat16(v * inv_scale);
+        tmp[e] = from_f32<T>(v * inv_scale);
       }
       *reinterpret_cast<uint4*>(Ka + c * (NKT * 16) + j * 16) = *reinterpret_cast<const uint4*>(tmp);
     }
@@ -419,10 +444,11 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
         asm volatile("bar.sync %0, 256;" ::"r"(2 + g) : "memory");  // both partials read before the denominators reuse the slots
         mb = mx * c2;
       }
+      if constexpr (WsStab<T>::shift != 0.f) mb -= WsStab<T>::shift;
       const uint32_t rhash = DROP ? drop_row_hash(seed0, seed1, (uint32_t)bw, (uint32_t)p.heads, (uint32_t)head, kN, (uint32_t)rown) : 0u;
       float lsum0 = 0.f, lsum1 = 0.f;
       const float e0 = ex2f(-mb);                                  // weight of every masked (zeroed) logit
-      const uint32_t e0pair = pack_bf16(e0, e0);
+      const uint32_t e0pair = pack2t<T>(e0, e0);
       const uint32_t* selrow = sel_s + id_slot_w(rid) * (kN / 4);
       WS_PROF(1);
 
@@ -450,7 +476,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
               p0 = ex2f(x0);
               p1 = ex2f(x1);
             }
-            pk[q] = pack_bf16(p0, p1);
+            pk[q] = pack2t<T>(p0, p1);
           }
           if (do_mask) {
             const uint4* sp = reinterpret_cast<const uint4*>(selrow + u * (kUK / 4) + c * 8);
@@ -467,7 +493,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
           }
           if (DROP) {
             const uint32_t kw = drop_keep_word(rhash, (uint32_t)(u * (kUK / 32) + c), dth);
-            drop_apply16w(pk, kw, lsum0, lsum1);
+            drop_apply16w<T>(pk, kw, lsum0, lsum1);
           }
           tmem_st16(trow + buf * kUK + c * 16, pk);
         }
@@ -503,18 +529,18 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
           l_run = part_s[rown] + part_s[kN + rown];
         }
         const float inv = (DROP ? p.inv_keep : 1.f) / l_run;
-        __nv_bfloat16* og = (__nv_bfloat16*)p.out + ((size_t)bw * kN + rown) * p.C + head * DH;
+        T* og = (T*)p.out + ((size_t)bw * kN + rown) * p.C + head * DH;
         if constexpr (DH % 4 == 0) {
 #pragma unroll
           for (int d = 0; d < DH; d += 4) {
             uint2 v;
-            v.x = pack_bf16(o_run[d] * inv, o_run[d + 1] * inv);
-            v.y = pack_bf16(o_run[d + 2] * inv, o_run[d + 3] * inv);
+            v.x = pack2t<T>(o_run[d] * inv, o_run[d + 1] * inv);
+            v.y = pack2t<T>(o_run[d + 2] * inv, o_run[d + 3] * inv);
             *reinterpret_cast<uint2*>(og + d) = v;
           }
         } else {
 #pragma unroll
-          for (int d = 0; d < DH; ++d) og[d] = __float2bfloat16(o_run[d] * inv);
+          for (int d = 0; d < DH; ++d) og[d] = from_f32<T>(o_run[d] * inv);
         }
         p.lse[((size_t)bw * p.heads + head) * kN + rown] = (mb + __log2f(l_run)) * 0.6931471805599453f;
       }
@@ -544,16 +570,16 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
         for (int n = st; n < kN; n += kStageThreads) {
           const int id_ = n % p.wd;
           for (int e = DH; e < KS * 16; ++e)
-            *reinterpret_cast<__nv_bfloat16*>(opnd + L.q + (e >> 3) * (kN * 16) + n * 16 + (e & 7) * 2) =
+            *reinterpret_cast<T*>(opnd + L.q + (e >> 3) * (kN * 16) + n * 16 + (e & 7) * 2) =
                 (e - DH < p.wd && e - DH == id_) ? one : zero;
         }
         for (int j = st; j < NKT; j += kStageThreads) {
           const int jd = j % p.wd;
           for (int e = DH; e < KS * 16; ++e)
-            *reinterpret_cast<__nv_bfloat16*>(opnd + L.k + (e >> 3) * (NKT * 16) + j * 16 + (e & 7) * 2) =
-                (j < kN && e - DH < p.wd) ? __float2bfloat16(td_s[(e - DH) * p.wd + jd] * inv_scale) : zero;
+            *reinterpret_cast<T*>(opnd + L.k + (e >> 3) * (NKT * 16) + j * 16 + (e & 7) * 2) =
+                (j < kN && e - DH < p.wd) ? from_f32<T>(td_s[(e - DH) * p.wd + jd] * inv_scale) : zero;
           for (int e = DH; e < DHP; ++e)
-            *reinterpret_cast<__nv_bfloat16*>(opnd + L.v + (j >> 3) * (NDC * 128) + (e >> 3) * 128 + (j & 7) * 16 + (e & 7) * 2) =
+            *reinterpret_cast<T*>(opnd + L.v + (j >> 3) * (NDC * 128) + (e >> 3) * 128 + (j & 7) * 16 + (e & 7) * 2) =
                 e == DH ? one : zero;
         }
       }
@@ -603,14 +629,14 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
         if constexpr (PIECES) {
           // asynchronous 8-byte copies (LDGSTS): every piece of the window in flight at once, no register staging -- the
           // global round trip (~3 K clk under load) is paid once per window instead of once per register batch
-          auto cp8 = [](uint8_t* dst, const __nv_bfloat16* src) {
+          auto cp8 = [](uint8_t* dst, const T* src) {
             asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
           };
-          const __nv_bfloat16* qb = (const __nv_bfloat16*)p.q + (size_t)bw * kN * p.ldq + head * DH;
-          const __nv_bfloat16* kb = (const __nv_bfloat16*)p.k + (size_t)bw * kN * p.ldq + head * DH;
-          const __nv_bfloat16* vb = (const __nv_bfloat16*)p.v + (size_t)bw * kN * p.ldq + head * DH;
-          const __nv_bfloat16* kpb = (const __nv_bfloat16*)p.kp + (size_t)b * p.I * p.ldp + head * DH;
-          const __nv_bfloat16* vpb = (const __nv_bfloat16*)p.vp + (size_t)b * p.I * p.ldp + head * DH;
+          const T* qb = (const T*)p.q + (size_t)bw * kN * p.ldq + head * DH;
+          const T* kb = (const T*)p.k + (size_t)bw * kN * p.ldq + head * DH;
+          const T* vb = (const T*)p.v + (size_t)bw * kN * p.ldq + head * DH;
+          const T* kpb = (const T*)p.kp + (size_t)b * p.I * p.ldp + head * DH;
+          const T* vpb = (const T*)p.vp + (size_t)b * p.I * p.ldp + head * DH;
           for (int i = st; i < kN * PPR; i += kStageThreads) {       // content rows: Q, K, V share the (row, part) decode
             const int row = i / PPR, part = i - row * PPR;
             const uint32_t so = (uint32_t)(row * p.ldq + part * 4);
@@ -627,30 +653,30 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
           }
           asm volatile("cp.async.wait_all;" ::: "memory");
         } else {
-          auto stage_q = [&](int t, const __nv_bfloat16 (&row)[DH]) {
+          auto stage_q = [&](int t, const T (&row)[DH]) {
             const int n = t * 128 + st;
             qn2[t] = sumsq_w<DH>(row);
             qn2_s[n] = qn2[t];
             const int id_ = n % p.wd;
-            __nv_bfloat16 extra[4];
+            T extra[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u) extra[u] = (u == id_) ? one : zero;
             store_chunks_w<DH, KS>(Qs, kN * 16, n, row, extra, p.wd);
           };
-          auto stage_k = [&](int j, const __nv_bfloat16 (&row)[DH]) {
+          auto stage_k = [&](int j, const T (&row)[DH]) {
             const bool content = j < kN;
             kmax2 = fmaxf(kmax2, sumsq_w<DH>(row));
             const int jd = j % p.wd;
-            __nv_bfloat16 extra[4];
+            T extra[4];
 #pragma unroll
             for (int u = 0; u < 4; ++u)
-              extra[u] = (content && u < p.wd) ? __float2bfloat16(td_s[u * p.wd + jd] * inv_scale) : zero;
+              extra[u] = (content && u < p.wd) ? from_f32<T>(td_s[u * p.wd + jd] * inv_scale) : zero;
             store_chunks_w<DH, KS>(Ks, NKT * 16, j, row, extra, p.wd);
           };
-          auto stage_v = [&](int j, const __nv_bfloat16 (&row)[DH]) {
+          auto stage_v = [&](int j, const T (&row)[DH]) {
 #pragma unroll
             for (int dc = 0; dc < NDC; ++dc) {
-              __align__(16) __nv_bfloat16 tmp[8];
+              __align__(16) T tmp[8];
 #pragma unroll
               for (int e = 0; e < 8; ++e)
                 tmp[e] = (dc * 8 + e < DH) ? row[dc * 8 + e < DH ? dc * 8 + e : 0] : (dc * 8 + e == DH ? one : zero);
@@ -659,14 +685,14 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
           };
 #pragma unroll
           for (int t = 0; t < 2; ++t) {
-            __nv_bfloat16 row[DH];
-            load_row_w<DH>((const __nv_bfloat16*)p.q + ((size_t)bw * kN + t * 128 + st) * p.ldq + head * DH, row);
+            T row[DH];
+            load_row_w<DH>((const T*)p.q + ((size_t)bw * kN + t * 128 + st) * p.ldq + head * DH, row);
             stage_q(t, row);
           }
           for (int j = st; j < NKT; j += 128) {
-            __nv_bfloat16 row[DH], vrow[DH];
-            load_row_w<DH>((const __nv_bfloat16*)(j < kN ? p.k : p.kp) + kv_off(j), row);
-            load_row_w<DH>((const __nv_bfloat16*)(j < kN ? p.v : p.vp) + kv_off(j), vrow);
+            T row[DH], vrow[DH];
+            load_row_w<DH>((const T*)(j < kN ? p.k : p.kp) + kv_off(j), row);
+            load_row_w<DH>((const T*)(j < kN ? p.v : p.vp) + kv_off(j), vrow);
             stage_k(j, row);
             stage_v(j, vrow);
           }
@@ -683,8 +709,9 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
 #pragma unroll
             for (int part = 0; part < PPR; ++part) {
               const uint2 w = *reinterpret_cast<const uint2*>(base + (part >> 1) * chunk_stride + row * 16 + (part & 1) * 8);
-              const float f0 = __uint_as_float(w.x << 16), f1 = __uint_as_float(w.x & 0xffff0000u);
-              const float f2 = __uint_as_float(w.y << 16), f3 = __uint_as_float(w.y & 0xffff0000u);
+              float f0, f1, f2, f3;
+              unpack2t<T>(w.x, f0, f1);
+              unpack2t<T>(w.y, f2, f3);
               a = fmaf(f0, f0, fmaf(f1, f1, fmaf(f2, f2, fmaf(f3, f3, a))));
             }
             return a;
@@ -727,7 +754,10 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
         for (int t = 0; t < 2; ++t) {
           const float qk = sqrtf(qn2[t]) * kmax, rb = rowb_s[t * 128 + st];
           const float mbt = c2 * 1.01f * (qk + fmaxf(rb, 0.f));
-          loose |= (mbt - c2 * (rb - qk)) > 2.f * kMaxBoundW;
+          // (fp16: in a masked row the key that attains rb may be masked -- its logit is 0 -- so only min(rb - qk, 0) is a
+          // lower bound of the row maximum there)
+          const float lb = (MASKED && WsStab<T>::shift != 0.f) ? fminf(rb - qk, 0.f) : rb - qk;
+          loose |= (mbt - c2 * lb) > WsStab<T>::max_gap;
         }
         if (loose) atomicOr(&hdr->exact, 1);
       }
@@ -752,8 +782,8 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
     {
       const int g = __shfl_sync(0xffffffffu, warp - kIssue0, 0);
       const uint32_t tg = __shfl_sync(0xffffffffu, tmem, 0) + (uint32_t)(g * GC);
-      const uint32_t idescS64 = make_idesc_bf16(128, 64, 0, 0), idescS32 = make_idesc_bf16(128, 32, 0, 0);
-      const uint32_t idescPV = make_idesc_bf16(128, DHP, 0, 1);
+      const uint32_t idescS64 = make_idesc<T>(128, 64, 0, 0), idescS32 = make_idesc<T>(128, 32, 0, 0);
+      const uint32_t idescPV = make_idesc<T>(128, DHP, 0, 1);
       struct Cur {
         int it, pass, u, npass;
         bool stop, need_open;
@@ -868,7 +898,7 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
   if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-template <int DH>
+template <int DH, typename T>
 int launch_ws(const AttnParams& p, cudaStream_t st) {
   constexpr int DHP = WCfg<DH>::DHP, KS = WCfg<DH>::KS;
   const int NKT = kN + p.I;
@@ -879,8 +909,8 @@ int launch_ws(const AttnParams& p, cudaStream_t st) {
   if (grid < p.heads) grid = p.heads;
   const int need = p.B * p.P * p.heads;
   if (grid > need) grid = need;
-  auto kern = p.drop_thresh ? (p.ids ? attn_fwd_ws_kernel<DH, true, true> : attn_fwd_ws_kernel<DH, false, true>)
-                            : (p.ids ? attn_fwd_ws_kernel<DH, true, false> : attn_fwd_ws_kernel<DH, false, false>);
+  auto kern = p.drop_thresh ? (p.ids ? attn_fwd_ws_kernel<DH, true, true, T> : attn_fwd_ws_kernel<DH, false, true, T>)
+                            : (p.ids ? attn_fwd_ws_kernel<DH, true, false, T> : attn_fwd_ws_kernel<DH, false, false, T>);
   PWA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   if (p.work) PWA_CUDA_OK(cudaMemsetAsync(p.work, 0, sizeof(unsigned int) * p.heads, st));
   kern<<<grid, kThreadsW, smem, st>>>(p);
@@ -897,16 +927,21 @@ bool attn_ws_supported(const AttnParams& p, int dtype) {
   return L.total <= 224u * 1024u;
 }
 
-int attn_ws_forward(const AttnParams& p, cudaStream_t st) {
+template <typename T>
+static int ws_forward_t(const AttnParams& p, cudaStream_t st) {
   switch (p.C / p.heads) {
-    case 3: return launch_ws<3>(p, st);
-    case 6: return launch_ws<6>(p, st);
-    case 12: return launch_ws<12>(p, st);
-    case 24: return launch_ws<24>(p, st);
-    case 48: return launch_ws<48>(p, st);
+    case 3: return launch_ws<3, T>(p, st);
+    case 6: return launch_ws<6, T>(p, st);
+    case 12: return launch_ws<12, T>(p, st);
+    case 24: return launch_ws<24, T>(p, st);
+    case 48: return launch_ws<48, T>(p, st);
   }
   set_error("tcgen05 attention: head_dim %d not instantiated", p.C / p.heads);
   return PWA_ERR_UNSUPPORTED;
+}
+
+int attn_ws_forward(const AttnParams& p, int dtype, cudaStream_t st) {
+  return dtype == PWA_F16 ? ws_forward_t<__half>(p, st) : ws_forward_t<__nv_bfloat16>(p, st);
 }
 
 }  // namespace pwa

@@ -88,7 +88,7 @@ static int dropout_launch(const void* x, void* y, int64_t n, float p_drop, const
                           void* stream) {
   PWA_CHECK_ARG(x && y && seed_dev, "pwa_dropout: null pointer");
   PWA_CHECK_ARG(n >= 0 && p_drop >= 0.f && p_drop < 1.f, "pwa_dropout: n=%lld p=%g", (long long)n, (double)p_drop);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_dropout: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_dropout: bad dtype %d", dtype);
   PWA_CHECK_ARG(((uintptr_t)x & 15) == 0 && ((uintptr_t)y & 15) == 0, "pwa_dropout: buffers must be 16-byte aligned");
   if (n == 0) return PWA_OK;
   int t = (int)(p_drop * 256.f + 0.5f);
@@ -104,10 +104,14 @@ static int dropout_launch(const void* x, void* y, int64_t n, float p_drop, const
   if (dtype == PWA_F32) {
     if (colsum) dropout_kernel<float, true><<<(unsigned)blocks, threads, 0, st>>>((const float*)x, (float*)y, (long)n, (uint32_t)t, inv_keep, sd, colsum, C);
     else dropout_kernel<float, false><<<(unsigned)blocks, threads, 0, st>>>((const float*)x, (float*)y, (long)n, (uint32_t)t, inv_keep, sd, nullptr, 0);
-  } else {
+  } else if (dtype == PWA_BF16) {
     using B = __nv_bfloat16;
     if (colsum) dropout_kernel<B, true><<<(unsigned)blocks, threads, 0, st>>>((const B*)x, (B*)y, (long)n, (uint32_t)t, inv_keep, sd, colsum, C);
     else dropout_kernel<B, false><<<(unsigned)blocks, threads, 0, st>>>((const B*)x, (B*)y, (long)n, (uint32_t)t, inv_keep, sd, nullptr, 0);
+  } else {
+    using H = __half;
+    if (colsum) dropout_kernel<H, true><<<(unsigned)blocks, threads, 0, st>>>((const H*)x, (H*)y, (long)n, (uint32_t)t, inv_keep, sd, colsum, C);
+    else dropout_kernel<H, false><<<(unsigned)blocks, threads, 0, st>>>((const H*)x, (H*)y, (long)n, (uint32_t)t, inv_keep, sd, nullptr, 0);
   }
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;

@@ -28,17 +28,26 @@ __device__ __forceinline__ uint32_t add_bf16x2(uint32_t a, uint32_t b) {
   const __nv_bfloat162 r = __floats2bfloat162_rn(fa.x + fb.x, fa.y + fb.y);
   return *reinterpret_cast<const uint32_t*>(&r);
 }
+__device__ __forceinline__ uint32_t add_f16x2(uint32_t a, uint32_t b) {
+  const float2 fa = __half22float2(*reinterpret_cast<const __half2*>(&a));
+  const float2 fb = __half22float2(*reinterpret_cast<const __half2*>(&b));
+  const __half2 r = __floats2half2_rn(fa.x + fb.x, fa.y + fb.y);
+  return *reinterpret_cast<const uint32_t*>(&r);
+}
 __device__ __forceinline__ uint32_t add_f32(uint32_t a, uint32_t b) { return __float_as_uint(__uint_as_float(a) + __uint_as_float(b)); }
 
-template <int EB> __device__ __forceinline__ uint32_t add_w(uint32_t a, uint32_t b) { return EB == 4 ? add_f32(a, b) : add_bf16x2(a, b); }
-
-template <int EB> __device__ __forceinline__ uint4 vadd(uint4 a, uint4 b) {
-  return make_uint4(add_w<EB>(a.x, b.x), add_w<EB>(a.y, b.y), add_w<EB>(a.z, b.z), add_w<EB>(a.w, b.w));
+// EB = element bytes; H: the 16-bit elements are fp16 (else bf16)
+template <int EB, bool H> __device__ __forceinline__ uint32_t add_w(uint32_t a, uint32_t b) {
+  return EB == 4 ? add_f32(a, b) : (H ? add_f16x2(a, b) : add_bf16x2(a, b));
 }
-template <int EB> __device__ __forceinline__ uint2 vadd(uint2 a, uint2 b) { return make_uint2(add_w<EB>(a.x, b.x), add_w<EB>(a.y, b.y)); }
-template <int EB> __device__ __forceinline__ uint32_t vadd(uint32_t a, uint32_t b) { return add_w<EB>(a, b); }
-template <int EB> __device__ __forceinline__ uint16_t vadd(uint16_t a, uint16_t b) {   // one bf16
-  return (uint16_t)(add_bf16x2((uint32_t)a, (uint32_t)b) & 0xffffu);
+
+template <int EB, bool H> __device__ __forceinline__ uint4 vadd(uint4 a, uint4 b) {
+  return make_uint4(add_w<EB, H>(a.x, b.x), add_w<EB, H>(a.y, b.y), add_w<EB, H>(a.z, b.z), add_w<EB, H>(a.w, b.w));
+}
+template <int EB, bool H> __device__ __forceinline__ uint2 vadd(uint2 a, uint2 b) { return make_uint2(add_w<EB, H>(a.x, b.x), add_w<EB, H>(a.y, b.y)); }
+template <int EB, bool H> __device__ __forceinline__ uint32_t vadd(uint32_t a, uint32_t b) { return add_w<EB, H>(a, b); }
+template <int EB, bool H> __device__ __forceinline__ uint16_t vadd(uint16_t a, uint16_t b) {   // one 16-bit element
+  return (uint16_t)(add_w<EB, H>((uint32_t)a, (uint32_t)b) & 0xffffu);
 }
 
 __device__ __forceinline__ void vzero(uint4& v) { v = make_uint4(0, 0, 0, 0); }
@@ -66,7 +75,7 @@ struct Div32 {
 
 // One thread = kUnroll vectors, strided by the grid so that a warp's accesses stay contiguous.
 // vpr = vectors per row; chunk q -> (row, c) with row in [0, B * rows_dst).
-template <int VB, int EB, bool ADD>
+template <int VB, int EB, bool ADD, bool H>
 __global__ void __launch_bounds__(256) gather_rows_kernel(const typename VecT<VB>::type* __restrict__ a,
                                                           const typename VecT<VB>::type* __restrict__ b,
                                                           typename VecT<VB>::type* __restrict__ dst,
@@ -100,11 +109,11 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const typename VecT<VB
     }
 #pragma unroll
     for (int u = 0; u < kUnroll; ++u)
-      if (live[u]) dst[q0 + u * stride] = ADD ? vadd<EB>(va[u], vb[u]) : va[u];
+      if (live[u]) dst[q0 + u * stride] = ADD ? vadd<EB, H>(va[u], vb[u]) : va[u];
   }
 }
 
-template <int VB, int EB>
+template <int VB, int EB, bool H = false>
 int launch_gather(const void* a, const void* b, void* dst, const int32_t* map, int B, long long rows_src, long long rows_dst,
                   int row_bytes, cudaStream_t st) {
   using V = typename VecT<VB>::type;
@@ -118,9 +127,9 @@ int launch_gather(const void* a, const void* b, void* dst, const int32_t* map, i
   const dim3 grid((unsigned)blocks, (unsigned)B);
   const size_t ss = (size_t)rows_src * vpr, ds = (size_t)rows_dst * vpr;
   if (b)
-    gather_rows_kernel<VB, EB, true><<<grid, 256, 0, st>>>((const V*)a, (const V*)b, (V*)dst, map, (uint32_t)total, dv, ss, ds);
+    gather_rows_kernel<VB, EB, true, H><<<grid, 256, 0, st>>>((const V*)a, (const V*)b, (V*)dst, map, (uint32_t)total, dv, ss, ds);
   else
-    gather_rows_kernel<VB, EB, false><<<grid, 256, 0, st>>>((const V*)a, nullptr, (V*)dst, map, (uint32_t)total, dv, ss, ds);
+    gather_rows_kernel<VB, EB, false, false><<<grid, 256, 0, st>>>((const V*)a, nullptr, (V*)dst, map, (uint32_t)total, dv, ss, ds);
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
@@ -135,7 +144,7 @@ extern "C" int pwa_gather_rows(const void* src_a, const void* src_b, void* dst, 
   PWA_CHECK_ARG(src_a && dst && map, "pwa_gather_rows: null pointer");
   PWA_CHECK_ARG(B > 0 && C > 0 && rows_src > 0 && rows_dst > 0, "pwa_gather_rows: bad shape B=%d C=%d rows %lld -> %lld", B, C,
                 (long long)rows_src, (long long)rows_dst);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_gather_rows: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_gather_rows: bad dtype %d", dtype);
   const int eb = dtype == PWA_F32 ? 4 : 2;
   const int row_bytes = C * eb;
   const uintptr_t al = (uintptr_t)src_a | (uintptr_t)src_b | (uintptr_t)dst;
@@ -151,6 +160,14 @@ extern "C" int pwa_gather_rows(const void* src_a, const void* src_b, void* dst, 
       case 16: return launch_gather<16, 4>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
       case 8: return launch_gather<8, 4>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
       default: return launch_gather<4, 4>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
+    }
+  }
+  if (dtype == PWA_F16 && src_b) {                                      // only the fused add depends on the 16-bit format
+    switch (vb) {
+      case 16: return launch_gather<16, 2, true>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
+      case 8: return launch_gather<8, 2, true>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
+      case 4: return launch_gather<4, 2, true>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
+      default: return launch_gather<2, 2, true>(src_a, src_b, dst, map, B, rows_src, rows_dst, row_bytes, st);
     }
   }
   switch (vb) {

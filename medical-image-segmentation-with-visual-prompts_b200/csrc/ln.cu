@@ -14,8 +14,8 @@ namespace pwa {
 
 constexpr int kLnThreads = 256;
 
-// 16-byte lane vectors where the row length allows (8 bf16 / 4 fp32), else 8-byte (4 bf16)
-template <typename T, int EPV> struct Vec;
+// 16-byte lane vectors where the row length allows (8 bf16 or fp16 / 4 fp32), else 8-byte (4 bf16 or fp16)
+template <typename T, int EPV> struct Vec;      // 16-bit T (bf16, fp16) below; fp32 specialised
 template <> struct Vec<float, 4> {
   static __device__ __forceinline__ void load(const float* p, float (&v)[4]) {
     const float4 t = __ldg(reinterpret_cast<const float4*>(p));
@@ -25,34 +25,45 @@ template <> struct Vec<float, 4> {
     *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
   }
 };
-__device__ __forceinline__ void unpack2(uint32_t w, float& a, float& b) {
+template <typename T> __device__ __forceinline__ void unpack2(uint32_t w, float& a, float& b);
+template <> __device__ __forceinline__ void unpack2<__nv_bfloat16>(uint32_t w, float& a, float& b) {
   a = __uint_as_float(w << 16);
   b = __uint_as_float(w & 0xffff0000u);
 }
-__device__ __forceinline__ uint32_t pack2(float a, float b) {
+template <> __device__ __forceinline__ void unpack2<__half>(uint32_t w, float& a, float& b) {
+  const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&w));
+  a = f.x;
+  b = f.y;
+}
+template <typename T> __device__ __forceinline__ uint32_t pack2(float a, float b);
+template <> __device__ __forceinline__ uint32_t pack2<__nv_bfloat16>(float a, float b) {
   const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
   return *reinterpret_cast<const uint32_t*>(&v);
 }
-template <> struct Vec<__nv_bfloat16, 4> {
-  static __device__ __forceinline__ void load(const __nv_bfloat16* p, float (&v)[4]) {
+template <> __device__ __forceinline__ uint32_t pack2<__half>(float a, float b) {
+  const __half2 v = __floats2half2_rn(a, b);
+  return *reinterpret_cast<const uint32_t*>(&v);
+}
+template <typename T> struct Vec<T, 4> {
+  static __device__ __forceinline__ void load(const T* p, float (&v)[4]) {
     const uint2 t = __ldg(reinterpret_cast<const uint2*>(p));
-    unpack2(t.x, v[0], v[1]);
-    unpack2(t.y, v[2], v[3]);
+    unpack2<T>(t.x, v[0], v[1]);
+    unpack2<T>(t.y, v[2], v[3]);
   }
-  static __device__ __forceinline__ void store(__nv_bfloat16* p, const float (&v)[4]) {
-    *reinterpret_cast<uint2*>(p) = make_uint2(pack2(v[0], v[1]), pack2(v[2], v[3]));
+  static __device__ __forceinline__ void store(T* p, const float (&v)[4]) {
+    *reinterpret_cast<uint2*>(p) = make_uint2(pack2<T>(v[0], v[1]), pack2<T>(v[2], v[3]));
   }
 };
-template <> struct Vec<__nv_bfloat16, 8> {
-  static __device__ __forceinline__ void load(const __nv_bfloat16* p, float (&v)[8]) {
+template <typename T> struct Vec<T, 8> {
+  static __device__ __forceinline__ void load(const T* p, float (&v)[8]) {
     const uint4 t = __ldg(reinterpret_cast<const uint4*>(p));
-    unpack2(t.x, v[0], v[1]);
-    unpack2(t.y, v[2], v[3]);
-    unpack2(t.z, v[4], v[5]);
-    unpack2(t.w, v[6], v[7]);
+    unpack2<T>(t.x, v[0], v[1]);
+    unpack2<T>(t.y, v[2], v[3]);
+    unpack2<T>(t.z, v[4], v[5]);
+    unpack2<T>(t.w, v[6], v[7]);
   }
-  static __device__ __forceinline__ void store(__nv_bfloat16* p, const float (&v)[8]) {
-    *reinterpret_cast<uint4*>(p) = make_uint4(pack2(v[0], v[1]), pack2(v[2], v[3]), pack2(v[4], v[5]), pack2(v[6], v[7]));
+  static __device__ __forceinline__ void store(T* p, const float (&v)[8]) {
+    *reinterpret_cast<uint4*>(p) = make_uint4(pack2<T>(v[0], v[1]), pack2<T>(v[2], v[3]), pack2<T>(v[4], v[5]), pack2<T>(v[6], v[7]));
   }
 };
 template <int EPV> __device__ __forceinline__ void loadf(const float* p, float (&v)[EPV]) {
@@ -299,7 +310,7 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 8 ? 4 : (NV * EPV
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// Bulk-copy variants (bf16, one 16-byte vector per lane): the register kernels above keep one row per lane group in
+// Bulk-copy variants (bf16 / fp16, one 16-byte vector per lane): the register kernels above keep one row per lane group in
 // flight, i.e. 16-48 bytes per thread, and at 4 CTAs/SM (56-64 registers) that is 16-48 KB per SM -- Little's law
 // wants ~45 KB for the measured 6.6 TB/s, and the plain forward sat at 2.9 TB/s.  Here the operand tiles of a CTA
 // iteration (256/G consecutive rows = one contiguous 3-4 KB chunk per operand) are fetched by cp.async.bulk into a
@@ -329,23 +340,24 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src, uint32
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                    ln_smem_u32(dst_smem)), "l"(src), "r"(bytes), "r"(ln_smem_u32(bar)) : "memory");
 }
-__device__ __forceinline__ void lds_vec8(const __nv_bfloat16* p, float (&v)[8]) {
+template <typename T>
+__device__ __forceinline__ void lds_vec8(const T* p, float (&v)[8]) {
   const uint4 t = *reinterpret_cast<const uint4*>(p);
-  unpack2(t.x, v[0], v[1]);
-  unpack2(t.y, v[2], v[3]);
-  unpack2(t.z, v[4], v[5]);
-  unpack2(t.w, v[6], v[7]);
+  unpack2<T>(t.x, v[0], v[1]);
+  unpack2<T>(t.y, v[2], v[3]);
+  unpack2<T>(t.z, v[4], v[5]);
+  unpack2<T>(t.w, v[6], v[7]);
 }
 
 // ring of `stages` buffers, each holding `nop` operand tiles of GPB rows; tile t of this CTA = blockIdx.x + t * gridDim.x
-template <int GPB>
+template <int GPB, typename T>
 struct BulkRing {
   uint8_t* buf;
   uint64_t* full;
   uint32_t tile_bytes;      // GPB * C * 2
   int nop, C, stages;
   long rows, n_tiles;
-  const __nv_bfloat16* src[3];
+  const T* src[3];
   __device__ __forceinline__ void issue(long tile, int s) const {      // one thread
     const long row0 = tile * GPB;
     const long left = rows - row0;
@@ -353,27 +365,26 @@ struct BulkRing {
     ln_mbar_expect_tx(&full[s], bytes * nop);
     for (int o = 0; o < nop; ++o) bulk_g2s(buf + ((size_t)s * nop + o) * tile_bytes, src[o] + row0 * C, bytes, &full[s]);
   }
-  __device__ __forceinline__ const __nv_bfloat16* tile(int s, int o) const {
-    return reinterpret_cast<const __nv_bfloat16*>(buf + ((size_t)s * nop + o) * tile_bytes);
+  __device__ __forceinline__ const T* tile(int s, int o) const {
+    return reinterpret_cast<const T*>(buf + ((size_t)s * nop + o) * tile_bytes);
   }
 };
 
 // R rows per lane group and iteration (tile = R * 256/G rows): the per-iteration overhead (mbarrier wait, block barrier,
 // refill, addressing, loop) is paid once per R rows, and the shuffle reductions of the R rows interleave.
-template <int G, int R>
-__global__ void __launch_bounds__(kLnThreads, R == 1 ? 4 : 3) ln_fwd_bulk_kernel(const __nv_bfloat16* __restrict__ x, const __nv_bfloat16* __restrict__ res,
+template <int G, int R, typename T>
+__global__ void __launch_bounds__(kLnThreads, R == 1 ? 4 : 3) ln_fwd_bulk_kernel(const T* __restrict__ x, const T* __restrict__ res,
                                                                     const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                                    __nv_bfloat16* __restrict__ sum_out, __nv_bfloat16* __restrict__ y,
+                                                                    T* __restrict__ sum_out, T* __restrict__ y,
                                                                     float* __restrict__ mean_out, float* __restrict__ rstd_out,
                                                                     long rows, int C, float eps) {
-  using T = __nv_bfloat16;
   constexpr int GPB = kLnThreads / G, TR = GPB * R, EPV = 8;
   extern __shared__ __align__(128) uint8_t ln_sm[];
   __shared__ __align__(8) uint64_t full[kMaxStages];
   const int gl = threadIdx.x % G, gr = threadIdx.x / G;
   const int nvec = C / EPV;
   const bool has_res = res != nullptr;
-  BulkRing<TR> ring;
+  BulkRing<TR, T> ring;
   ring.buf = ln_sm; ring.full = full; ring.tile_bytes = (uint32_t)TR * C * 2u; ring.nop = has_res ? 2 : 1; ring.C = C;
   ring.stages = kMaxStages / ring.nop / R;
   ring.rows = rows; ring.n_tiles = (rows + TR - 1) / TR;
@@ -407,8 +418,8 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 4 : 3) ln_fwd_bulk_kernel
 #pragma unroll
       for (int e = 0; e < EPV; ++e) v[r][e] = rr[r][e] = 0.f;
       if (lane_live && row0 + r * GPB < rows) {
-        lds_vec8(ring.tile(s, 0) + (r * GPB + gr) * C + gl * EPV, v[r]);
-        if (has_res) lds_vec8(ring.tile(s, 1) + (r * GPB + gr) * C + gl * EPV, rr[r]);
+        lds_vec8<T>(ring.tile(s, 0) + (r * GPB + gr) * C + gl * EPV, v[r]);
+        if (has_res) lds_vec8<T>(ring.tile(s, 1) + (r * GPB + gr) * C + gl * EPV, rr[r]);
       }
     }
     __syncthreads();                                    // every lane holds its vectors: the buffer can be refilled
@@ -468,14 +479,13 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 4 : 3) ln_fwd_bulk_kernel
   }
 }
 
-template <int G, int R>
-__global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel(const __nv_bfloat16* __restrict__ dy, const __nv_bfloat16* __restrict__ x,
+template <int G, int R, typename T>
+__global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel(const T* __restrict__ dy, const T* __restrict__ x,
                                                                     const float* __restrict__ gamma, const float* __restrict__ mean_in,
-                                                                    const float* __restrict__ rstd_in, const __nv_bfloat16* __restrict__ dres,
-                                                                    __nv_bfloat16* __restrict__ dx, float* __restrict__ dgamma,
+                                                                    const float* __restrict__ rstd_in, const T* __restrict__ dres,
+                                                                    T* __restrict__ dx, float* __restrict__ dgamma,
                                                                     float* __restrict__ dbeta, float* __restrict__ dres_colsum,
                                                                     float* __restrict__ dx_colsum, long rows, int C) {
-  using T = __nv_bfloat16;
   constexpr int GPB = kLnThreads / G, TR = GPB * R, EPV = 8;
   extern __shared__ __align__(128) uint8_t ln_sm[];
   __shared__ __align__(8) uint64_t full[kMaxStages];
@@ -483,7 +493,7 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel
   const int nvec = C / EPV;
   const bool has_res = dres != nullptr;
   const bool want_rs = dres_colsum != nullptr && has_res, want_xs = dx_colsum != nullptr;
-  BulkRing<TR> ring;
+  BulkRing<TR, T> ring;
   ring.buf = ln_sm; ring.full = full; ring.tile_bytes = (uint32_t)TR * C * 2u; ring.nop = has_res ? 3 : 2; ring.C = C;
   ring.stages = kMaxStages / ring.nop / R;
   ring.rows = rows; ring.n_tiles = (rows + TR - 1) / TR;
@@ -523,9 +533,9 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel
 #pragma unroll
       for (int e = 0; e < EPV; ++e) d[r][e] = xv[r][e] = rs[r][e] = 0.f;
       if (lane_live && row0 + r * GPB < rows) {
-        lds_vec8(ring.tile(s, 0) + (r * GPB + gr) * C + gl * EPV, d[r]);
-        lds_vec8(ring.tile(s, 1) + (r * GPB + gr) * C + gl * EPV, xv[r]);
-        if (has_res) lds_vec8(ring.tile(s, 2) + (r * GPB + gr) * C + gl * EPV, rs[r]);
+        lds_vec8<T>(ring.tile(s, 0) + (r * GPB + gr) * C + gl * EPV, d[r]);
+        lds_vec8<T>(ring.tile(s, 1) + (r * GPB + gr) * C + gl * EPV, xv[r]);
+        if (has_res) lds_vec8<T>(ring.tile(s, 2) + (r * GPB + gr) * C + gl * EPV, rs[r]);
       }
     }
     __syncthreads();
@@ -660,9 +670,8 @@ static int ln_launch(bool fwd, const LnArgs& a, cudaStream_t st) {
   return PWA_OK;
 }
 
-template <int G, int R>
+template <int G, int R, typename T>
 static int ln_launch_bulk_r(bool fwd, const LnArgs& a, cudaStream_t st) {
-  using T = __nv_bfloat16;
   constexpr int TR = kLnThreads / G * R;
   const int nop = fwd ? (a.res ? 2 : 1) : (a.res ? 3 : 2);
   // (backward epilogue: the per-warp column sums, 8 x 4 x C floats, reuse the ring memory: >= 192 * C bytes for every G, R)
@@ -673,24 +682,24 @@ static int ln_launch_bulk_r(bool fwd, const LnArgs& a, cudaStream_t st) {
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
   if (fwd) {
-    PWA_CUDA_OK(cudaFuncSetAttribute(ln_fwd_bulk_kernel<G, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ln_fwd_bulk_kernel<G, R><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm, (T*)a.o1,
+    PWA_CUDA_OK(cudaFuncSetAttribute(ln_fwd_bulk_kernel<G, R, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ln_fwd_bulk_kernel<G, R, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm, (T*)a.o1,
                                                                          (T*)a.o2, a.f1, a.f2, a.rows, a.C, a.eps);
   } else {
-    PWA_CUDA_OK(cudaFuncSetAttribute(ln_bwd_bulk_kernel<G, R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ln_bwd_bulk_kernel<G, R><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.b, a.gamma, a.bm, a.rstd,
+    PWA_CUDA_OK(cudaFuncSetAttribute(ln_bwd_bulk_kernel<G, R, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ln_bwd_bulk_kernel<G, R, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.b, a.gamma, a.bm, a.rstd,
                                                                          (const T*)a.res, (T*)a.o1, a.f1, a.f2, a.f3, a.f4, a.rows, a.C);
   }
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
 
-template <int G>
+template <int G, typename T>
 static int ln_launch_bulk(bool fwd, const LnArgs& a, cudaStream_t st) {
   // measured (tools/bench_ln.py): R = 2 is 8-13 % faster in backward, within +-5 % in forward
   static const int rf = env_int("PWA_LN_BULK_RF", 1), rb = env_int("PWA_LN_BULK_RB", 2);
-  if ((fwd ? rf : rb) == 2) return ln_launch_bulk_r<G, 2>(fwd, a, st);
-  return ln_launch_bulk_r<G, 1>(fwd, a, st);
+  if ((fwd ? rf : rb) == 2) return ln_launch_bulk_r<G, 2, T>(fwd, a, st);
+  return ln_launch_bulk_r<G, 1, T>(fwd, a, st);
 }
 
 template <typename T, int EPV>
@@ -700,10 +709,10 @@ static int ln_dispatch_v(bool fwd, const LnArgs& a, cudaStream_t st) {
     // one vector per lane, rows contiguous: the bulk-copy kernels (PWA_LN_BULK=0 selects the register kernels)
     static const int use_bulk = env_int("PWA_LN_BULK", 1);
     if (use_bulk && nvec <= 32) {
-      if (nvec <= 4) return ln_launch_bulk<4>(fwd, a, st);
-      if (nvec <= 8) return ln_launch_bulk<8>(fwd, a, st);
-      if (nvec <= 16) return ln_launch_bulk<16>(fwd, a, st);
-      return ln_launch_bulk<32>(fwd, a, st);
+      if (nvec <= 4) return ln_launch_bulk<4, T>(fwd, a, st);
+      if (nvec <= 8) return ln_launch_bulk<8, T>(fwd, a, st);
+      if (nvec <= 16) return ln_launch_bulk<16, T>(fwd, a, st);
+      return ln_launch_bulk<32, T>(fwd, a, st);
     }
   }
   const int R = env_int(fwd ? "PWA_LN_RF" : "PWA_LN_RB", 1);       // rows per group per iteration (tuning knob)
@@ -748,10 +757,11 @@ extern "C" int pwa_ln_fwd(const void* x, const void* res, const float* gamma, co
   PWA_CHECK_ARG(x && gamma && beta && y && mean && rstd, "pwa_ln_fwd: null pointer");
   PWA_CHECK_ARG(res == nullptr || sum_out != nullptr, "pwa_ln_fwd: residual given without sum_out");
   PWA_CHECK_ARG(rows >= 0 && C > 0 && C % 4 == 0 && C <= 2048, "pwa_ln_fwd: need C %% 4 == 0, C <= 2048 (C=%d)", C);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_ln_fwd: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_ln_fwd: bad dtype %d", dtype);
   if (rows == 0) return PWA_OK;
   cudaStream_t st = (cudaStream_t)stream;
   LnArgs a = {x, nullptr, res, gamma, beta, nullptr, sum_out, y, mean, rstd, nullptr, nullptr, (long)rows, C, eps};
+  if (dtype == PWA_F16) return ln_dispatch<__half>(true, a, st);
   return dtype == PWA_F32 ? ln_dispatch<float>(true, a, st) : ln_dispatch<__nv_bfloat16>(true, a, st);
 }
 
@@ -760,7 +770,7 @@ extern "C" int pwa_ln_bwd2(const void* dy, const void* x, const float* gamma, co
                            int64_t rows, int C, int dtype, void* stream) {
   PWA_CHECK_ARG(dy && x && gamma && mean && rstd && dx && dgamma && dbeta, "pwa_ln_bwd: null pointer");
   PWA_CHECK_ARG(rows >= 0 && C > 0 && C % 4 == 0 && C <= 2048, "pwa_ln_bwd: need C %% 4 == 0, C <= 2048 (C=%d)", C);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_ln_bwd: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_ln_bwd: bad dtype %d", dtype);
   PWA_CHECK_ARG(dres_colsum == nullptr || dres != nullptr, "pwa_ln_bwd: dres_colsum without dres");
   cudaStream_t st = (cudaStream_t)stream;
   PWA_CUDA_OK(cudaMemsetAsync(dgamma, 0, (size_t)C * 4, st));
@@ -769,6 +779,7 @@ extern "C" int pwa_ln_bwd2(const void* dy, const void* x, const float* gamma, co
   if (dx_colsum) PWA_CUDA_OK(cudaMemsetAsync(dx_colsum, 0, (size_t)C * 4, st));
   if (rows == 0) return PWA_OK;
   LnArgs a = {dy, x, dres, gamma, mean, rstd, dx, nullptr, dgamma, dbeta, dres_colsum, dx_colsum, (long)rows, C, 0.f};
+  if (dtype == PWA_F16) return ln_dispatch<__half>(false, a, st);
   return dtype == PWA_F32 ? ln_dispatch<float>(false, a, st) : ln_dispatch<__nv_bfloat16>(false, a, st);
 }
 

@@ -22,7 +22,7 @@
 namespace pwa {
 
 int partition_tma_run(bool is_partition, const void* src, const void* src2, void* dst, int B, int C, const pwa_geom* g,
-                      const int32_t* lo, int eb, cudaStream_t st);   // partition_tma.cu
+                      const int32_t* lo, int eb, bool f16, cudaStream_t st);   // partition_tma.cu
 
 struct PartParams {
   int B, C;
@@ -73,6 +73,9 @@ template <> __device__ __forceinline__ uint16_t add_elem<uint16_t>(uint16_t a, u
   const float fa = __uint_as_float((uint32_t)a << 16), fb = __uint_as_float((uint32_t)b << 16);
   const __nv_bfloat16 r = __float2bfloat16_rn(fa + fb);
   return *reinterpret_cast<const uint16_t*>(&r);
+}
+template <> __device__ __forceinline__ __half add_elem<__half>(__half a, __half b) {
+  return __float2half_rn(__half2float(a) + __half2float(b));
 }
 
 template <typename T>
@@ -125,10 +128,15 @@ struct Slab {
   }
 };
 
-// word-wise add of two token words: one fp32 or a pair of bf16 (computed in fp32, rounded once: same as torch)
-template <int EB>
+// word-wise add of two token words: one fp32 or a pair of bf16 / fp16 (H) (computed in fp32, rounded once: same as torch)
+template <int EB, bool H = false>
 __device__ __forceinline__ uint32_t add_word(uint32_t a, uint32_t b) {
   if (EB == 4) return __float_as_uint(__uint_as_float(a) + __uint_as_float(b));
+  if (H) {
+    const float2 fx = __half22float2(*reinterpret_cast<const __half2*>(&a)), fy = __half22float2(*reinterpret_cast<const __half2*>(&b));
+    const __half2 r = __floats2half2_rn(fx.x + fy.x, fx.y + fy.y);
+    return *reinterpret_cast<const uint32_t*>(&r);
+  }
   const __nv_bfloat162 x = *reinterpret_cast<const __nv_bfloat162*>(&a), y = *reinterpret_cast<const __nv_bfloat162*>(&b);
   const float2 fx = __bfloat1622float2(x), fy = __bfloat1622float2(y);
   const __nv_bfloat162 r = __floats2bfloat162_rn(fx.x + fy.x, fx.y + fy.y);
@@ -214,7 +222,7 @@ __global__ void __launch_bounds__(256) partition_fast_kernel(const uint32_t* __r
   }
 }
 
-template <int EB>
+template <int EB, bool H>
 __global__ void __launch_bounds__(256) reverse_fast_kernel(const uint32_t* __restrict__ tok, const uint32_t* __restrict__ tok2,
                                                            uint32_t* __restrict__ x, PartParams p) {
   extern __shared__ uint32_t smem[];
@@ -241,7 +249,7 @@ __global__ void __launch_bounds__(256) reverse_fast_kernel(const uint32_t* __res
       p.div_wd.divmod(rem, t2, t3);
       size_t g = ((win0 + p3) * p.N + row0 + rem) * tok_stride_w + cw0 + cw;
       uint32_t v = __ldg(tok + g);
-      if (tok2) v = add_word<EB>(v, __ldg(tok2 + g));
+      if (tok2) v = add_word<EB, H>(v, __ldg(tok2 + g));
       smem[(t2 * p.Dp + t3 * p.P3 + p3) * p.pitch + cw] = v;
     }
   }
@@ -395,7 +403,7 @@ __global__ void __launch_bounds__(256) partition_vec_kernel(const uint32_t* __re
   }
 }
 
-template <int EB>
+template <int EB, bool H>
 __global__ void __launch_bounds__(256) reverse_vec_kernel(const uint32_t* __restrict__ tok, const uint32_t* __restrict__ tok2,
                                                           uint32_t* __restrict__ x, PartParams p) {
   using V = VecCfg<EB>;
@@ -422,7 +430,7 @@ __global__ void __launch_bounds__(256) reverse_vec_kernel(const uint32_t* __rest
       for (int k = 0; k < kTokK; ++k)
         if (k < m.nk && m.soff[k] >= 0) {
           uint32_t v = __ldg(gb + m.goff[k]);
-          if (tok2) v = add_word<EB>(v, __ldg(tok2 + goff0 + m.goff[k]));
+          if (tok2) v = add_word<EB, H>(v, __ldg(tok2 + goff0 + m.goff[k]));
           sb[m.soff[k]] = v;
         }
     }
@@ -519,7 +527,7 @@ static int fill_params(PartParams& p, int B, int C, const pwa_geom* g, int use_c
   return 0;
 }
 
-template <int EB>
+template <int EB, bool H = false>
 static int launch_vec(bool is_partition, const void* src, const void* src2, void* dst, const PartParams& p, cudaStream_t st) {
   size_t smem = (size_t)p.ww * p.Dp * p.pitch * 4;
   dim3 grid((unsigned)((size_t)p.B * p.Hp * p.P2 * p.nchunk));
@@ -529,14 +537,14 @@ static int launch_vec(bool is_partition, const void* src, const void* src2, void
     partition_vec_kernel<EB><<<grid, 256, smem, st>>>((const uint32_t*)src, (uint32_t*)dst, p);
   } else {
     // (the attribute is per DEVICE: set it on every launch -- cheap, capture-safe, correct for one process driving several GPUs)
-    PWA_CUDA_OK(cudaFuncSetAttribute(reverse_vec_kernel<EB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    reverse_vec_kernel<EB><<<grid, 256, smem, st>>>((const uint32_t*)src, (const uint32_t*)src2, (uint32_t*)dst, p);
+    PWA_CUDA_OK(cudaFuncSetAttribute(reverse_vec_kernel<EB, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    reverse_vec_kernel<EB, H><<<grid, 256, smem, st>>>((const uint32_t*)src, (const uint32_t*)src2, (uint32_t*)dst, p);
   }
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
 
-template <int EB>
+template <int EB, bool H = false>
 static int launch_fast(bool is_partition, const void* src, const void* src2, void* dst, const PartParams& p, cudaStream_t st) {
   size_t smem = (size_t)p.ww * p.Dp * p.pitch * 4;
   dim3 grid((unsigned)((size_t)p.B * p.Hp * p.P2 * p.nchunk));
@@ -546,14 +554,14 @@ static int launch_fast(bool is_partition, const void* src, const void* src2, voi
     partition_fast_kernel<EB><<<grid, 256, smem, st>>>((const uint32_t*)src, (uint32_t*)dst, p);
   } else {
     // (the attribute is per DEVICE: set it on every launch -- cheap, capture-safe, correct for one process driving several GPUs)
-    PWA_CUDA_OK(cudaFuncSetAttribute(reverse_fast_kernel<EB>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    reverse_fast_kernel<EB><<<grid, 256, smem, st>>>((const uint32_t*)src, (const uint32_t*)src2, (uint32_t*)dst, p);
+    PWA_CUDA_OK(cudaFuncSetAttribute(reverse_fast_kernel<EB, H>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    reverse_fast_kernel<EB, H><<<grid, 256, smem, st>>>((const uint32_t*)src, (const uint32_t*)src2, (uint32_t*)dst, p);
   }
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
 
-template <typename T>
+template <typename T, typename TA = T>
 static int launch_generic(bool is_partition, const void* src, const void* src2, void* dst, const PartParams& p, cudaStream_t st) {
   size_t total = is_partition ? (size_t)p.B * p.P * p.N * p.C : (size_t)p.B * p.C * p.H * p.W * p.D;
   if (total == 0) return PWA_OK;
@@ -562,7 +570,7 @@ static int launch_generic(bool is_partition, const void* src, const void* src2, 
   if (is_partition)
     partition_generic_kernel<T><<<blocks, 256, 0, st>>>((const T*)src, (T*)dst, p, total);
   else
-    reverse_generic_kernel<T><<<blocks, 256, 0, st>>>((const T*)src, (const T*)src2, (T*)dst, p, total);
+    reverse_generic_kernel<TA><<<blocks, 256, 0, st>>>((const TA*)src, (const TA*)src2, (TA*)dst, p, total);
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
@@ -571,7 +579,7 @@ static int run(bool is_partition, const void* src, const void* src2, void* dst, 
                int use_crop_lo, int dtype, void* stream) {
   PWA_CHECK_ARG(src && dst && g, "pwa_partition/reverse: null pointer");
   PWA_CHECK_ARG(B > 0 && C > 0, "pwa_partition/reverse: bad B=%d C=%d", B, C);
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_partition/reverse: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_partition/reverse: bad dtype %d", dtype);
   const int eb = dtype == PWA_F32 ? 4 : 2;
   PartParams p;
   bool fast = false, vec = false;
@@ -582,7 +590,7 @@ static int run(bool is_partition, const void* src, const void* src2, void* dst, 
   static const bool no_tma = getenv("PWA_NO_TMA") != nullptr;
   if (!(use_crop_lo & (2 | 4 | 8)) && !no_tma) {
     const int32_t* lo = (use_crop_lo & 1) ? g->crop_lo : g->data_lo;
-    const int rc = partition_tma_run(is_partition, src, src2, dst, B, C, g, lo, eb, st0);
+    const int rc = partition_tma_run(is_partition, src, src2, dst, B, C, g, lo, eb, dtype == PWA_F16, st0);
     if (rc != PWA_ERR_UNSUPPORTED) return rc;
   }
   if (use_crop_lo & 2) fast = vec = false;
@@ -590,6 +598,11 @@ static int run(bool is_partition, const void* src, const void* src2, void* dst, 
   if (((uintptr_t)src | (uintptr_t)src2 | (uintptr_t)dst) & 3) fast = false;   // staged paths move aligned 32-bit words
   if (((uintptr_t)src | (uintptr_t)src2 | (uintptr_t)dst) & 15) vec = false;   // ... or aligned 16-byte vectors
   cudaStream_t st = (cudaStream_t)stream;
+  if (dtype == PWA_F16 && src2) {                        // only the fused add of reverse_add depends on the 16-bit format
+    if (fast && vec) return launch_vec<2, true>(false, src, src2, dst, p, st);
+    if (fast) return launch_fast<2, true>(false, src, src2, dst, p, st);
+    return launch_generic<uint16_t, __half>(false, src, src2, dst, p, st);
+  }
   if (fast && vec) return eb == 4 ? launch_vec<4>(is_partition, src, src2, dst, p, st) : launch_vec<2>(is_partition, src, src2, dst, p, st);
   if (fast) return eb == 4 ? launch_fast<4>(is_partition, src, src2, dst, p, st) : launch_fast<2>(is_partition, src, src2, dst, p, st);
   return eb == 4 ? launch_generic<uint32_t>(is_partition, src, src2, dst, p, st)

@@ -277,15 +277,20 @@ __global__ void __launch_bounds__(kPartThreads, 4) partition_tma_kernel(const __
   }
 }
 
-template <int EB> __device__ __forceinline__ uint32_t addw(uint32_t a, uint32_t b) {
+template <int EB, bool H> __device__ __forceinline__ uint32_t addw(uint32_t a, uint32_t b) {
   if (EB == 4) return __float_as_uint(__uint_as_float(a) + __uint_as_float(b));
+  if (H) {                                                   // fp16 pair
+    const float2 fa = __half22float2(*reinterpret_cast<const __half2*>(&a)), fb = __half22float2(*reinterpret_cast<const __half2*>(&b));
+    const __half2 r = __floats2half2_rn(fa.x + fb.x, fa.y + fb.y);
+    return *reinterpret_cast<const uint32_t*>(&r);
+  }
   const float2 fa = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&a));
   const float2 fb = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&b));
   const __nv_bfloat162 r = __floats2bfloat162_rn(fa.x + fb.x, fa.y + fb.y);
   return *reinterpret_cast<const uint32_t*>(&r);
 }
 
-template <int EB, bool ADD>
+template <int EB, bool ADD, bool H = false>
 __global__ void __launch_bounds__(kRevThreads, 4) reverse_tma_kernel(const __grid_constant__ CUtensorMap xmap,
                                                                   const uint32_t* __restrict__ tok,
                                                                   const uint32_t* __restrict__ tok2, const TmaPartParams p) {
@@ -315,7 +320,7 @@ __global__ void __launch_bounds__(kRevThreads, 4) reverse_tma_kernel(const __gri
       for (int u = 0; u < U; ++u) {
         const uint32_t i = i0 + u * kRevThreads;
         if (i < npieces) {
-          if (ADD) v[u] = make_uint4(addw<EB>(v[u].x, w[u].x), addw<EB>(v[u].y, w[u].y), addw<EB>(v[u].z, w[u].z), addw<EB>(v[u].w, w[u].w));
+          if (ADD) v[u] = make_uint4(addw<EB, H>(v[u].x, w[u].x), addw<EB, H>(v[u].y, w[u].y), addw<EB, H>(v[u].z, w[u].z), addw<EB, H>(v[u].w, w[u].w));
           *reinterpret_cast<uint4*>(cv.dst + pc[u].soff) = v[u];
         }
       }
@@ -441,7 +446,7 @@ bool set_smem(K kern, size_t bytes) {
 // Returns PWA_OK when the TMA kernel was launched, PWA_ERR_UNSUPPORTED when the shape is outside its envelope (the
 // caller then uses the vector / word / generic kernels of partition.cu), another error code on failure.
 int partition_tma_run(bool is_partition, const void* src, const void* src2, void* dst, int B, int C, const pwa_geom* g,
-                      const int32_t* lo, int eb, cudaStream_t st) {
+                      const int32_t* lo, int eb, bool f16, cudaStream_t st) {
   TmaPartParams p;
   // TMA stores fault on negative start coordinates (measured on B200, driver 580): padded geometries, whose crop
   // needs them, keep the vector kernel on the store side; loads zero-fill out-of-bounds boxes as documented
@@ -470,10 +475,11 @@ int partition_tma_run(bool is_partition, const void* src, const void* src2, void
       if (ok) partition_tma_kernel<4><<<grid, kPartThreads, smem, st>>>(map, (uint32_t*)dst, p);
     }
   } else {
-#define PWA_REV(EBV, ADDV)                                                                                              \
-  ok = set_smem(reverse_tma_kernel<EBV, ADDV>, smem);                                                                    \
-  if (ok) reverse_tma_kernel<EBV, ADDV><<<grid, kRevThreads, smem, st>>>(map, (const uint32_t*)src, (const uint32_t*)src2, p)
-    if (eb == 2 && src2) { PWA_REV(2, true); }
+#define PWA_REV(EBV, ...)                                                                                               \
+  ok = set_smem(reverse_tma_kernel<EBV, __VA_ARGS__>, smem);                                                             \
+  if (ok) reverse_tma_kernel<EBV, __VA_ARGS__><<<grid, kRevThreads, smem, st>>>(map, (const uint32_t*)src, (const uint32_t*)src2, p)
+    if (eb == 2 && src2 && f16) { PWA_REV(2, true, true); }
+    else if (eb == 2 && src2) { PWA_REV(2, true); }
     else if (eb == 2) { PWA_REV(2, false); }
     else if (src2) { PWA_REV(4, true); }
     else { PWA_REV(4, false); }

@@ -32,7 +32,7 @@ __global__ void __launch_bounds__(32 * kRowGroups) colsum_f32_kernel(const float
   }
 }
 
-// Column sums of a token matrix: dst[c] = sum_r x[r][c], x [rows][C] bf16 or fp32, dst fp32.  This is the bias gradient of
+// Column sums of a token matrix: dst[c] = sum_r x[r][c], x [rows][C] bf16, fp16 or fp32, dst fp32.  This is the bias gradient of
 // the q|k|v projection (reference window_attention.py:28-30: three nn.Linear with bias; torch autograd sums dy over the
 // tokens there): dy = the packed dq|dk|dv rows the attention backward kernel wrote, 127 MB at the first stage.  torch's
 // generic reduction needed 36-62 us per call for it (0.5-2.3 TB/s).  blockDim is a multiple of the 16-byte vectors per
@@ -90,8 +90,8 @@ extern "C" int pwa_colsum_f32(const float* src, float* dst, int S, int64_t n, vo
 
 extern "C" int pwa_colsum_rows(const void* x, float* dst, int64_t rows, int C, int dtype, void* stream) {
   PWA_CHECK_ARG(x != nullptr && dst != nullptr, "pwa_colsum_rows: null pointer");
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16, "pwa_colsum_rows: bad dtype %d", dtype);
-  const int E = dtype == PWA_BF16 ? 8 : 4;
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_colsum_rows: bad dtype %d", dtype);
+  const int E = dtype == PWA_F32 ? 4 : 8;
   PWA_CHECK_ARG(rows >= 0 && C >= E && C % E == 0 && C / E <= 512, "pwa_colsum_rows: rows=%lld C=%d (need C %% %d == 0, C <= %d)",
                 (long long)rows, C, E, 512 * E);
   PWA_CHECK_ARG(((uintptr_t)x & 15) == 0, "pwa_colsum_rows: x must be 16-byte aligned");
@@ -106,6 +106,7 @@ extern "C" int pwa_colsum_rows(const void* x, float* dst, int64_t rows, int C, i
   if (blocks < 1) blocks = 1;
   const size_t smem = (size_t)threads * 16;
   if (dtype == PWA_BF16) colsum_rows_kernel<__nv_bfloat16><<<(unsigned)blocks, threads, smem * 2, st>>>((const __nv_bfloat16*)x, dst, nvec, C);
+  else if (dtype == PWA_F16) colsum_rows_kernel<__half><<<(unsigned)blocks, threads, smem * 2, st>>>((const __half*)x, dst, nvec, C);
   else colsum_rows_kernel<float><<<(unsigned)blocks, threads, smem, st>>>((const float*)x, dst, nvec, C);
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;

@@ -3,6 +3,7 @@
 // Bit layouts follow the PTX ISA "tcgen05" chapter (cross-checked against cute/arch/mma_sm100_desc.hpp).
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -137,10 +138,19 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_
   return d;         // base_offset = 0, lbo_mode = 0, layout_type = SWIZZLE_NONE (0)
 }
 
-// Instruction descriptor for kind::f16, bf16 x bf16 -> fp32, dense.
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
+// A / B format code of a kind::f16 instruction descriptor (bits 7-9 and 10-12): F16 = 0, BF16 = 1
+template <typename T> struct F16Kind;
+template <> struct F16Kind<__nv_bfloat16> { static constexpr uint32_t fmt = 1; };
+template <> struct F16Kind<__half> { static constexpr uint32_t fmt = 0; };
+
+// Instruction descriptor for kind::f16, T x T -> fp32 (T = bf16 or fp16), dense.
+template <typename T>
+__host__ __device__ constexpr uint32_t make_idesc(int M, int N, int a_mn_major, int b_mn_major) {
+  return (1u << 4) | (F16Kind<T>::fmt << 7) | (F16Kind<T>::fmt << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
          ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+__host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
+  return make_idesc<__nv_bfloat16>(M, N, a_mn_major, b_mn_major);
 }
 
 // D[tmem] (+)= A[smem] * B[smem]      (single thread issues)
@@ -168,6 +178,24 @@ __device__ __forceinline__ void mma_commit(uint64_t* bar) {
 __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
   __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);  // .x = lo (low 16 bits)
   return *reinterpret_cast<uint32_t*>(&v);
+}
+__device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
+  __half2 v = __floats2half2_rn(lo, hi);             // .x = lo (low 16 bits); overflow rounds to +-inf, NaN stays NaN
+  return *reinterpret_cast<uint32_t*>(&v);
+}
+// pair pack / unpack of the element type T (bf16 or fp16) of the tcgen05 kernels
+template <typename T> __device__ __forceinline__ uint32_t pack2t(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t pack2t<__nv_bfloat16>(float lo, float hi) { return pack_bf16(lo, hi); }
+template <> __device__ __forceinline__ uint32_t pack2t<__half>(float lo, float hi) { return pack_f16(lo, hi); }
+template <typename T> __device__ __forceinline__ void unpack2t(uint32_t w, float& lo, float& hi);
+template <> __device__ __forceinline__ void unpack2t<__nv_bfloat16>(uint32_t w, float& lo, float& hi) {
+  lo = __uint_as_float(w << 16);
+  hi = __uint_as_float(w & 0xffff0000u);
+}
+template <> __device__ __forceinline__ void unpack2t<__half>(uint32_t w, float& lo, float& hi) {
+  const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&w));
+  lo = f.x;
+  hi = f.y;
 }
 
 }  // namespace tc

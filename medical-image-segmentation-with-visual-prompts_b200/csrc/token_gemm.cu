@@ -12,8 +12,8 @@
 // phases of different tiles overlap:
 //   bulk copy (cp.async.bulk, mbarrier complete_tx) of the contiguous x / res tiles -> shared memory
 //   -> per-row statistics in registers (no shuffles: a thread owns its row; exact mean, then centred variance, computed on
-//      the bf16 values that are stored, like csrc/ln.cu) -> s / z tiles written back in place (bulk stores) and z into the
-//      UMMA canonical K-major layout -> C/16 MMAs of N = NCH output channels -> tcgen05.ld, + bias, bf16, staged row-major
+//      the bf16 / fp16 values that are stored, like csrc/ln.cu) -> s / z tiles written back in place (bulk stores) and z into the
+//      UMMA canonical K-major layout -> C/16 MMAs of N = NCH output channels -> tcgen05.ld, + bias, rounded, staged row-major
 //      -> bulk stores of the output rows.
 // Weights wider than fits beside the tiles are split into chunks of NCH output channels over CTAs (blockIdx % n_chunks);
 // a CTA keeps its chunk resident for all of its tiles.
@@ -65,19 +65,17 @@ __device__ __forceinline__ void bulk_s2g(void* dst_gmem, const void* src_smem, u
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void unpack8(const uint4& w, float (&v)[8]) {
+template <typename T> __device__ __forceinline__ void unpack8(const uint4& w, float (&v)[8]) {
   const uint32_t u[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    v[2 * i] = __uint_as_float(u[i] << 16);
-    v[2 * i + 1] = __uint_as_float(u[i] & 0xffff0000u);
-  }
+  for (int i = 0; i < 4; ++i) unpack2t<T>(u[i], v[2 * i], v[2 * i + 1]);
 }
-__device__ __forceinline__ uint4 pack8(const float (&v)[8]) {
-  return make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
+template <typename T> __device__ __forceinline__ uint4 pack8(const float (&v)[8]) {
+  return make_uint4(pack2t<T>(v[0], v[1]), pack2t<T>(v[2], v[3]), pack2t<T>(v[4], v[5]), pack2t<T>(v[6], v[7]));
 }
 
-template <bool HAS_LN, bool HAS_RES, bool HAS_DROP>
+// T: element type of every token tensor, W and bias (bf16 or fp16; the pointers of TokGemmParams only carry the 16-bit width)
+template <typename T, bool HAS_LN, bool HAS_RES, bool HAS_DROP>
 __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
   extern __shared__ __align__(128) uint8_t smem[];
   __shared__ __align__(8) uint64_t bar_ld, bar_mma;
@@ -106,7 +104,7 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
     gam_s[i] = HAS_LN ? p.gamma[i] : 1.f;
     bet_s[i] = HAS_LN ? p.beta[i] : 0.f;
   }
-  for (int i = tid; i < NCH; i += kTM) bias_s[i] = (p.bias && i < nvalid) ? __bfloat162float(p.bias[n0 + i]) : 0.f;
+  for (int i = tid; i < NCH; i += kTM) bias_s[i] = (p.bias && i < nvalid) ? to_f32(reinterpret_cast<const T*>(p.bias)[n0 + i]) : 0.f;
   if (tid == 0) {
     mbar_init(&bar_ld, 1);
     mbar_init(&bar_mma, 1);
@@ -121,7 +119,7 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
   tc_fence_after();
   const uint32_t tmem = tmem_base_s;
   const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
-  const uint32_t idesc = make_idesc_bf16(128, NCH, 0, 0);
+  const uint32_t idesc = make_idesc<T>(128, NCH, 0, 0);
   const uint32_t s0 = HAS_DROP ? p.seed[0] : 0u, s1 = HAS_DROP ? p.seed[1] : 0u;
   const long n_tiles = (p.T + kTM - 1) / kTM;
   const int stride = gridDim.x / p.n_chunks;
@@ -150,7 +148,7 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
       float sum = 0.f;
       for (int c = 0; c < NC8; ++c) {
         float v[8];
-        unpack8(xr[c], v);
+        unpack8<T>(xr[c], v);
         if (HAS_DROP) {
           const long q0 = (row * C + c * 8) >> 2;                   // same mask as pwa_dropout: one hash per 4 elements
 #pragma unroll
@@ -162,24 +160,24 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
               v[h * 4 + e] = ((bits >> (8 * e)) & 0xffu) >= p.drop_thresh ? v[h * 4 + e] * p.inv_keep : 0.f;
           }
           if (!HAS_RES) {                                           // dropped values rounded as pwa_dropout stores them
-            const uint4 w = pack8(v);
-            unpack8(w, v);
+            const uint4 w = pack8<T>(v);
+            unpack8<T>(w, v);
           }
         }
         if (HAS_RES) {
           if (HAS_DROP) {                                           // pwa_dropout rounds its output to bf16 before the add
-            const uint4 w = pack8(v);
-            unpack8(w, v);
+            const uint4 w = pack8<T>(v);
+            unpack8<T>(w, v);
           }
           float r[8];
-          unpack8(rr[c], r);
+          unpack8<T>(rr[c], r);
 #pragma unroll
           for (int e = 0; e < 8; ++e) v[e] += r[e];
         }
         if (HAS_RES || HAS_DROP) {
-          const uint4 w = pack8(v);
+          const uint4 w = pack8<T>(v);
           xr[c] = w;
-          unpack8(w, v);
+          unpack8<T>(w, v);
         }
 #pragma unroll
         for (int e = 0; e < 8; ++e) sum += v[e];
@@ -189,7 +187,7 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
         float q = 0.f;
         for (int c = 0; c < NC8; ++c) {
           float v[8];
-          unpack8(xr[c], v);
+          unpack8<T>(xr[c], v);
 #pragma unroll
           for (int e = 0; e < 8; ++e) {
             const float d = v[e] - mean;
@@ -208,7 +206,7 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
       float v[8];
       uint4 w = make_uint4(0, 0, 0, 0);
       if (live) {
-        unpack8(xr[c], v);
+        unpack8<T>(xr[c], v);
         if (HAS_LN) {
           const float4 g0 = *reinterpret_cast<const float4*>(gam_s + c * 8), g1 = *reinterpret_cast<const float4*>(gam_s + c * 8 + 4);
           const float4 b0 = *reinterpret_cast<const float4*>(bet_s + c * 8), b1 = *reinterpret_cast<const float4*>(bet_s + c * 8 + 4);
@@ -216,7 +214,7 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
 #pragma unroll
           for (int e = 0; e < 8; ++e) v[e] = fmaf((v[e] - mean) * rstd, gm[e], bt[e]);
         }
-        w = pack8(v);
+        w = pack8<T>(v);
         if (HAS_LN) rr[c] = w;
       }
       *reinterpret_cast<uint4*>(As + (c * kTM + tid) * 16) = w;   // rows beyond the tensor feed zeros
@@ -248,8 +246,8 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
       for (int e = 0; e < 16; ++e) v[e] += bias_s[c * 16 + e];
       uint4* dst = reinterpret_cast<uint4*>(Os + ((size_t)tid * NCH + c * 16) * 2);
       const float lo[8] = {v[0], v[1], v[2], v[3], v[4], v[5], v[6], v[7]}, hi[8] = {v[8], v[9], v[10], v[11], v[12], v[13], v[14], v[15]};
-      dst[0] = pack8(lo);
-      dst[1] = pack8(hi);
+      dst[0] = pack8<T>(lo);
+      dst[1] = pack8<T>(hi);
     }
     tc_fence_before();
     fence_proxy_async_smem();
@@ -270,6 +268,18 @@ __global__ void __launch_bounds__(kTM) token_gemm_kernel(TokGemmParams p) {
   if (warp == 0) tmem_dealloc(tmem, tcols);
 }
 
+template <typename T>
+void (*select_kernel(bool ln, bool rs, bool dr))(TokGemmParams) {
+  if (ln && rs && dr) return token_gemm_kernel<T, true, true, true>;
+  if (ln && rs) return token_gemm_kernel<T, true, true, false>;
+  if (ln && dr) return token_gemm_kernel<T, true, false, true>;
+  if (ln) return token_gemm_kernel<T, true, false, false>;
+  if (rs && dr) return token_gemm_kernel<T, false, true, true>;
+  if (rs) return token_gemm_kernel<T, false, true, false>;
+  if (dr) return token_gemm_kernel<T, false, false, true>;
+  return token_gemm_kernel<T, false, false, false>;
+}
+
 }  // namespace
 
 }  // namespace pwa
@@ -283,7 +293,16 @@ extern "C" int pwa_token_gemm_supported(int C, int Cout) {
 extern "C" int pwa_token_gemm_fwd(const void* x, const void* res, const float* gamma, const float* beta, const void* W,
                                   const void* bias, void* sum_out, void* ln_out, void* y, float* mean, float* rstd,
                                   int64_t T, int C, int Cout, float eps, float p_drop, const void* seed_dev, void* stream) {
+  return pwa_token_gemm_fwd_dt(x, res, gamma, beta, W, bias, sum_out, ln_out, y, mean, rstd, T, C, Cout, eps, p_drop, seed_dev,
+                               PWA_BF16, stream);
+}
+
+extern "C" int pwa_token_gemm_fwd_dt(const void* x, const void* res, const float* gamma, const float* beta, const void* W,
+                                     const void* bias, void* sum_out, void* ln_out, void* y, float* mean, float* rstd,
+                                     int64_t T, int C, int Cout, float eps, float p_drop, const void* seed_dev, int dtype,
+                                     void* stream) {
   PWA_CHECK_ARG(x && W && y, "pwa_token_gemm_fwd: null pointer");
+  PWA_CHECK_ARG(dtype == PWA_BF16 || dtype == PWA_F16, "pwa_token_gemm_fwd: bad dtype %d (bf16 or fp16)", dtype);
   PWA_CHECK_ARG(pwa_token_gemm_supported(C, Cout), "pwa_token_gemm_fwd: need C %% 16 == 0, 16 <= C <= 192, Cout %% 16 == 0 (C=%d Cout=%d)", C, Cout);
   PWA_CHECK_ARG((gamma == nullptr) == (beta == nullptr), "pwa_token_gemm_fwd: gamma and beta go together");
   PWA_CHECK_ARG(p_drop >= 0.f && p_drop < 1.f && (p_drop == 0.f || seed_dev), "pwa_token_gemm_fwd: dropout needs seed words");
@@ -324,15 +343,7 @@ extern "C" int pwa_token_gemm_fwd(const void* x, const void* res, const float* g
   if (grid > n_tiles * p.n_chunks) grid = n_tiles * p.n_chunks;
   if (grid < p.n_chunks) grid = p.n_chunks;
   const bool ln = gamma != nullptr, rs = res != nullptr, dr = p.drop_thresh != 0;
-  void (*kern)(TokGemmParams) = nullptr;
-  if (ln && rs && dr) kern = token_gemm_kernel<true, true, true>;
-  else if (ln && rs) kern = token_gemm_kernel<true, true, false>;
-  else if (ln && dr) kern = token_gemm_kernel<true, false, true>;
-  else if (ln) kern = token_gemm_kernel<true, false, false>;
-  else if (rs && dr) kern = token_gemm_kernel<false, true, true>;
-  else if (rs) kern = token_gemm_kernel<false, true, false>;
-  else if (dr) kern = token_gemm_kernel<false, false, true>;
-  else kern = token_gemm_kernel<false, false, false>;
+  void (*kern)(TokGemmParams) = dtype == PWA_F16 ? select_kernel<__half>(ln, rs, dr) : select_kernel<__nv_bfloat16>(ln, rs, dr);
   PWA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total));
   kern<<<(unsigned)grid, kTM, L.total, (cudaStream_t)stream>>>(p);
   PWA_CUDA_OK(cudaGetLastError());

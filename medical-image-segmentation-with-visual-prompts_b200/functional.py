@@ -12,7 +12,8 @@ import torch
 from . import _lib
 from .geometry import Geometry
 
-_DT = {torch.float32: _lib.PWA_F32, torch.bfloat16: _lib.PWA_BF16}
+_DT = {torch.float32: _lib.PWA_F32, torch.bfloat16: _lib.PWA_BF16, torch.float16: _lib.PWA_F16}
+_LOWP = (torch.bfloat16, torch.float16)          # the 16-bit compute types: tcgen05 kernels where the shape allows
 
 
 class KernelStats:
@@ -59,7 +60,7 @@ class _timed:
 
 def _dtype_code(t: torch.Tensor) -> int:
     if t.dtype not in _DT:
-        raise TypeError(f"pwa kernels support float32 and bfloat16, got {t.dtype}")
+        raise TypeError(f"pwa kernels support float32, bfloat16 and float16, got {t.dtype}")
     return _DT[t.dtype]
 
 
@@ -302,7 +303,7 @@ class _WindowAttention(torch.autograd.Function):
         lse = torch.empty((B, P, heads, N), dtype=torch.float32, device=q.device)
         work = torch.empty(heads, dtype=torch.int32, device=q.device) if DYNAMIC_WORK else None
         s = _shape_struct(B, P, Cc, heads, I, ws, scale, p_drop=p_drop, seed_dev=seed, work=work,
-                          sel=sel_table_for(ids) if q.dtype == torch.bfloat16 and impl != IMPL_F32 else None)
+                          sel=sel_table_for(ids) if q.dtype in _LOWP and impl != IMPL_F32 else None)
         with torch.cuda.device(q.device), _timed("attn_fwd", 1, 4.0 * B * P * N * (N + I) * Cc, q):
             rc = _lib.lib.pwa_attn_fwd(_ptr(q), _ptr(k), _ptr(v), _ptr(kp), _ptr(vp), _ptr(th), _ptr(tw), _ptr(td),
                                        _ptr(tok), _ptr(ids), _ptr(out), _ptr(lse), C.byref(s), _dtype_code(q), impl,
@@ -326,7 +327,7 @@ class _WindowAttention(torch.autograd.Function):
         dtok = torch.empty_like(tok) if I else None
         delta = torch.empty_like(lse)
         s = _shape_struct(B, P, Cc, heads, I, ws, scale, p_drop=p_drop, seed_dev=seed,
-                          sel=sel_table_for(ids) if q.dtype == torch.bfloat16 and impl != IMPL_F32 else None)
+                          sel=sel_table_for(ids) if q.dtype in _LOWP and impl != IMPL_F32 else None)
         with torch.cuda.device(q.device), _timed("attn_bwd", 2, 8.0 * B * P * N * (N + I) * Cc, q):
             rc = _lib.lib.pwa_attn_bwd(_ptr(q), _ptr(k), _ptr(v), _ptr(kp), _ptr(vp), _ptr(th), _ptr(tw), _ptr(td),
                                        _ptr(tok), _ptr(ids), _ptr(out), _ptr(lse), _ptr(dout), _ptr(dq), _ptr(dk),
@@ -649,7 +650,7 @@ class _WindowAttentionPacked(torch.autograd.Function):
         lse = torch.empty((B, P, heads, N), dtype=torch.float32, device=qkv.device)
         work = torch.empty(heads, dtype=torch.int32, device=qkv.device) if DYNAMIC_WORK else None
         s = _shape_struct(B, P, Cc, heads, I, ws, scale, p_drop=p_drop, ld_qkv=C3, ld_p=2 * Cc, seed_dev=seed, work=work,
-                          sel=sel_table_for(ids) if qkv.dtype == torch.bfloat16 and impl != IMPL_F32 else None)
+                          sel=sel_table_for(ids) if qkv.dtype in _LOWP and impl != IMPL_F32 else None)
         q0 = qkv.data_ptr()
         p0 = 0 if kvp is None else kvp.data_ptr()
         vpp = C.c_void_p
@@ -677,7 +678,7 @@ class _WindowAttentionPacked(torch.autograd.Function):
         dtok = torch.empty_like(tok) if I else None
         delta = torch.empty_like(lse)
         s = _shape_struct(B, P, Cc, heads, I, ws, scale, p_drop=p_drop, ld_qkv=C3, ld_p=2 * Cc, seed_dev=seed,
-                          sel=sel_table_for(ids) if qkv.dtype == torch.bfloat16 and impl != IMPL_F32 else None)
+                          sel=sel_table_for(ids) if qkv.dtype in _LOWP and impl != IMPL_F32 else None)
         q0, d0 = qkv.data_ptr(), dqkv.data_ptr()
         p0 = 0 if kvp is None else kvp.data_ptr()
         vpp = C.c_void_p
@@ -778,6 +779,8 @@ def _mm_f32(a, b):
     try:
         return torch.mm(a, b, out_dtype=torch.float32)
     except (TypeError, RuntimeError):
+        if a.dtype == torch.float16:          # an fp16 result would overflow / round the fp32 sums: upcast instead
+            return torch.mm(a.float(), b.float())
         return torch.mm(a, b).float()
 
 
@@ -801,13 +804,13 @@ def colsum_f32(part):
 
 
 def colsum_rows(x2):
-    """[T, C] bf16 / fp32 -> fp32 [C] column sums on the pwa kernel (csrc/reduce.cu: pwa_colsum_rows): the bias gradient of a
+    """[T, C] bf16 / fp16 / fp32 -> fp32 [C] column sums on the pwa kernel (csrc/reduce.cu: pwa_colsum_rows): the bias gradient of a
     Linear whose output gradient is x2 (window_attention.py:28-30).  torch's generic reduction for shapes outside the
     kernel's envelope (C not a multiple of 16 bytes, strided rows)."""
     _require_cuda(x2)
     T, Cc = x2.shape
     e = 16 // x2.element_size()
-    if x2.dtype not in (torch.float32, torch.bfloat16) or not x2.is_contiguous() or Cc % e or Cc // e > 512 or x2.data_ptr() % 16:
+    if x2.dtype not in _DT or not x2.is_contiguous() or Cc % e or Cc // e > 512 or x2.data_ptr() % 16:
         return x2.sum(dim=0, dtype=torch.float32)
     if T == 0:
         return torch.zeros(Cc, dtype=torch.float32, device=x2.device)
@@ -887,7 +890,7 @@ def multi_linear(x, bias, *weights, lowp=None, bias_grad=True, lowp_bias=None):
 # token-domain GEMMs with fused LayerNorm / residual / dropout prologue (csrc/token_gemm.cu, tcgen05)
 # ------------------------------------------------------------------------------------------------
 def token_gemm_supported(C: int, Cout: int, dtype) -> bool:
-    return dtype == torch.bfloat16 and bool(_lib.lib.pwa_token_gemm_supported(int(C), int(Cout)))
+    return dtype in _LOWP and bool(_lib.lib.pwa_token_gemm_supported(int(C), int(Cout)))
 
 
 def token_gemm_profitable(C: int, rows: int) -> bool:
@@ -908,8 +911,9 @@ def _token_gemm_raw(x2, res2, g32, b32, w, bias, want_sum, want_ln, want_stats, 
     rstd = torch.empty(rows, dtype=torch.float32, device=dev) if want_stats else None
     nbytes = ((1 if res2 is None else 2) + (1 if want_sum else 0) + (1 if want_ln else 0)) * x2.numel() * 2 + y.numel() * 2
     with torch.cuda.device(dev), _timed("token_gemm", 1, float(nbytes), x2):
-        rc = _lib.lib.pwa_token_gemm_fwd(_ptr(x2), _ptr(res2), _ptr(g32), _ptr(b32), _ptr(w), _ptr(bias), _ptr(s), _ptr(z), _ptr(y),
-                                         _ptr(mean), _ptr(rstd), rows, Cc, Cout, float(eps), float(p_drop), _ptr(seed), _stream(x2))
+        rc = _lib.lib.pwa_token_gemm_fwd_dt(_ptr(x2), _ptr(res2), _ptr(g32), _ptr(b32), _ptr(w), _ptr(bias), _ptr(s), _ptr(z),
+                                            _ptr(y), _ptr(mean), _ptr(rstd), rows, Cc, Cout, float(eps), float(p_drop), _ptr(seed),
+                                            _dtype_code(x2), _stream(x2))
     _lib.check(rc, "pwa_token_gemm_fwd")
     return y, s, z, mean, rstd
 

@@ -42,7 +42,7 @@ class PatchMerging(nn.Module):
         from ... import functional as PF
         k = 8 if self.merge_last_dim else 4
         if x.is_cuda and x.dim() == 5 and x.shape[1] > 1 and x.permute(0, 2, 3, 4, 1).is_contiguous() \
-                and PF.layer_norm_supported(k * x.shape[1]) and x.dtype in (torch.float32, torch.bfloat16):
+                and PF.layer_norm_supported(k * x.shape[1]) and x.dtype in (torch.float32, torch.bfloat16, torch.float16):
             from ...geometry import rowmap_merge_from_voxels
             b, c = x.shape[:2]
             rm, (h2, w2, d2) = rowmap_merge_from_voxels(tuple(int(v) for v in x.shape[2:]), bool(self.merge_last_dim))

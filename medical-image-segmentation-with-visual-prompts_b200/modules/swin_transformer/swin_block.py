@@ -221,10 +221,15 @@ class SwinTransformerBlock(nn.Module):
         self.mlp = nn.Linear(hidden_channels, hidden_channels)    # the reference "MLP" is ONE Linear (:141-143)
 
     def _compute_dtype(self, x):
+        """bf16 for a bf16 input or under autocast(bfloat16); fp16 for an fp16 input or under autocast(float16) (torch's
+        default autocast dtype); else fp32.  The 16-bit types run on the tcgen05 kernels, fp32 on the CUDA-core ones."""
         if x.dtype == torch.bfloat16:
             return torch.bfloat16
-        if torch.is_autocast_enabled() and torch.get_autocast_dtype('cuda') == torch.bfloat16:
+        autocast = torch.get_autocast_dtype('cuda') if torch.is_autocast_enabled() else None
+        if autocast == torch.bfloat16:
             return torch.bfloat16
+        if x.dtype == torch.float16 or autocast == torch.float16:
+            return torch.float16
         return torch.float32
 
     def _lowp_weights(self, cdt):

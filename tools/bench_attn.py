@@ -41,7 +41,9 @@ def main():
     ap.add_argument("--batch", type=int, default=4)
     ap.add_argument("--stages", default="enc0,enc1,enc2,dec0")
     ap.add_argument("--dropout", type=float, default=0.0)
+    ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp16"], help="element type of the attention kernels")
     args = ap.parse_args()
+    adt = torch.bfloat16 if args.dtype == "bf16" else torch.float16
     dev = torch.device("cuda")
     B, I = args.batch, 64
     torch.manual_seed(0)
@@ -51,8 +53,8 @@ def main():
             g = pwa_b200.get_geometry(dims, WS, (4, 4, 2) if shifted else (0, 0, 0))
             P, N = g.P, g.N
             if "attn" in args.what:
-                qkv = torch.randn(B, P, N, 3 * C, device=dev).to(torch.bfloat16).requires_grad_(True)
-                kvp = torch.randn(B, I, 2 * C, device=dev).to(torch.bfloat16).requires_grad_(True)
+                qkv = torch.randn(B, P, N, 3 * C, device=dev).to(adt).requires_grad_(True)
+                kvp = torch.randn(B, I, 2 * C, device=dev).to(adt).requires_grad_(True)
                 th, tw, td = (0.3 * torch.randn(heads, w, w, device=dev) for w in WS)
                 tok = 0.3 * torch.randn(heads, I, device=dev)
                 ids = g.region_ids(dev) if g.masked else None
@@ -66,7 +68,7 @@ def main():
                 t_f = timeit(lambda: fwd(), args.iters)
                 t_fb = timeit(lambda: fwd().backward(go), args.iters)
                 fl = 4.0 * B * P * N * (N + I) * C
-                print(json.dumps({"kernel": "attn", "stage": name, "shifted": shifted, "B": B, "P": P, "drop": args.dropout, "fwd_us": round(t_f, 1),
+                print(json.dumps({"kernel": "attn", "dtype": args.dtype, "stage": name, "shifted": shifted, "B": B, "P": P, "drop": args.dropout, "fwd_us": round(t_f, 1),
                                   "bwd_us": round(t_fb - t_f, 1), "fwd_tflops": round(fl / t_f / 1e6, 1),
                                   "bwd_tflops": round(2 * fl / max(t_fb - t_f, 1e-3) / 1e6, 1),
                                   "fwd_Gexp_s": round(B * P * heads * N * (N + I) / t_f / 1e3, 1)}))
