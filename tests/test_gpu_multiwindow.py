@@ -24,6 +24,7 @@ pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 RTOL_F32 = 1e-4
 RTOL_BF16 = 2e-2
+RTOL_F16 = 5e-3            # tests/test_gpu_fp16.py (that module imports this one, so the value is restated here)
 WS = (8, 8, 4)
 N = 256
 NAMES = ["q", "k", "v", "kp", "vp", "th", "tw", "td", "tok"]
@@ -193,7 +194,8 @@ def _block_oracle(blk, x, p, go, heads, shift_cfg):
 @pytest.mark.parametrize("stage,shifted,dtype,rtol", [
     ("enc0", True, torch.bfloat16, RTOL_BF16), ("enc0", False, torch.bfloat16, RTOL_BF16),
     ("enc2", True, torch.bfloat16, RTOL_BF16), ("dec0", True, torch.bfloat16, RTOL_BF16),
-    ("enc1", True, torch.float32, RTOL_F32), ("enc0", True, torch.float32, RTOL_F32)])
+    ("enc1", True, torch.float32, RTOL_F32), ("enc0", True, torch.float32, RTOL_F32),
+    ("enc0", True, torch.float16, RTOL_F16), ("enc2", True, torch.float16, RTOL_F16)])
 def test_block_full_size_vs_oracle(stage, shifted, dtype, rtol):
     """Whole SwinTransformerBlock (partition, LayerNorms, projections, attention, reverse; all 21 gradient tensors) at a
     BASELINE stage shape against R.block_forward in float64."""

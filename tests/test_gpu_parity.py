@@ -364,7 +364,7 @@ def test_block_full_size_runs_and_matches_oracle_sample():
 
 
 @pytest.mark.parametrize("C", [12, 48, 96, 192, 384, 768, 1536, 2048])
-@pytest.mark.parametrize("dtype,rtol", [(torch.float32, 1e-5), (torch.bfloat16, RTOL_BF16)])
+@pytest.mark.parametrize("dtype,rtol", [(torch.float32, 1e-5), (torch.bfloat16, RTOL_BF16), (torch.float16, 2e-3)])
 @pytest.mark.parametrize("with_res", [False, True])
 def test_layer_norm_kernels(C, dtype, rtol, with_res):
     """pwa LayerNorm (+ fused residual add) forward/backward against torch in float64."""
@@ -380,8 +380,8 @@ def test_layer_norm_kernels(C, dtype, rtol, with_res):
     r64 = res.double().requires_grad_(True) if with_res else None
     g64, b64 = gamma.double().requires_grad_(True), beta.double().requires_grad_(True)
     s64 = x64 + r64 if with_res else x64
-    if with_res and dtype == torch.bfloat16:
-        s64 = s64 + (s64.detach().to(dtype).double() - s64.detach())      # the kernel normalises the STORED bf16 sum
+    if with_res and dtype != torch.float32:
+        s64 = s64 + (s64.detach().to(dtype).double() - s64.detach())      # the kernel normalises the STORED 16-bit sum
     y64 = torch.nn.functional.layer_norm(s64, (C,), g64, b64, 1e-6)
     loss = (y64 * go_y.double()).sum() + ((s64 * go_s.double()).sum() if with_res else 0)
     loss.backward()
@@ -758,11 +758,11 @@ def test_colsum_f32_matches_torch(S, shape):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("T,C", [(442368, 144), (55296, 288), (28672, 576), (1, 8), (1037, 48), (3, 4096), (0, 48), (777, 20)])
-@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32])
+@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32, torch.float16])
 def test_colsum_rows_matches_float64(T, C, dtype):
     """pwa_colsum_rows (bias gradient of the q|k|v projection, window_attention.py:28-30) against a float64 sum of the
     same values; ragged row counts, the widest row the kernel takes, an empty matrix, and a width outside the envelope
-    (C = 20 in bf16: torch's reduction)."""
+    (C = 20 in bf16 / fp16: torch's reduction)."""
     from pwa_b200 import functional as PF
     torch.manual_seed(T + C)
     x = (torch.randn(T, C, device=DEV) + 0.25).to(dtype)
@@ -789,7 +789,7 @@ def test_token_split_weight_gradient(T, co, ci):
     assert (dw.double() - ref).abs().max().item() <= 1e-4 * ref.abs().max().item()
 
 
-@pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
+@pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16, torch.float16])
 @pytest.mark.parametrize("n", [4096, 1000003])
 def test_seeded_projection_dropout_matches_oracle_mask(dtype, n):
     """pwa_dropout (the seeded stand-in for nn.Dropout(proj_drop), window_attention.py:60): exactly the mask the oracle
@@ -808,21 +808,22 @@ def test_seeded_projection_dropout_matches_oracle_mask(dtype, n):
     assert rel_linf(x.grad, (g.double() * keep).to(dtype)) < (1e-6 if dtype == torch.float32 else 4e-3)
 
 
-@pytest.mark.parametrize("C", [12, 48, 96, 192, 768])
-def test_dropout_backward_emits_bias_gradient(C):
+@pytest.mark.parametrize("C,dtype", [pytest.param(C, t, id=str(C) if t == torch.bfloat16 else f"{C}-{str(t)[6:]}")
+                                     for t in (torch.bfloat16, torch.float16, torch.float32) for C in (12, 48, 96, 192, 768)])
+def test_dropout_backward_emits_bias_gradient(C, dtype):
     """pwa_dropout_colsum: the masked gradient AND its column sums (= the gradient of the bias of the Linear in front of the
     dropout) in one pass, against torch."""
     torch.manual_seed(C)
     rows = 1000 + C
     lin = torch.nn.Linear(C, C).to(DEV)
-    x = torch.randn(rows, C, device=DEV).bfloat16()
+    x = torch.randn(rows, C, device=DEV).to(dtype)
     seed = torch.tensor([5, 6], dtype=torch.int32, device=DEV)
     o = PF.multi_linear(x, lin.bias, lin.weight, bias_grad=False)
     y = PF.seeded_dropout(o, 0.1, seed, bias_of_x=lin.bias)
-    g = torch.randn(rows, C, device=DEV).bfloat16()
+    g = torch.randn(rows, C, device=DEV).to(dtype)
     y.backward(g)
     keep = R.elementwise_dropout_keep_factor([5, 6], rows * C, 0.1).to(DEV).reshape(rows, C)
-    ref = (g.double() * keep).sum(0)                 # (the kernel sums the fp32 products, before the bf16 rounding of dx)
+    ref = (g.double() * keep).sum(0)                 # (the kernel sums the fp32 products, before the 16-bit rounding of dx)
     assert rel_linf(lin.bias.grad, ref) < 1e-5
 
 
