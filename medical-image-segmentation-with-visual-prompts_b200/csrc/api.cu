@@ -44,6 +44,16 @@ static int fill(AttnParams& p, const pwa_attn_shape* s, const char* who) {
   return PWA_OK;
 }
 
+bool attn_tc_supported(const AttnParams& p, int dtype) {
+  if (dtype != PWA_BF16 && dtype != PWA_F16) return false;
+  if (p.N != 256) return false;                                  // two 128-row query tiles / two 128-key content blocks
+  if (p.wd > 4 || p.wh + p.ww > 16) return false;                // one-hot bias columns must fit the staged layout
+  if (p.I % 32 != 0 || p.I > 128) return false;                  // prompt keys are read in 32-column chunks
+  const int dh = p.C / p.heads;
+  if (!(dh == 3 || dh == 6 || dh == 12 || dh == 24 || dh == 48)) return false;   // the instantiated head dims
+  return attn_ws_fits(p) && attn_tc_bwd_fits(p);
+}
+
 }  // namespace pwa
 
 using namespace pwa;
@@ -93,13 +103,7 @@ extern "C" int pwa_attn_fwd(const void* q, const void* k, const void* v, const v
     set_error("pwa_attn_fwd: tcgen05 kernel does not support this shape/dtype");
     return PWA_ERR_UNSUPPORTED;
   }
-  if (impl == 2 || (impl == 0 && tc_ok)) {
-    // PWA_FWD_WS=0 (test infrastructure): the round-1 kernel (four 128-thread CTAs per SM) for A/B measurements -- bf16
-    // only: fp16 always runs the warp-specialised kernel (tc_ok implies that it takes the shape)
-    static const int use_ws = getenv("PWA_FWD_WS") ? atoi(getenv("PWA_FWD_WS")) : 1;
-    if ((use_ws || dtype == PWA_F16) && attn_ws_supported(p, dtype)) return attn_ws_forward(p, dtype, st);
-    return attn_tc_forward(p, st);
-  }
+  if (impl == 2 || (impl == 0 && tc_ok)) return attn_ws_forward(p, dtype, st);
   return attn_f32_forward(p, dtype, st);
 }
 
@@ -130,7 +134,7 @@ extern "C" int pwa_attn_bwd(const void* q, const void* k, const void* v, const v
     PWA_CUDA_OK(cudaMemsetAsync(dkp, 0, (size_t)p.B * p.I * p.C * 4, st));
     PWA_CUDA_OK(cudaMemsetAsync(dvp, 0, (size_t)p.B * p.I * p.C * 4, st));
   }
-  const bool tc_ok = attn_tc_bwd_supported(p, dtype);
+  const bool tc_ok = attn_tc_supported(p, dtype);
   if (impl == 2 && !tc_ok) {
     set_error("pwa_attn_bwd: tcgen05 kernel does not support this shape/dtype");
     return PWA_ERR_UNSUPPORTED;

@@ -127,13 +127,12 @@ __device__ __forceinline__ uint32_t drop_transpose_tile(uint32_t x, int lane) {
 int attn_f32_forward(const AttnParams& p, int dtype, cudaStream_t st);
 int attn_f32_backward(const AttnParams& p, int dtype, cudaStream_t st);
 
-// tcgen05 / TMEM kernels.  attn_tc_supported: bf16 -> the round-1 forward's envelope (attn_tc.cu, bf16 only); fp16 -> the
-// shapes that BOTH the warp-specialised forward and the backward take (the round-1 forward never runs fp16)
+// tcgen05 / TMEM kernels, bf16 or fp16.  attn_tc_supported (api.cu) is the one envelope that forward and backward dispatch
+// on: the shapes the kernels are written for plus the budgets below.  The *_fits checks assume a shape inside that envelope.
 bool attn_tc_supported(const AttnParams& p, int dtype);
-int attn_tc_forward(const AttnParams& p, cudaStream_t st);                 // bf16 only
-bool attn_ws_supported(const AttnParams& p, int dtype);       // attn_tc_ws.cu: warp-specialised forward
-int attn_ws_forward(const AttnParams& p, int dtype, cudaStream_t st);     // bf16 or fp16
-bool attn_tc_bwd_supported(const AttnParams& p, int dtype);   // attn_tc_bwd.cu
-int attn_tc_backward(const AttnParams& p, int dtype, cudaStream_t st);    // bf16 or fp16
+bool attn_ws_fits(const AttnParams& p);                                   // attn_tc_ws.cu: shared memory of the forward
+int attn_ws_forward(const AttnParams& p, int dtype, cudaStream_t st);
+bool attn_tc_bwd_fits(const AttnParams& p);                               // attn_tc_bwd.cu: TMEM and shared memory of the backward
+int attn_tc_backward(const AttnParams& p, int dtype, cudaStream_t st);
 
 }  // namespace pwa

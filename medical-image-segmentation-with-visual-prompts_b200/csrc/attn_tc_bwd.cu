@@ -97,7 +97,7 @@ __host__ __device__ inline BwdSmem bwd_layout(int KS, int DHP, int NKT, int wh, 
   s.delta = o; o += kN * 4;
   s.wp = o; o += kN * 2;                          // bf16 exp(-lse) per query (value of a masked P entry)
   s.rs = o; o += kN * 4;                          // dropout hash of every query row (csrc/attn.cuh: drop_row_hash)
-  s.sel = o; o += masked ? kIds * (kN / 4) * 4 : 0;   // PRMT selectors [id slot][4 tokens], as in attn_tc.cu
+  s.sel = o; o += masked ? kIds * (kN / 4) * 4 : 0;   // PRMT selectors [id slot][4 tokens], as in the forward (attn_tc_ws.cu)
   s.ids = o; o += kN;
   s.opnd_bytes = (o + 127) & ~127u;
   uint32_t sh = 0;
@@ -961,8 +961,7 @@ int launch_bwd_tc(const AttnParams& p, cudaStream_t st) {
 
 }  // namespace
 
-bool attn_tc_bwd_supported(const AttnParams& p, int dtype) {
-  if (!attn_tc_supported(p, dtype)) return false;
+bool attn_tc_bwd_fits(const AttnParams& p) {
   const int dh = p.C / p.heads;
   const int KS = (dh + 4 + 15) / 16, DHP = (dh + 15) / 16 * 16;
   if (128 + DHP + 3 * KS * 16 + 48 > 512) return false;

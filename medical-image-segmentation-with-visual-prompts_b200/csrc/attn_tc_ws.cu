@@ -1,4 +1,4 @@
-// (b) fused prompted window attention forward, warp-specialised (tcgen05 + TMEM, bf16 or fp16 I/O) -- round-2 kernel.
+// (b) fused prompted window attention forward, warp-specialised (tcgen05 + TMEM, bf16 or fp16 I/O).
 //
 // One persistent CTA per SM (768 threads = 24 warps, 6 per scheduler) = one fixed head, walking (sample, window) pairs.
 // The softmax of this path is bound by the MUFU pipe (one ex2 per logit, 16 / clk / SM), so everything else is taken off
@@ -20,10 +20,10 @@
 //                       to three operand sets in flight), |q|^2 per row and max |k|^2 (stabiliser), region ids and the
 //                       PRMT selector table of the window (one cp.async.bulk of a host-built table, pwa_attn_sel_table);
 //                       they also fetch the next window index from the per-head work counter.
-// The arithmetic is that of attn_tc.cu (round 1): no row-max pass (norm-bound stabiliser with an exact-max sweep as the
-// rare fallback), no online rescaling, relative-position bias folded into the QK^T MMA through one-hot / table columns,
-// multiplicative pre-softmax shift mask (window_attention.py:49-58), ones column of V for the softmax denominator,
-// bit-sliced dropout keep words (csrc/attn.cuh).  TMEM: per group 3 x 64 columns of S / P plus 1-2 O accumulators.
+// The arithmetic: no row-max pass (norm-bound stabiliser with an exact-max sweep as the rare fallback), no online
+// rescaling, relative-position bias folded into the QK^T MMA through one-hot / table columns, multiplicative pre-softmax
+// shift mask (window_attention.py:49-58), ones column of V for the softmax denominator, bit-sliced dropout keep words
+// (csrc/attn.cuh).  TMEM: per group 3 x 64 columns of S / P plus 1-2 O accumulators.
 #include <type_traits>
 
 #include "attn.cuh"
@@ -83,41 +83,6 @@ __device__ __forceinline__ void fadd2w(float& s0, float& s1, float a0, float a1)
   asm("mov.b64 %0, {%1, %2};" : "=l"(s) : "f"(s0), "f"(s1));
   asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(s), "l"(a));
   asm("mov.b64 {%0, %1}, %2;" : "=f"(s0), "=f"(s1) : "l"(d));
-}
-// general packed fp32 pair ops: (d0, d1) = (a0, a1) * (b0, b1) + (c0, c1)
-__device__ __forceinline__ void fma2g(float& d0, float& d1, float a0, float a1, float b0, float b1, float c0, float c1) {
-  unsigned long long a, b, c, d;
-  asm("mov.b64 %0, {%1, %2};" : "=l"(a) : "f"(a0), "f"(a1));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(b) : "f"(b0), "f"(b1));
-  asm("mov.b64 %0, {%1, %2};" : "=l"(c) : "f"(c0), "f"(c1));
-  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(a), "l"(b), "l"(c));
-  asm("mov.b64 {%0, %1}, %2;" : "=f"(d0), "=f"(d1) : "l"(d));
-}
-// exp2 of a PAIR on the FMA pipe (x <= 0): Cody-Waite split with round-to-nearest by a magic-number add, degree-3 minimax
-// polynomial of 2^f on [-0.5, 0.5] (max relative error 7.5e-5, far inside bf16's 2^-9), exponent patched in with one
-// integer multiply-add per element.  The MUFU pipe (16 ex2 / clk / SM) is what bounds this kernel once the softmax warps
-// are kept fed, so a fixed share of every chunk's pairs (kPolyPairs, a bit per packed pair) takes this path instead:
-// 6 packed FMA-pipe instructions + 2 FMNMX + 2 IMAD per pair against two MUFU slots of 8 clk each.
-// Measured at enc0 (make POLY=0x8888 / 0xA4A4 = 4 / 6 of 16 pairs): 227 -> 220 / 222 us unshifted, 222 -> 233 / 234 us shifted,
-// 277 -> 308 / 320 us with dropout: the exp phases run at ~85 % of the MUFU rate but only ~70 % of a softmax warp's time is
-// exp phase, and the extra issue slots cost as much as the freed MUFU slots give.  Off by default.
-#ifndef PWA_WS_POLY_PAIRS
-#define PWA_WS_POLY_PAIRS 0x0u
-#endif
-constexpr uint32_t kPolyPairsW = PWA_WS_POLY_PAIRS;
-__device__ __forceinline__ void poly_exp2_pair(float x0, float x1, float& p0, float& p1) {
-  constexpr float kMagic = 12582912.f;                     // 1.5 * 2^23: round(x) lands in the low mantissa bits
-  x0 = fmaxf(x0, -125.f);
-  x1 = fmaxf(x1, -125.f);
-  float t0, t1, r0, r1, f0, f1, q0, q1;
-  fma2g(t0, t1, x0, x1, 1.f, 1.f, kMagic, kMagic);
-  fma2g(r0, r1, t0, t1, 1.f, 1.f, -kMagic, -kMagic);
-  fma2g(f0, f1, r0, r1, -1.f, -1.f, x0, x1);               // [-0.5, 0.5]
-  fma2g(q0, q1, f0, f1, 0.05517132f, 0.05517132f, 0.24261054f, 0.24261054f);
-  fma2g(q0, q1, q0, q1, f0, f1, 0.69326097f, 0.69326097f);
-  fma2g(q0, q1, q0, q1, f0, f1, 0.99992812f, 0.99992812f);
-  p0 = __int_as_float(__float_as_int(q0) + (__float_as_int(t0) << 23));
-  p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(t1) << 23));
 }
 
 __device__ __forceinline__ uint32_t hadd2_bf16(uint32_t a, uint32_t b) {
@@ -468,14 +433,9 @@ __global__ void __launch_bounds__(kThreadsW, 1) attn_fwd_ws_kernel(AttnParams p)
           uint32_t pk[16];
 #pragma unroll
           for (int q = 0; q < 16; ++q) {
-            float x0, x1, p0, p1;
+            float x0, x1;
             ffma2w(x0, x1, __uint_as_float(r[2 * q]), __uint_as_float(r[2 * q + 1]), c2, -mb);
-            if ((kPolyPairsW >> q) & 1u) {
-              poly_exp2_pair(x0, x1, p0, p1);
-            } else {
-              p0 = ex2f(x0);
-              p1 = ex2f(x1);
-            }
+            const float p0 = ex2f(x0), p1 = ex2f(x1);
             pk[q] = pack2t<T>(p0, p1);
           }
           if (do_mask) {
@@ -920,11 +880,9 @@ int launch_ws(const AttnParams& p, cudaStream_t st) {
 
 }  // namespace
 
-bool attn_ws_supported(const AttnParams& p, int dtype) {
-  if (!attn_tc_supported(p, dtype)) return false;
+bool attn_ws_fits(const AttnParams& p) {
   const int dh = p.C / p.heads;
-  const WsSmem L = ws_layout((dh + 4 + 15) / 16, (dh + 1 + 15) / 16 * 16, kN + p.I, true);
-  return L.total <= 224u * 1024u;
+  return ws_layout((dh + 4 + 15) / 16, (dh + 1 + 15) / 16 * 16, kN + p.I, true).total <= 224u * 1024u;
 }
 
 template <typename T>

@@ -6,8 +6,6 @@
 //   forward : s = x (+ res) ; y = (s - mean) * rstd * gamma + beta ; saves mean, rstd   (also writes s if res)
 //   backward: dx = rstd * (g - mean(g) - xhat * mean(g * xhat)) (+ dres), g = dy * gamma ;
 //             dgamma += sum_rows dy * xhat ; dbeta += sum_rows dy   (register partials -> smem -> fp32 atomics)
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace pwa {
@@ -81,11 +79,10 @@ __device__ __forceinline__ float group_sum(float v) {
   return v;
 }
 
-// A row is handled by a group of G lanes, each lane owning NV vectors of EPV elements; every group works on R rows
-// per iteration with all of their loads issued before the first use (memory-level parallelism: these kernels are
-// pure HBM streams of 2-4 passes over [rows, C]).
-template <typename T, int G, int NV, int EPV, int R>
-__global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 16 ? 4 : (NV * EPV * R <= 32 ? 2 : 1))) ln_fwd_kernel(const T* __restrict__ x, const T* __restrict__ res,
+// A row is handled by a group of G lanes, each lane owning NV vectors of EPV elements, with all of its loads issued
+// before the first use (these kernels are pure HBM streams of 2-4 passes over [rows, C]).
+template <typename T, int G, int NV, int EPV>
+__global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 16 ? 4 : (NV * EPV <= 32 ? 2 : 1))) ln_fwd_kernel(const T* __restrict__ x, const T* __restrict__ res,
                                                             const float* __restrict__ gamma, const float* __restrict__ beta,
                                                             T* __restrict__ sum_out, T* __restrict__ y,
                                                             float* __restrict__ mean_out, float* __restrict__ rstd_out,
@@ -105,73 +102,66 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 16 ? 4 : (NV * EP
   const float invC = 1.f / (float)C;
   const bool has_res = res != nullptr;
   // the loop bound is uniform per CTA so that the sub-warp shuffles always run with all 32 lanes
-  for (long base = (long)blockIdx.x * (GPB * R); base < rows; base += (long)gridDim.x * (GPB * R)) {
-    float v[R][NV][EPV], rr[R][NV][EPV];
+  for (long base = (long)blockIdx.x * GPB; base < rows; base += (long)gridDim.x * GPB) {
+    const long row = base + gr;
+    float v[NV][EPV], rr[NV][EPV];
 #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const long row = base + r * GPB + gr;
+    for (int k = 0; k < NV; ++k) {
+      const int vi = gl + k * G;
 #pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const int vi = gl + k * G;
+      for (int e = 0; e < EPV; ++e) v[k][e] = rr[k][e] = 0.f;
+      if (vi < nvec && row < rows) {
+        Vec<T, EPV>::load(x + row * C + vi * EPV, v[k]);
+        if (has_res) Vec<T, EPV>::load(res + row * C + vi * EPV, rr[k]);
+      }
+    }
+    const bool live = row < rows;
+    float s = 0.f;
 #pragma unroll
-        for (int e = 0; e < EPV; ++e) v[r][k][e] = rr[r][k][e] = 0.f;
-        if (vi < nvec && row < rows) {
-          Vec<T, EPV>::load(x + row * C + vi * EPV, v[r][k]);
-          if (has_res) Vec<T, EPV>::load(res + row * C + vi * EPV, rr[r][k]);
+    for (int k = 0; k < NV; ++k) {
+      const int vi = gl + k * G;
+      if (vi < nvec && live) {
+        if (has_res) {
+#pragma unroll
+          for (int e = 0; e < EPV; ++e) v[k][e] += rr[k][e];
+          // the residual sum is stored in the I/O dtype and the statistics use the STORED value
+          Vec<T, EPV>::store(sum_out + row * C + vi * EPV, v[k]);
+          if (sizeof(T) == 2) {
+#pragma unroll
+            for (int e = 0; e < EPV; ++e) v[k][e] = to_f32(from_f32<T>(v[k][e]));
+          }
+        }
+#pragma unroll
+        for (int e = 0; e < EPV; ++e) s += v[k][e];
+      }
+    }
+    const float mean = group_sum<G>(s) * invC;
+    float q = 0.f;
+#pragma unroll
+    for (int k = 0; k < NV; ++k) {
+      const int vi = gl + k * G;
+      if (vi < nvec) {
+#pragma unroll
+        for (int e = 0; e < EPV; ++e) {
+          const float d = v[k][e] - mean;
+          q = fmaf(d, d, q);
         }
       }
     }
+    const float rstd = rsqrtf(group_sum<G>(q) * invC + eps);
 #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const long row = base + r * GPB + gr;
-      const bool live = row < rows;
-      float s = 0.f;
+    for (int k = 0; k < NV; ++k) {
+      const int vi = gl + k * G;
+      if (vi < nvec && live) {
+        float o[EPV];
 #pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const int vi = gl + k * G;
-        if (vi < nvec && live) {
-          if (has_res) {
-#pragma unroll
-            for (int e = 0; e < EPV; ++e) v[r][k][e] += rr[r][k][e];
-            // the residual sum is stored in the I/O dtype and the statistics use the STORED value
-            Vec<T, EPV>::store(sum_out + row * C + vi * EPV, v[r][k]);
-            if (sizeof(T) == 2) {
-#pragma unroll
-              for (int e = 0; e < EPV; ++e) v[r][k][e] = to_f32(from_f32<T>(v[r][k][e]));
-            }
-          }
-#pragma unroll
-          for (int e = 0; e < EPV; ++e) s += v[r][k][e];
-        }
+        for (int e = 0; e < EPV; ++e) o[e] = fmaf((v[k][e] - mean) * rstd, gm[k][e], bt[k][e]);
+        Vec<T, EPV>::store(y + row * C + vi * EPV, o);
       }
-      const float mean = group_sum<G>(s) * invC;
-      float q = 0.f;
-#pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const int vi = gl + k * G;
-        if (vi < nvec) {
-#pragma unroll
-          for (int e = 0; e < EPV; ++e) {
-            const float d = v[r][k][e] - mean;
-            q = fmaf(d, d, q);
-          }
-        }
-      }
-      const float rstd = rsqrtf(group_sum<G>(q) * invC + eps);
-#pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const int vi = gl + k * G;
-        if (vi < nvec && live) {
-          float o[EPV];
-#pragma unroll
-          for (int e = 0; e < EPV; ++e) o[e] = fmaf((v[r][k][e] - mean) * rstd, gm[k][e], bt[k][e]);
-          Vec<T, EPV>::store(y + row * C + vi * EPV, o);
-        }
-      }
-      if (gl == 0 && live) {
-        mean_out[row] = mean;
-        rstd_out[row] = rstd;
-      }
+    }
+    if (gl == 0 && live) {
+      mean_out[row] = mean;
+      rstd_out[row] = rstd;
     }
   }
 }
@@ -181,8 +171,8 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 16 ? 4 : (NV * EP
 // the gradient of `proj(...) + bias`, dres that of `mlp(...) + bias`), which saves two full reduction passes.
 // PLAIN: no residual-path gradient and no column sums (the PatchMerging norm, down.py:44: rows of 384-1536 channels, where
 // the three extra per-column register arrays of the general kernel meant spills and one CTA per SM)
-template <typename T, int G, int NV, int EPV, int R, bool PLAIN = false>
-__global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 8 ? 4 : (NV * EPV * R <= 16 ? 2 : 1))) ln_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ x,
+template <typename T, int G, int NV, int EPV, bool PLAIN = false>
+__global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 8 ? 4 : (NV * EPV <= 16 ? 2 : 1))) ln_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ x,
                                                             const float* __restrict__ gamma, const float* __restrict__ mean_in,
                                                             const float* __restrict__ rstd_in, const T* __restrict__ dres,
                                                             T* __restrict__ dx, float* __restrict__ dgamma,
@@ -195,7 +185,7 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 8 ? 4 : (NV * EPV
   const bool has_res = !PLAIN && dres != nullptr;
   const bool want_rs = !PLAIN && dres_colsum != nullptr && has_res, want_xs = !PLAIN && dx_colsum != nullptr;
   for (int i = threadIdx.x; i < 4 * C; i += kLnThreads) red[i] = 0.f;
-  constexpr int NVX = PLAIN ? 1 : NV, EPX = PLAIN ? 1 : EPV, RX = PLAIN ? 1 : R;     // (PLAIN: the extra arrays are never touched)
+  constexpr int NVX = PLAIN ? 1 : NV, EPX = PLAIN ? 1 : EPV;     // (PLAIN: the extra arrays are never touched)
   float gm[NV][EPV], ag[NV][EPV], ab[NV][EPV], ar[NVX][EPX], ax[NVX][EPX];
 #pragma unroll
   for (int k = 0; k < NV; ++k) {
@@ -208,70 +198,61 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV * R <= 8 ? 4 : (NV * EPV
     }
   }
   const float invC = 1.f / (float)C;
-  for (long base = (long)blockIdx.x * (GPB * R); base < rows; base += (long)gridDim.x * (GPB * R)) {
-    float d[R][NV][EPV], xv[R][NV][EPV], rs[RX][NVX][EPX];
-    float mean[R], rstd[R];
+  for (long base = (long)blockIdx.x * GPB; base < rows; base += (long)gridDim.x * GPB) {
+    const long row = base + gr;
+    const bool live = row < rows;
+    float d[NV][EPV], xv[NV][EPV], rs[NVX][EPX];
+    const float mean = live ? __ldg(mean_in + row) : 0.f;
+    const float rstd = live ? __ldg(rstd_in + row) : 0.f;
 #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const long row = base + r * GPB + gr;
-      const bool live = row < rows;
-      mean[r] = live ? __ldg(mean_in + row) : 0.f;
-      rstd[r] = live ? __ldg(rstd_in + row) : 0.f;
+    for (int k = 0; k < NV; ++k) {
+      const int vi = gl + k * G;
 #pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const int vi = gl + k * G;
-#pragma unroll
-        for (int e = 0; e < EPV; ++e) {
-          d[r][k][e] = xv[r][k][e] = 0.f;
-          if constexpr (!PLAIN) rs[r][k][e] = 0.f;
-        }
-        if (vi < nvec && live) {
-          Vec<T, EPV>::load(dy + row * C + vi * EPV, d[r][k]);
-          Vec<T, EPV>::load(x + row * C + vi * EPV, xv[r][k]);
-          if constexpr (!PLAIN) {
-            if (has_res) Vec<T, EPV>::load(dres + row * C + vi * EPV, rs[r][k]);
-          }
+      for (int e = 0; e < EPV; ++e) {
+        d[k][e] = xv[k][e] = 0.f;
+        if constexpr (!PLAIN) rs[k][e] = 0.f;
+      }
+      if (vi < nvec && live) {
+        Vec<T, EPV>::load(dy + row * C + vi * EPV, d[k]);
+        Vec<T, EPV>::load(x + row * C + vi * EPV, xv[k]);
+        if constexpr (!PLAIN) {
+          if (has_res) Vec<T, EPV>::load(dres + row * C + vi * EPV, rs[k]);
         }
       }
     }
+    float s1 = 0.f, s2 = 0.f;
 #pragma unroll
-    for (int r = 0; r < R; ++r) {
-      const long row = base + r * GPB + gr;
-      const bool live = row < rows;
-      float s1 = 0.f, s2 = 0.f;
+    for (int k = 0; k < NV; ++k) {
+      if (gl + k * G >= nvec) continue;                 // (dead rows hold zeros and mean = rstd = 0: they add nothing)
 #pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        if (gl + k * G >= nvec) continue;                 // (dead rows hold zeros and mean = rstd = 0: they add nothing)
+      for (int e = 0; e < EPV; ++e) {
+        const float xh = (xv[k][e] - mean) * rstd;
+        const float g = d[k][e] * gm[k][e];
+        xv[k][e] = xh;
+        s1 += g;
+        s2 = fmaf(g, xh, s2);
+        ag[k][e] = fmaf(d[k][e], xh, ag[k][e]);
+        ab[k][e] += d[k][e];
+        d[k][e] = g;
+      }
+    }
+    s1 = group_sum<G>(s1) * invC;
+    s2 = group_sum<G>(s2) * invC;
+#pragma unroll
+    for (int k = 0; k < NV; ++k) {
+      const int vi = gl + k * G;
+      if (vi < nvec && live) {
+        float o[EPV];
 #pragma unroll
         for (int e = 0; e < EPV; ++e) {
-          const float xh = (xv[r][k][e] - mean[r]) * rstd[r];
-          const float g = d[r][k][e] * gm[k][e];
-          xv[r][k][e] = xh;
-          s1 += g;
-          s2 = fmaf(g, xh, s2);
-          ag[k][e] = fmaf(d[r][k][e], xh, ag[k][e]);
-          ab[k][e] += d[r][k][e];
-          d[r][k][e] = g;
-        }
-      }
-      s1 = group_sum<G>(s1) * invC;
-      s2 = group_sum<G>(s2) * invC;
-#pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const int vi = gl + k * G;
-        if (vi < nvec && live) {
-          float o[EPV];
-#pragma unroll
-          for (int e = 0; e < EPV; ++e) {
-            o[e] = rstd[r] * (d[r][k][e] - s1 - xv[r][k][e] * s2);
-            if constexpr (!PLAIN) {
-              o[e] += rs[r][k][e];
-              ar[k][e] += rs[r][k][e];
-              ax[k][e] += o[e];
-            }
+          o[e] = rstd * (d[k][e] - s1 - xv[k][e] * s2);
+          if constexpr (!PLAIN) {
+            o[e] += rs[k][e];
+            ar[k][e] += rs[k][e];
+            ax[k][e] += o[e];
           }
-          Vec<T, EPV>::store(dx + row * C + vi * EPV, o);
         }
+        Vec<T, EPV>::store(dx + row * C + vi * EPV, o);
       }
     }
   }
@@ -622,11 +603,6 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel
   }
 }
 
-static int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-
 struct LnArgs {
   const void *a, *b, *res;
   const float *gamma, *bm, *rstd;
@@ -637,14 +613,14 @@ struct LnArgs {
   float eps;
 };
 
-template <typename T, int G, int NV, int EPV, int R>
+template <typename T, int G, int NV, int EPV>
 static int ln_launch(bool fwd, const LnArgs& a, cudaStream_t st) {
   constexpr int GPB = kLnThreads / G;
-  long blocks = (a.rows + GPB * R - 1) / (GPB * R);
+  long blocks = (a.rows + GPB - 1) / GPB;
   // backward: fewer CTAs -> fewer global atomics; with few rows (the late PatchMerging norms: 7 K rows of 768 channels) every
   // CTA should also run several iterations, or its epilogue (4C shared words zeroed, 2C..4C shared + global atomics)
   // outweighs its share of the rows: 48 -> see tools/bench_ln.py
-  long cap = 148L * (fwd ? env_int("PWA_LN_CAPF", 8) : env_int("PWA_LN_CAPB", 4));
+  long cap = 148L * (fwd ? 8 : 4);
   if (!fwd) {
     const long few = blocks / 6 > 148 ? blocks / 6 : (blocks < 148 ? blocks : 148);
     if (few < cap) cap = few;
@@ -652,88 +628,72 @@ static int ln_launch(bool fwd, const LnArgs& a, cudaStream_t st) {
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
   if (fwd) {
-    ln_fwd_kernel<T, G, NV, EPV, R><<<(unsigned)blocks, kLnThreads, 0, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm,
-                                                                              (T*)a.o1, (T*)a.o2, a.f1, a.f2, a.rows, a.C, a.eps);
+    ln_fwd_kernel<T, G, NV, EPV><<<(unsigned)blocks, kLnThreads, 0, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm,
+                                                                           (T*)a.o1, (T*)a.o2, a.f1, a.f2, a.rows, a.C, a.eps);
   } else {
     if constexpr (NV >= 2) {
       if (a.res == nullptr && a.f3 == nullptr && a.f4 == nullptr) {
-        ln_bwd_kernel<T, G, NV, EPV, R, true><<<(unsigned)blocks, kLnThreads, 4 * a.C * sizeof(float), st>>>(
+        ln_bwd_kernel<T, G, NV, EPV, true><<<(unsigned)blocks, kLnThreads, 4 * a.C * sizeof(float), st>>>(
             (const T*)a.a, (const T*)a.b, a.gamma, a.bm, a.rstd, nullptr, (T*)a.o1, a.f1, a.f2, nullptr, nullptr, a.rows, a.C);
         PWA_CUDA_OK(cudaGetLastError());
         return PWA_OK;
       }
     }
-    ln_bwd_kernel<T, G, NV, EPV, R><<<(unsigned)blocks, kLnThreads, 4 * a.C * sizeof(float), st>>>(
+    ln_bwd_kernel<T, G, NV, EPV><<<(unsigned)blocks, kLnThreads, 4 * a.C * sizeof(float), st>>>(
         (const T*)a.a, (const T*)a.b, a.gamma, a.bm, a.rstd, (const T*)a.res, (T*)a.o1, a.f1, a.f2, a.f3, a.f4, a.rows, a.C);
   }
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
 
-template <int G, int R, typename T>
-static int ln_launch_bulk_r(bool fwd, const LnArgs& a, cudaStream_t st) {
-  constexpr int TR = kLnThreads / G * R;
+// Rows per lane group and iteration of the bulk kernels, measured (tools/bench_ln.py): R = 2 is 8-13 % faster in backward,
+// within +-5 % in forward.  At most 4 CTAs per SM forward, 2 backward (the bytes in flight no longer depend on the occupancy).
+template <int G, typename T>
+static int ln_launch_bulk(bool fwd, const LnArgs& a, cudaStream_t st) {
+  constexpr int RF = 1, RB = 2;
+  const int R = fwd ? RF : RB, TR = kLnThreads / G * R;
   const int nop = fwd ? (a.res ? 2 : 1) : (a.res ? 3 : 2);
-  // (backward epilogue: the per-warp column sums, 8 x 4 x C floats, reuse the ring memory: >= 192 * C bytes for every G, R)
+  // (backward epilogue: the per-warp column sums, 8 x 4 x C floats, reuse the ring memory: >= 192 * C bytes for every G)
   const size_t smem = (size_t)(kMaxStages / nop / R) * nop * TR * a.C * 2;
   long blocks = (a.rows + TR - 1) / TR;
-  // (backward: 3 CTAs/SM = 85 registers, no spills; the bytes in flight no longer depend on the occupancy)
-  const long cap = 148L * (fwd ? env_int("PWA_LN_BULK_CTAS_F", R == 1 ? 4 : 3) : env_int("PWA_LN_BULK_CTAS_B", R == 1 ? 3 : 2));
+  const long cap = 148L * (fwd ? 4 : 2);
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
   if (fwd) {
-    PWA_CUDA_OK(cudaFuncSetAttribute(ln_fwd_bulk_kernel<G, R, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ln_fwd_bulk_kernel<G, R, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm, (T*)a.o1,
-                                                                         (T*)a.o2, a.f1, a.f2, a.rows, a.C, a.eps);
+    PWA_CUDA_OK(cudaFuncSetAttribute(ln_fwd_bulk_kernel<G, RF, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ln_fwd_bulk_kernel<G, RF, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm,
+                                                                          (T*)a.o1, (T*)a.o2, a.f1, a.f2, a.rows, a.C, a.eps);
   } else {
-    PWA_CUDA_OK(cudaFuncSetAttribute(ln_bwd_bulk_kernel<G, R, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ln_bwd_bulk_kernel<G, R, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.b, a.gamma, a.bm, a.rstd,
-                                                                         (const T*)a.res, (T*)a.o1, a.f1, a.f2, a.f3, a.f4, a.rows, a.C);
+    PWA_CUDA_OK(cudaFuncSetAttribute(ln_bwd_bulk_kernel<G, RB, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ln_bwd_bulk_kernel<G, RB, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.b, a.gamma, a.bm, a.rstd,
+                                                                          (const T*)a.res, (T*)a.o1, a.f1, a.f2, a.f3, a.f4, a.rows, a.C);
   }
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
 
-template <int G, typename T>
-static int ln_launch_bulk(bool fwd, const LnArgs& a, cudaStream_t st) {
-  // measured (tools/bench_ln.py): R = 2 is 8-13 % faster in backward, within +-5 % in forward
-  static const int rf = env_int("PWA_LN_BULK_RF", 1), rb = env_int("PWA_LN_BULK_RB", 2);
-  if ((fwd ? rf : rb) == 2) return ln_launch_bulk_r<G, 2, T>(fwd, a, st);
-  return ln_launch_bulk_r<G, 1, T>(fwd, a, st);
-}
-
 template <typename T, int EPV>
 static int ln_dispatch_v(bool fwd, const LnArgs& a, cudaStream_t st) {
   const int nvec = a.C / EPV;
+#define LN_CASE(G, NV) return ln_launch<T, G, NV, EPV>(fwd, a, st)
   if constexpr (sizeof(T) == 2 && EPV == 8) {
-    // one vector per lane, rows contiguous: the bulk-copy kernels (PWA_LN_BULK=0 selects the register kernels)
-    static const int use_bulk = env_int("PWA_LN_BULK", 1);
-    if (use_bulk && nvec <= 32) {
-      if (nvec <= 4) return ln_launch_bulk<4, T>(fwd, a, st);
-      if (nvec <= 8) return ln_launch_bulk<8, T>(fwd, a, st);
-      if (nvec <= 16) return ln_launch_bulk<16, T>(fwd, a, st);
-      return ln_launch_bulk<32, T>(fwd, a, st);
-    }
+    // one vector per lane, rows contiguous: the bulk-copy kernels
+    if (nvec <= 4) return ln_launch_bulk<4, T>(fwd, a, st);
+    if (nvec <= 8) return ln_launch_bulk<8, T>(fwd, a, st);
+    if (nvec <= 16) return ln_launch_bulk<16, T>(fwd, a, st);
+    if (nvec <= 32) return ln_launch_bulk<32, T>(fwd, a, st);
+  } else {
+    if (nvec <= 4) LN_CASE(4, 1);
+    if (nvec <= 8) LN_CASE(8, 1);
+    if (nvec <= 16) LN_CASE(16, 1);
+    if (nvec <= 32) LN_CASE(32, 1);
   }
-  const int R = env_int(fwd ? "PWA_LN_RF" : "PWA_LN_RB", 1);       // rows per group per iteration (tuning knob)
-#define LN_CASE(G, NV, R) return ln_launch<T, G, NV, EPV, R>(fwd, a, st)
-#define LN_CASE_R(G)                    \
-  do {                                  \
-    if (R >= 4) LN_CASE(G, 1, 4);       \
-    if (R == 2) LN_CASE(G, 1, 2);       \
-    LN_CASE(G, 1, 1);                   \
-  } while (0)
-  if (nvec <= 4) LN_CASE_R(4);
-  if (nvec <= 8) LN_CASE_R(8);
-  if (nvec <= 16) LN_CASE_R(16);
-  if (nvec <= 32) LN_CASE_R(32);
-  if (nvec <= 64) LN_CASE(32, 2, 1);
-  if (nvec <= 128) LN_CASE(32, 4, 1);
+  if (nvec <= 64) LN_CASE(32, 2);
+  if (nvec <= 128) LN_CASE(32, 4);
   // C in (1024, 2048]: PatchMerging norms of wide stages (8 * 192 = 1536, 4 * 384 = 1536, down.py:13-14); these rows
   // live in more registers than a thread has (spills) -- rare shapes, correctness over speed
-  if (nvec <= 256) LN_CASE(32, 8, 1);
-  if (EPV == 4 && nvec <= 512) LN_CASE(32, 16, 1);
-#undef LN_CASE_R
+  if (nvec <= 256) LN_CASE(32, 8);
+  if (EPV == 4 && nvec <= 512) LN_CASE(32, 16);
 #undef LN_CASE
   set_error("layer norm: C=%d too large (max 2048)", a.C);
   return PWA_ERR_UNSUPPORTED;
@@ -743,7 +703,7 @@ template <typename T>
 static int ln_dispatch(bool fwd, const LnArgs& a, cudaStream_t st) {
   if constexpr (sizeof(T) == 2) {
     const uintptr_t al = (uintptr_t)a.a | (uintptr_t)a.b | (uintptr_t)a.res | (uintptr_t)a.o1 | (uintptr_t)a.o2;
-    if (a.C % 8 == 0 && (al & 15) == 0 && env_int("PWA_LN_EPV", 8) == 8) return ln_dispatch_v<T, 8>(fwd, a, st);
+    if (a.C % 8 == 0 && (al & 15) == 0) return ln_dispatch_v<T, 8>(fwd, a, st);
   }
   return ln_dispatch_v<T, 4>(fwd, a, st);
 }

@@ -15,8 +15,6 @@
 // whole D-lines, the token side moves runs of ww*wd*CT contiguous elements per window.
 // All traffic is 32-bit words (one fp32 or a pair of bf16 channels); bf16 needs a 2x2 in-register
 // transpose (PRMT) because x is contiguous along D and tokens along C.
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace pwa {
@@ -587,8 +585,7 @@ static int run(bool is_partition, const void* src, const void* src2, void* dst, 
   // `use_crop_lo & 2` forces the generic kernel, `& 4` the word kernel, `& 8` the vector kernel (tests cross-check
   // the paths); otherwise the TMA-staged kernel (partition_tma.cu) takes every shape inside its envelope
   cudaStream_t st0 = (cudaStream_t)stream;
-  static const bool no_tma = getenv("PWA_NO_TMA") != nullptr;
-  if (!(use_crop_lo & (2 | 4 | 8)) && !no_tma) {
+  if (!(use_crop_lo & (2 | 4 | 8))) {
     const int32_t* lo = (use_crop_lo & 1) ? g->crop_lo : g->data_lo;
     const int rc = partition_tma_run(is_partition, src, src2, dst, B, C, g, lo, eb, dtype == PWA_F16, st0);
     if (rc != PWA_ERR_UNSUPPORTED) return rc;

@@ -14,8 +14,9 @@
 // partition:  TMA load -> smem [c][a'][D_box]  --transpose-->  smem token blocks  -> coalesced 16-byte stores
 // reverse  :  coalesced 16-byte loads (+ fused residual add) -> smem token blocks --transpose--> smem [c][a'][D_box]
 //             -> TMA store
-// Persistent CTAs, 2-4 per SM; the partition kernel can keep up to 3 more TMA loads in flight behind an mbarrier
-// (PWA_TMA_STAGES; measured no faster than more resident CTAs).  Pure byte movement: bit-exact by construction.
+// Persistent CTAs, 2-4 per SM, one staged tile each: the partition kernel issues the next tile's TMA load as soon as the
+// current one has left shared memory (a deeper ring of loads was measured no faster than more resident CTAs).  Pure byte
+// movement: bit-exact by construction.
 //
 // Shared-memory layouts are chosen so that both sides of the transposition are bank-conflict free:
 //   * D_box = padded line length rounded up to an ODD number of 16-byte chunks: lanes that differ in a' hit
@@ -23,7 +24,6 @@
 //   * token blocks (window p3, w' position t2) hold wd tokens x CT channels and are padded to a pitch of
 //     4 (mod 32) words: lanes that differ in t2 hit different banks on the 4-byte side.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "tc_common.cuh"
@@ -38,7 +38,6 @@ namespace {
 // 1024 threads made it slower), i.e. the kernels are bound by the TMA line rate for short lines, not by the SM side.
 constexpr int kPartThreads = 256;
 constexpr int kRevThreads = 256;
-constexpr int kMaxStages = 4;
 constexpr int kWW = 8;            // lanes are mapped as (a' = lane & 7, channel word = lane >> 3)
 
 struct TmaPartParams {
@@ -51,11 +50,9 @@ struct TmaPartParams {
   int dbox;          // elements per staged line
   int cw;            // channel words per token in this chunk (CT * eb / 4)
   int bp;            // token block pitch in words
-  int src_bytes;     // one staged x tile, rounded up to 128 bytes (stage pitch)
+  int src_bytes;     // one staged x tile, rounded up to 128 bytes
   int box_bytes;     // exact bytes one TMA box transfers
-  int nstage;
   int ntiles;
-  int nsplit;        // TMA boxes per tile (split along channels: several requests in flight per tile)
   int d0, dsh;       // TMA start coordinate along D (16-byte aligned, <= -lod) and the column shift it leaves: column j = dp + dsh
   FastDiv div_perblk, div_cpt;
 };
@@ -119,7 +116,7 @@ struct Carve {
 __device__ __forceinline__ Carve carve(uint8_t* smem, const TmaPartParams& p) {
   Carve c;
   c.src = smem;
-  c.dst = reinterpret_cast<uint32_t*>(smem + (size_t)p.nstage * p.src_bytes);
+  c.dst = reinterpret_cast<uint32_t*>(smem + p.src_bytes);
   c.doff = reinterpret_cast<int*>(c.dst + (size_t)p.P3 * kWW * p.bp);
   return c;
 }
@@ -226,43 +223,30 @@ template <int EB>
 __global__ void __launch_bounds__(kPartThreads, 4) partition_tma_kernel(const __grid_constant__ CUtensorMap xmap,
                                                                     uint32_t* __restrict__ tok, const TmaPartParams p) {
   extern __shared__ __align__(128) uint8_t smem[];
-  __shared__ __align__(8) uint64_t full[kMaxStages];
+  __shared__ __align__(8) uint64_t full;
   const Carve cv = carve(smem, p);
   const int tid = threadIdx.x;
   fill_doff(cv.doff, p);
   if (tid == 0) {
-    for (int i = 0; i < kMaxStages; ++i) mbar_init(&full[i], 1);
+    mbar_init(&full, 1);
     fence_mbar_init();
   }
   __syncthreads();
-  auto issue = [&](int tile, int stage) {
+  auto issue = [&](int tile) {
     const Tile t(p, tile);
     if (!t.h_ok) return;                                   // a padding row: nothing to load, the tile is all zeros
-    mbar_expect_tx(&full[stage], (uint32_t)p.box_bytes);
-    const int cs = p.CT / p.nsplit, piece_bytes = p.box_bytes / p.nsplit;
-    for (int k = 0; k < p.nsplit; ++k)
-      tma_load_5d(cv.src + (size_t)stage * p.src_bytes + (size_t)k * piece_bytes, &xmap, &full[stage], p.d0, t.r, t.a0, t.h,
-                  t.b * p.C + t.chunk * p.CT + k * cs);
+    mbar_expect_tx(&full, (uint32_t)p.box_bytes);
+    tma_load_5d(cv.src, &xmap, &full, p.d0, t.r, t.a0, t.h, t.b * p.C + t.chunk * p.CT);
   };
-  // prologue: nstage - 1 tiles in flight
-  if (tid == 0)
-    for (int k = 0; k < p.nstage - 1 || k == 0; ++k) {
-      const int tile = blockIdx.x + k * gridDim.x;
-      if (tile < p.ntiles && (k == 0 || p.nstage > 1)) issue(tile, k);
-    }
-  uint32_t phase = 0u;                                     // bit s = parity to wait for on stage s
+  if (tid == 0 && blockIdx.x < p.ntiles) issue(blockIdx.x);
+  uint32_t phase = 0u;
   const uint32_t npieces = (uint32_t)p.P3 * kWW * p.div_perblk.d;
-  int it = 0;
-  for (int tile = blockIdx.x; tile < p.ntiles; tile += gridDim.x, ++it) {
-    const int stage = it % p.nstage;
-    const int next = tile + (p.nstage > 1 ? p.nstage - 1 : 1) * gridDim.x;
-    // the stage being refilled was last read by the transposition of the previous tile, which ended before its barrier (B)
-    if (p.nstage > 1 && tid == 0 && next < p.ntiles) issue(next, (it + p.nstage - 1) % p.nstage);
+  for (int tile = blockIdx.x; tile < p.ntiles; tile += gridDim.x) {
     const Tile t(p, tile);
     if (t.h_ok) {
-      mbar_wait(&full[stage], (phase >> stage) & 1u);
-      phase ^= 1u << stage;
-      transpose_tile<EB, true, kPartThreads>(cv.src + (size_t)stage * p.src_bytes, cv.dst, cv.doff, p, t.q);
+      mbar_wait(&full, phase);
+      phase ^= 1u;
+      transpose_tile<EB, true, kPartThreads>(cv.src, cv.dst, cv.doff, p, t.q);
     } else {
       for (uint32_t i = tid; i < (uint32_t)p.P3 * kWW * p.bp / 4; i += kPartThreads)
         reinterpret_cast<uint4*>(cv.dst)[i] = make_uint4(0, 0, 0, 0);
@@ -272,8 +256,8 @@ __global__ void __launch_bounds__(kPartThreads, 4) partition_tma_kernel(const __
       const Piece pc = piece(p, t, i);
       *reinterpret_cast<uint4*>(tok + pc.goff) = *reinterpret_cast<const uint4*>(cv.dst + pc.soff);
     }
-    __syncthreads();                                       // (C) token blocks and this stage are free again
-    if (p.nstage == 1 && tid == 0 && next < p.ntiles) issue(next, 0);
+    __syncthreads();                                       // (C) token blocks and the staged tile are free again
+    if (tid == 0 && tile + (int)gridDim.x < p.ntiles) issue(tile + gridDim.x);
   }
 }
 
@@ -357,6 +341,11 @@ EncodeTiledFn encode_fn() {
   return fn;
 }
 
+// staged x tile + token blocks + line offset table
+size_t smem_bytes(const TmaPartParams& p) {
+  return (size_t)p.src_bytes + (size_t)p.P3 * kWW * p.bp * 4 + (size_t)p.dbox * 4 + 16;
+}
+
 // Measured (profiles/r1_tma_partition.md): two or more resident CTAs per SM beat one CTA with a 3-deep TMA pipeline
 // (24 vs 29 us), so a tile (one staged x box + the token blocks) is sized for >= 2 CTAs per SM when the shape allows.
 constexpr size_t kSmemBudget = 200 * 1024;
@@ -396,39 +385,26 @@ bool plan(TmaPartParams& p, int B, int C, const pwa_geom* g, const int32_t* lo, 
     p.bp = blk + ((36 - blk % 32) % 32);                           // pitch = 4 (mod 32) words, a multiple of 4
     p.box_bytes = ct * kWW * p.dbox * eb;
     p.src_bytes = (p.box_bytes + 127) & ~127;
-    const size_t dst_bytes = (size_t)p.P3 * kWW * p.bp * 4, tab = (size_t)p.dbox * 4 + 16;
-    static const int max_stages = getenv("PWA_TMA_STAGES") ? atoi(getenv("PWA_TMA_STAGES")) : 1;
-    static const int want_split = getenv("PWA_TMA_SPLIT") ? atoi(getenv("PWA_TMA_SPLIT")) : 1;
-    for (int ns = max_stages < kMaxStages ? max_stages : kMaxStages; ns >= 1; --ns) {
-      if ((size_t)ns * p.src_bytes + dst_bytes + tab <= (pass == 0 ? kSmemTwoCtas : kSmemBudget)) {
-        p.nstage = ns;
-        p.nsplit = 1;
-        for (int k = want_split; k > 1; k /= 2)
-          if (ct % k == 0 && (p.box_bytes / k) % 128 == 0) { p.nsplit = k; break; }
-        const int cpt = p.cw / 4;
-        if ((size_t)p.P3 * kWW * p.wd * cpt >= 65536) return false;
-        p.div_perblk = FastDiv(p.wd * cpt);
-        p.div_cpt = FastDiv(cpt);
-        p.ntiles = B * p.Hp * p.P2 * p.nchunk;
-        return true;
-      }
+    if (smem_bytes(p) <= (pass == 0 ? kSmemTwoCtas : kSmemBudget)) {
+      const int cpt = p.cw / 4;
+      if ((size_t)p.P3 * kWW * p.wd * cpt >= 65536) return false;
+      p.div_perblk = FastDiv(p.wd * cpt);
+      p.div_cpt = FastDiv(cpt);
+      p.ntiles = B * p.Hp * p.P2 * p.nchunk;
+      return true;
     }
   }
   return false;
 }
 
-size_t smem_bytes(const TmaPartParams& p, int nstage) {
-  return (size_t)nstage * p.src_bytes + (size_t)p.P3 * kWW * p.bp * 4 + (size_t)p.dbox * 4 + 16;
-}
-
-bool make_map(CUtensorMap* map, const void* x, const TmaPartParams& p, int eb, int nsplit) {
+bool make_map(CUtensorMap* map, const void* x, const TmaPartParams& p, int eb) {
   EncodeTiledFn enc = encode_fn();
   if (!enc) return false;
   const cuuint64_t dims[5] = {(cuuint64_t)p.D, (cuuint64_t)p.P2, (cuuint64_t)(p.W / p.P2), (cuuint64_t)p.H,
                               (cuuint64_t)p.B * p.C};
   const cuuint64_t strides[4] = {(cuuint64_t)p.D * eb, (cuuint64_t)p.P2 * p.D * eb, (cuuint64_t)p.W * p.D * eb,
                                  (cuuint64_t)p.H * p.W * p.D * eb};
-  const cuuint32_t box[5] = {(cuuint32_t)p.dbox, 1u, (cuuint32_t)kWW, 1u, (cuuint32_t)(p.CT / nsplit)};
+  const cuuint32_t box[5] = {(cuuint32_t)p.dbox, 1u, (cuuint32_t)kWW, 1u, (cuuint32_t)p.CT};
   const cuuint32_t es[5] = {1u, 1u, 1u, 1u, 1u};
   const CUresult rc = enc(map, eb == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT32, 5, const_cast<void*>(x),
                           dims, strides, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
@@ -454,13 +430,9 @@ int partition_tma_run(bool is_partition, const void* src, const void* src2, void
   if (!plan(p, B, C, g, lo, eb)) return PWA_ERR_UNSUPPORTED;
   const void* xptr = is_partition ? src : dst;
   if (((uintptr_t)src | (uintptr_t)src2 | (uintptr_t)dst) & 15) return PWA_ERR_UNSUPPORTED;
-  if (!is_partition) {
-    p.nstage = 1;                                        // the reverse kernel stages one tile at a time
-    p.nsplit = 1;
-  }
   CUtensorMap map;
-  if (!make_map(&map, xptr, p, eb, p.nsplit)) return PWA_ERR_UNSUPPORTED;
-  const size_t smem = smem_bytes(p, p.nstage);
+  if (!make_map(&map, xptr, p, eb)) return PWA_ERR_UNSUPPORTED;
+  const size_t smem = smem_bytes(p);
   int per_sm = (int)((227 * 1024) / (smem + 1024));
   per_sm = per_sm < 1 ? 1 : (per_sm > 4 ? 4 : per_sm);
   int grid = 148 * per_sm;

@@ -118,7 +118,7 @@ def _run_ln(x, res, gamma, beta, dy, dres, want_rs, want_xs, dtype, detect=False
 # ---------------------------------------------------------------------------------------------------------------------
 # B. the LayerNorm branch table
 # ---------------------------------------------------------------------------------------------------------------------
-# C -> kernel under the default environment (ln_dispatch / ln_dispatch_v in csrc/ln.cu are the source of truth).
+# C -> kernel (ln_dispatch / ln_dispatch_v in csrc/ln.cu are the source of truth).
 # 16-bit rows with C % 8 == 0 and 16-byte aligned pointers take EPV = 8 (nvec = C / 8):
 #   nvec <= 32  -> bulk-copy kernels ln_{fwd,bwd}_bulk_kernel, G = 4 (C <= 32), 8 (C <= 64), 16 (C <= 128), 32 (C <= 256)
 #   nvec > 32   -> register kernels, G = 32: NV = 2 (C <= 512), 4 (C <= 1024), 8 (C <= 2048)
@@ -196,19 +196,19 @@ def test_layer_norm_zero_rows(dtype, C):
 # C. column reductions where every CTA loops
 # ---------------------------------------------------------------------------------------------------------------------
 def _ln_tiles(dtype, C, rows, fwd, with_res):
-    """(tiles, CTAs, ring stages) of the default LayerNorm launch; restates ln_dispatch / ln_launch_bulk_r / ln_launch in
-    csrc/ln.cu with no PWA_LN_* variable set (register kernels have no ring: stages = 1)."""
-    if dtype != F32 and C % 8 == 0 and C <= 256:          # bulk-copy kernels: PWA_LN_BULK_RF = 1, PWA_LN_BULK_RB = 2
+    """(tiles, CTAs, ring stages) of the LayerNorm launch; restates ln_dispatch / ln_launch_bulk / ln_launch in csrc/ln.cu
+    (register kernels have no ring: stages = 1)."""
+    if dtype != F32 and C % 8 == 0 and C <= 256:          # bulk-copy kernels: R = 1 rows per lane group forward, 2 backward
         nvec = C // 8
         G = 4 if nvec <= 4 else 8 if nvec <= 8 else 16 if nvec <= 16 else 32
         R_ = 1 if fwd else 2
         nop = (2 if with_res else 1) if fwd else (3 if with_res else 2)
         tiles = -(-rows // (256 // G * R_))
-        cap = 148 * ((4 if R_ == 1 else 3) if fwd else (3 if R_ == 1 else 2))
+        cap = 148 * (4 if fwd else 2)
         return tiles, max(1, min(tiles, cap)), 12 // nop // R_
     nvec = C // (8 if dtype != F32 and C % 8 == 0 else 4)
     G = 4 if nvec <= 4 else 8 if nvec <= 8 else 16 if nvec <= 16 else 32
-    tiles = -(-rows // (256 // G))                        # PWA_LN_RF = PWA_LN_RB = 1
+    tiles = -(-rows // (256 // G))                        # register kernels: one row per lane group
     cap = 148 * (8 if fwd else 4)
     if not fwd:
         few = tiles // 6 if tiles // 6 > 148 else min(tiles, 148)

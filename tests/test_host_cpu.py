@@ -3,6 +3,7 @@ include/pwa.h declares, the C host logic (geometry / region ids / index maps) is
 golden vectors from the live reference, and the nn.Module mirror keeps the reference's state-dict keys.
 No compute call that needs a GPU is made here."""
 import ctypes
+import json
 import os
 import re
 
@@ -26,6 +27,44 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), f"{name} declared in include/pwa.h but not exported"
     assert set(pwa_b200._lib.EXPORTED_SYMBOLS) == declared
     assert lib.pwa_version() == 100
+
+
+# Grid of pwa_attn_tc_supported queries: head dims, prompt counts and windows inside and around the tcgen05 envelope
+# (N = 256 windows that fail the wd <= 4 or wh + ww <= 16 limits, and N != 256), every dtype code, without and with
+# attention dropout.  The query takes no mask: the budgets are those of the masked kernels, which need the most memory.
+ENVELOPE_GRID = dict(dh=[2, 3, 4, 6, 8, 12, 16, 24, 32, 48, 64], I=[0, 16, 32, 64, 96, 128, 160],
+                     ws=[(8, 8, 4), (4, 8, 8), (8, 4, 8), (16, 4, 4), (16, 16, 1), (8, 16, 2), (4, 4, 4), (8, 8, 8), (7, 7, 7)],
+                     dtype=[pwa_b200._lib.PWA_F32, pwa_b200._lib.PWA_BF16, pwa_b200._lib.PWA_F16, 3], p_drop=[0.0, 0.1])
+
+
+def attn_tc_envelope(lib):
+    """[dh, I, ws, dtype, p_drop] of every ENVELOPE_GRID point that `lib.pwa_attn_tc_supported` accepts."""
+    heads, out = 4, []
+    for dh in ENVELOPE_GRID["dh"]:
+        for I in ENVELOPE_GRID["I"]:
+            for ws in ENVELOPE_GRID["ws"]:
+                for dtype in ENVELOPE_GRID["dtype"]:
+                    for p_drop in ENVELOPE_GRID["p_drop"]:
+                        s = pwa_b200._lib.PwaAttnShape(B=2, P=8, C=dh * heads, heads=heads, I=I, scale=dh ** -0.5, p_drop=p_drop)
+                        s.ws[:] = ws
+                        if lib.pwa_attn_tc_supported(ctypes.byref(s), dtype):
+                            out.append([dh, I, list(ws), dtype, p_drop])
+    return out
+
+
+def test_attn_tc_envelope_is_pinned():
+    """The shapes and dtypes that run on the tcgen05 attention kernels (forward and backward) are exactly those of the
+    recorded table (tests/golden/attn_tc_envelope.json, taken from the library when the envelope was still decided in
+    three places: the round-1 forward's shape and budget checks, then those of the warp-specialised forward and the
+    backward).  The library answers without a GPU."""
+    with open(os.path.join(ROOT, "tests", "golden", "attn_tc_envelope.json")) as f:
+        ref = json.load(f)
+    assert ref["grid"] == json.loads(json.dumps(ENVELOPE_GRID))
+    lib = pwa_b200._lib.lib
+    got = attn_tc_envelope(lib)
+    assert got == ref["supported"]
+    # the stage shapes of the model are inside: head dim 3-48 at the 8x8x4 window, 0-128 prompt tokens, bf16 and fp16
+    assert len(got) == 5 * 5 * 2 * 2
 
 
 @pytest.mark.parametrize("name", golden_names("geo_"))

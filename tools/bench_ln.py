@@ -1,6 +1,5 @@
 """LayerNorm kernel device time at the BASELINE stage shapes (run on the GPU box): raw C-ABI calls captured in a CUDA
-graph (20 launches per replay, rotating buffers larger than L2).  Tuning knobs (env): PWA_LN_RF / PWA_LN_RB (rows per
-lane group per iteration), PWA_LN_EPV (8 = 16-byte bf16 vectors), PWA_LN_CAPF / PWA_LN_CAPB (CTAs per SM)."""
+graph (20 launches per replay, rotating buffers larger than L2)."""
 import ctypes as C, json, os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -24,7 +23,6 @@ def graph_time(fn, reps=20):
     e0.record(); g.replay(); g.replay(); e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / (2 * reps) * 1e3
 
-env = {k: os.environ.get(k) for k in ("PWA_LN_RF", "PWA_LN_RB", "PWA_LN_EPV", "PWA_LN_CAPF", "PWA_LN_CAPB") if os.environ.get(k)}
 for rows, Cc in ((4 * 432 * 256, 48), (4 * 54 * 256, 96), (4 * 28 * 256, 192), (4 * 13824, 384), (4 * 1728, 768)):
     dt = torch.bfloat16
     mk = lambda: [torch.randn(rows, Cc, device=dev).to(dt) for _ in range(NB)]
@@ -48,6 +46,6 @@ for rows, Cc in ((4 * 432 * 256, 48), (4 * 54 * 256, 96), (4 * 28 * 256, 192), (
     fwd(0); torch.cuda.synchronize()
     nb = rows * Cc * 2
     t = [graph_time(f) for f in (fwd, fwd_res, bwd, bwd_res)]
-    print(json.dumps({"rows": rows, "C": Cc, "env": env, "fwd_us": round(t[0], 1), "fwd_GBs": round(2 * nb / t[0] / 1e3),
+    print(json.dumps({"rows": rows, "C": Cc, "fwd_us": round(t[0], 1), "fwd_GBs": round(2 * nb / t[0] / 1e3),
                       "fwd_res_us": round(t[1], 1), "fwd_res_GBs": round(4 * nb / t[1] / 1e3), "bwd_us": round(t[2], 1),
                       "bwd_GBs": round(3 * nb / t[2] / 1e3), "bwd_res_us": round(t[3], 1), "bwd_res_GBs": round(4 * nb / t[3] / 1e3)}))

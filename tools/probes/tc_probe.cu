@@ -1,4 +1,4 @@
-// Stand-alone probe for the tcgen05 building blocks used by attn_tc.cu (run on a B200):
+// Stand-alone probe for the tcgen05 building blocks of the attention kernels (run on a B200):
 //   S[128x128] = A[128x32] * B[128x32]^T   (SS MMA, K-major no-swizzle operands, 2 k-steps)  -> tcgen05.ld
 //   P = bf16(S * 0.01) -> tcgen05.st (packed bf16x2) ; O[128x16] = P * V[128x16]  (TS MMA, A from TMEM)
 // usage: tc_probe <variant>    bit0: swap LBO/SBO of the K-major operands
