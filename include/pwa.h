@@ -121,7 +121,8 @@ int pwa_colsum_f32(const float* src, float* dst, int S, int64_t n, void* stream)
 /* dst[c] = sum over r < rows of x[r][c]: x [rows][C] bf16, fp16 or fp32 (dtype), dst [C] fp32, both on the
  * DEVICE; dst is zeroed by the call.  The bias gradient of the q|k|v projection (window_attention.py:28-30: nn.Linear with
  * bias; torch autograd sums the packed dq|dk|dv rows over all tokens there).  C must be a multiple of the elements per
- * 16 bytes (8 for bf16 / fp16, 4 for fp32) and at most 512 such vectors; x 16-byte aligned.  fp32 atomics: the sum order is not fixed. */
+ * 16 bytes (8 for bf16 / fp16, 4 for fp32) and at most 512 such vectors; x 16-byte aligned.  fp32 atomics: the sum order is not fixed
+ * (pwa_colsum_rows_det fixes it). */
 int pwa_colsum_rows(const void* x, float* dst, int64_t rows, int C, int dtype, void* stream);
 
 /* y[i] = keep(i) ? x[i] / keep_rate : 0 for i < n, keep(i) a counter-based hash of the two uint32 words at seed_dev (DEVICE
@@ -282,6 +283,51 @@ int pwa_attn_dense_fwd(const void* q, const void* k, const void* v, const float*
 int pwa_attn_dense_bwd(const void* q, const void* k, const void* v, const float* bias, const float* mask, const void* out,
                        const float* lse, const void* dout, void* dq, void* dk, void* dv, float* dbias, float* delta,
                        const pwa_dense_attn* s, int dtype, void* stream);
+
+/* ---- deterministic reductions (torch.use_deterministic_algorithms) ----------------------------------------------------- */
+
+/* The entry points above that return fp32 sums over CTAs (pwa_attn_bwd's dkp, dvp, dth, dtw, dtd, dtok; the column sums of
+ * pwa_ln_bwd2, pwa_dropout_colsum and pwa_colsum_rows) add per-CTA partials with float atomics, so the last bits of those sums
+ * depend on scheduling.  Each has a sibling, `<name>_det`, that returns the same sums bitwise reproducibly: every CTA writes
+ * its partials in a fixed order to its own slot of a caller-provided DEVICE workspace, and a second pass (pwa_colsum_f32)
+ * sums the slots in index order.  A result is reproduced for the same GPU model, library build and shape.
+ *   - `<name>_det_workspace_size` returns the bytes the sibling needs (0 = none, NULL allowed) or a negative error code.  It
+ *     needs no GPU.  A workspace smaller than that makes the sibling return PWA_ERR_ARG.
+ *   - the siblings keep every other contract of their entry point: the same arguments and outputs, the caller's stream, no
+ *     allocation and no synchronisation (they can be captured into a CUDA graph); the workspace contents on entry do not
+ *     matter.
+ *   - pwa_attn_bwd_det runs the tcgen05 kernel only (no `impl` argument): outside pwa_attn_tc_supported it returns
+ *     PWA_ERR_UNSUPPORTED.  The fp32-math and dense-argument attention backwards have no deterministic form.
+ *   - pwa_bias_tables_bwd has no cross-CTA sums; its sibling replaces the shared-memory atomics of the per-distance table
+ *     gradient by fixed-order sums and needs no workspace. */
+int64_t pwa_attn_bwd_det_workspace_size(const pwa_attn_shape* s, int dtype);
+int pwa_attn_bwd_det(const void* q, const void* k, const void* v, const void* kp, const void* vp,
+                     const float* th, const float* tw, const float* td, const float* tok,
+                     const uint8_t* ids, const void* out, const float* lse, const void* dout,
+                     void* dq, void* dk, void* dv, float* dkp, float* dvp,
+                     float* dth, float* dtw, float* dtd, float* dtok, float* delta,
+                     void* workspace, int64_t workspace_bytes, const pwa_attn_shape* s, int dtype, void* stream);
+
+int64_t pwa_ln_bwd2_det_workspace_size(int64_t rows, int C, int dtype);
+int pwa_ln_bwd2_det(const void* dy, const void* x, const float* gamma, const float* mean, const float* rstd,
+                    const void* dres, void* dx, float* dgamma, float* dbeta, float* dres_colsum, float* dx_colsum,
+                    int64_t rows, int C, int dtype, void* workspace, int64_t workspace_bytes, void* stream);
+
+int64_t pwa_dropout_colsum_det_workspace_size(int64_t rows, int C, int dtype);
+int pwa_dropout_colsum_det(const void* x, void* y, int64_t rows, int C, float p_drop, const void* seed_dev, float* colsum,
+                           int dtype, void* workspace, int64_t workspace_bytes, void* stream);
+
+int64_t pwa_colsum_rows_det_workspace_size(int64_t rows, int C, int dtype);
+int pwa_colsum_rows_det(const void* x, float* dst, int64_t rows, int C, int dtype, void* workspace, int64_t workspace_bytes,
+                        void* stream);
+
+int64_t pwa_bias_tables_bwd_det_workspace_size(int heads, int E, const int32_t ws[3], const int32_t cap[3], int I);
+int pwa_bias_tables_bwd_det(const float* enc_h, const float* enc_w, const float* enc_d, const float* wc_h,
+                            const float* wc_w, const float* wc_d, const float* enc_tok, const float* w_tok,
+                            const float* dth, const float* dtw, const float* dtd, const float* dtok,
+                            float* denc_h, float* denc_w, float* denc_d, float* dwc_h, float* dwc_w, float* dwc_d,
+                            float* denc_tok, float* dw_tok, int heads, int E, const int32_t ws[3],
+                            const int32_t cap[3], int I, void* workspace, int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

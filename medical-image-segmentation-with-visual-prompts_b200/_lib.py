@@ -99,15 +99,32 @@ def _load():
     lib.pwa_bias_tables_fwd.argtypes = [f32p] * 8 + [f32p] * 4 + [i32, i32, i32p, i32p, i32, vp]
     lib.pwa_bias_tables_bwd.argtypes = [f32p] * 8 + [f32p] * 4 + [f32p] * 8 + [i32, i32, i32p, i32p, i32, vp]
     lib.pwa_bias_tables_fwd.restype = lib.pwa_bias_tables_bwd.restype = i32
+    # deterministic siblings (include/pwa.h): the same arguments plus (workspace, workspace_bytes); size queries return int64
+    lib.pwa_attn_bwd_det.argtypes = [vp] * 5 + [f32p] * 4 + [u8p, vp, f32p, vp] + [vp] * 3 + [f32p] * 7 + [vp, i64, sp, i32, vp]
+    lib.pwa_ln_bwd2_det.argtypes = lib.pwa_ln_bwd2.argtypes[:-1] + [vp, i64, vp]
+    lib.pwa_dropout_colsum_det.argtypes = lib.pwa_dropout_colsum.argtypes[:-1] + [vp, i64, vp]
+    lib.pwa_colsum_rows_det.argtypes = lib.pwa_colsum_rows.argtypes[:-1] + [vp, i64, vp]
+    lib.pwa_bias_tables_bwd_det.argtypes = lib.pwa_bias_tables_bwd.argtypes[:-1] + [vp, i64, vp]
+    lib.pwa_attn_bwd_det_workspace_size.argtypes = [sp, i32]
+    lib.pwa_ln_bwd2_det_workspace_size.argtypes = [i64, i32, i32]
+    lib.pwa_dropout_colsum_det_workspace_size.argtypes = [i64, i32, i32]
+    lib.pwa_colsum_rows_det_workspace_size.argtypes = [i64, i32, i32]
+    lib.pwa_bias_tables_bwd_det_workspace_size.argtypes = [i32, i32, i32p, i32p, i32]
+    for name in DETERMINISTIC_SYMBOLS:
+        getattr(lib, name).restype = i64 if name.endswith("_workspace_size") else i32
     for name in ("pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_partition", "pwa_reverse",
                  "pwa_attn_tc_supported", "pwa_attn_fwd", "pwa_attn_bwd"):
         getattr(lib, name).restype = i32
     return lib
 
 
+DETERMINISTIC_SYMBOLS = ("pwa_attn_bwd_det", "pwa_attn_bwd_det_workspace_size", "pwa_ln_bwd2_det", "pwa_ln_bwd2_det_workspace_size",
+                         "pwa_dropout_colsum_det", "pwa_dropout_colsum_det_workspace_size", "pwa_colsum_rows_det",
+                         "pwa_colsum_rows_det_workspace_size", "pwa_bias_tables_bwd_det", "pwa_bias_tables_bwd_det_workspace_size")
+
 lib = _load()
 
-EXPORTED_SYMBOLS = ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
+EXPORTED_SYMBOLS = DETERMINISTIC_SYMBOLS + ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
                     "pwa_partition", "pwa_reverse", "pwa_reverse_add", "pwa_gather_rows", "pwa_colsum_f32", "pwa_colsum_rows", "pwa_dropout", "pwa_dropout_colsum", "pwa_token_gemm_supported", "pwa_token_gemm_fwd", "pwa_token_gemm_fwd_dt", "pwa_attn_fwd", "pwa_attn_bwd", "pwa_attn_tc_supported", "pwa_attn_dense_fwd", "pwa_attn_dense_bwd",
                     "pwa_ln_fwd", "pwa_ln_bwd", "pwa_ln_bwd2", "pwa_bias_tables_fwd", "pwa_bias_tables_bwd")
 

@@ -142,3 +142,81 @@ extern "C" int pwa_attn_bwd(const void* q, const void* k, const void* v, const v
   if (impl == 2 || (impl == 0 && tc_ok)) return attn_tc_backward(p, dtype, st);
   return attn_f32_backward(p, dtype, st);
 }
+
+// Workspace of pwa_attn_bwd_det in floats: prompt dK / dV slots [slots][B][I][C] each, then the table gradient slots
+// [slots][heads][wh][wh], [..][ww][ww], [..][wd][wd], [slots][heads][I].
+struct DetLayout {
+  size_t kp, vp, th, tw, td, tok, total;
+};
+
+static DetLayout det_layout(const AttnParams& p) {
+  const size_t S = (size_t)attn_tc_bwd_slots(p), h = (size_t)p.heads;
+  DetLayout d;
+  size_t o = 0;
+  d.kp = o; o += S * p.B * p.I * p.C;
+  d.vp = o; o += S * p.B * p.I * p.C;
+  d.th = o; o += S * h * p.wh * p.wh;
+  d.tw = o; o += S * h * p.ww * p.ww;
+  d.td = o; o += S * h * p.wd * p.wd;
+  d.tok = o; o += S * h * p.I;
+  d.total = o;
+  return d;
+}
+
+// the deterministic backward exists for the tcgen05 kernel only (whose table gradients take the per-warp slot path)
+static bool det_supported(const AttnParams& p, int dtype) {
+  return attn_tc_supported(p, dtype) && p.ww * p.wd == 32 && p.wd == 4;
+}
+
+extern "C" int64_t pwa_attn_bwd_det_workspace_size(const pwa_attn_shape* s, int dtype) {
+  AttnParams p = {};
+  int rc = fill(p, s, "pwa_attn_bwd_det_workspace_size");
+  if (rc != PWA_OK) return rc;
+  if (!det_supported(p, dtype)) {
+    set_error("pwa_attn_bwd_det_workspace_size: no deterministic backward for this shape/dtype (tcgen05 envelope only)");
+    return PWA_ERR_UNSUPPORTED;
+  }
+  return (int64_t)det_layout(p).total * 4;
+}
+
+extern "C" int pwa_attn_bwd_det(const void* q, const void* k, const void* v, const void* kp, const void* vp, const float* th,
+                                const float* tw, const float* td, const float* tok, const uint8_t* ids, const void* out,
+                                const float* lse, const void* dout, void* dq, void* dk, void* dv, float* dkp, float* dvp,
+                                float* dth, float* dtw, float* dtd, float* dtok, float* delta, void* workspace,
+                                int64_t workspace_bytes, const pwa_attn_shape* s, int dtype, void* stream) {
+  AttnParams p = {};
+  int rc = fill(p, s, "pwa_attn_bwd_det");
+  if (rc != PWA_OK) return rc;
+  if (!det_supported(p, dtype)) {
+    set_error("pwa_attn_bwd_det: no deterministic backward for this shape/dtype: it needs the tcgen05 kernel (bf16 or fp16, "
+              "see pwa_attn_tc_supported)");
+    return PWA_ERR_UNSUPPORTED;
+  }
+  PWA_CHECK_ARG(q && k && v && th && tw && td && out && lse && dout && dq && dk && dv && dth && dtw && dtd && delta,
+                "pwa_attn_bwd_det: null pointer");
+  PWA_CHECK_ARG(p.I == 0 || (kp && vp && tok && dkp && dvp && dtok), "pwa_attn_bwd_det: prompt tensors missing for I=%d", p.I);
+  const DetLayout L = det_layout(p);
+  PWA_CHECK_ARG(workspace != nullptr && workspace_bytes >= (int64_t)L.total * 4,
+                "pwa_attn_bwd_det: workspace of %lld bytes, %lld needed", (long long)workspace_bytes, (long long)L.total * 4);
+  float* ws = (float*)workspace;
+  p.q = q; p.k = k; p.v = v; p.kp = kp; p.vp = vp;
+  p.th = th; p.tw = tw; p.td = td; p.tok = tok; p.ids = ids;
+  p.out = const_cast<void*>(out); p.lse = const_cast<float*>(lse); p.dout = dout;
+  p.dq = dq; p.dk = dk; p.dv = dv; p.delta = delta;
+  p.dkp = ws + L.kp; p.dvp = ws + L.vp;
+  p.dth = ws + L.th; p.dtw = ws + L.tw; p.dtd = ws + L.td; p.dtok = ws + L.tok;
+  cudaStream_t st = (cudaStream_t)stream;
+  PWA_CUDA_OK(cudaMemsetAsync(ws, 0, L.total * 4, st));     // slots of samples a CTA never reaches stay zero
+  rc = attn_tc_backward_det(p, dtype, st);
+  if (rc != PWA_OK) return rc;
+  const int S = attn_tc_bwd_slots(p);
+  const int64_t h = p.heads, nkp = (int64_t)p.B * p.I * p.C;
+  const struct { const float* src; float* dst; int64_t n; } red[6] = {
+      {p.dth, dth, h * p.wh * p.wh}, {p.dtw, dtw, h * p.ww * p.ww}, {p.dtd, dtd, h * p.wd * p.wd},
+      {p.dtok, dtok, h * p.I}, {p.dkp, dkp, nkp}, {p.dvp, dvp, nkp}};
+  for (int i = 0; i < (p.I > 0 ? 6 : 3); ++i) {
+    rc = pwa_colsum_f32(red[i].src, red[i].dst, S, red[i].n, stream);
+    if (rc != PWA_OK) return rc;
+  }
+  return PWA_OK;
+}

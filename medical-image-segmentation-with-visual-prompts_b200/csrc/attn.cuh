@@ -134,5 +134,9 @@ bool attn_ws_fits(const AttnParams& p);                                   // att
 int attn_ws_forward(const AttnParams& p, int dtype, cudaStream_t st);
 bool attn_tc_bwd_fits(const AttnParams& p);                               // attn_tc_bwd.cu: TMEM and shared memory of the backward
 int attn_tc_backward(const AttnParams& p, int dtype, cudaStream_t st);
+// deterministic tcgen05 backward (attn_tc_bwd.cu, Det<E> instantiations): p.dkp / p.dvp / p.dth / p.dtw / p.dtd / p.dtok are
+// the workspace slot arrays of pwa_attn_bwd_det, attn_tc_bwd_slots(p) slots each
+int attn_tc_backward_det(const AttnParams& p, int dtype, cudaStream_t st);
+int attn_tc_bwd_slots(const AttnParams& p);
 
 }  // namespace pwa

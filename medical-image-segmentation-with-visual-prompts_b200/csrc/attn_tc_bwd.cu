@@ -195,10 +195,18 @@ enum {
 // E: element type of the token tensors and of the MMA operands (bf16 or fp16).  P^T uses the exact log-sum-exp (P <= 1), so
 // fp16's range matters only for g = P (dP - delta), delta and the stored gradients: under a large loss scale they overflow to
 // inf (NaN where inf meets inf), never to a finite value, and a non-finite dout stays non-finite -- GradScaler sees it.
-template <int DH, bool MASKED, bool DROP, typename E>
+// ET = E or Det<E>.  Det<E> is the deterministic instantiation: the CTAs of grid slot `slot = blockIdx.x / heads` (one per
+// head) own workspace slots and write them without atomics, p.dkp / p.dvp being [slots][B][I][C] and p.dth / p.dtw / p.dtd /
+// p.dtok [slots][heads][...] (see pwa_attn_bwd_det, which sums the slots in a fixed order).  A CTA's windows are
+// bw = slot + k * (gridDim / heads), so its sample b = bw / P never decreases and each (slot, sample) row of the prompt
+// gradients has one writer.  The table gradients take the `fast` per-(key block, warp) path, the only one the tcgen05
+// envelope reaches: no shared-memory atomics either.
+template <int DH, bool MASKED, bool DROP, typename ET>
 // (72 registers is the hard cap: 25 warps spread 7/6/6/6 over the four sub-partitions of 16 384 registers each, and
 //  7 warps x 32 x 80 does not fit -- a __maxnreg__(80) build fails to launch)
 __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p) {
+  using E = typename Elem<ET>::type;
+  constexpr bool DET = Elem<ET>::det;
   constexpr int DHP = BCfg<DH>::DHP, KS = BCfg<DH>::KS, DKC = BCfg<DH>::DKC, NBUF = BCfg<DH>::NBUF;
   constexpr bool FOLD = BCfg<DH>::FOLD && !DROP;
   // TMEM column map: NBUF x [S^T 64 | dP^T 64], then the accumulators
@@ -610,6 +618,16 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
     int acc_b = -1;                                                // sample the register accumulators belong to
     auto flush_prompt = [&]() {
       if (!kRegPrompt || acc_b < 0 || lane_row >= p.I) return;
+      if constexpr (DET) {                                         // this CTA's slot row of sample acc_b: written once
+        const size_t o = (((size_t)bw0 * p.B + acc_b) * p.I + lane_row) * p.C + head * DH;
+#pragma unroll
+        for (int d = 0; d < (kRegPrompt ? DH : 1); ++d) {
+          p.dkp[o + d] = accp_k[d];
+          p.dvp[o + d] = accp_v[d];
+          accp_k[d] = accp_v[d] = 0.f;
+        }
+        return;
+      }
       float* gk = p.dkp + ((size_t)acc_b * p.I + lane_row) * p.C + head * DH;
       float* gv = p.dvp + ((size_t)acc_b * p.I + lane_row) * p.C + head * DH;
 #pragma unroll
@@ -739,8 +757,14 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
           for (int d = 0; d < DH; ++d) accp_v[d] = fmaf(dv[d], keep_scale, accp_v[d]);
         } else {
           float* gp = p.dvp + ((size_t)b * p.I + lane_row) * p.C + head * DH;
+          if constexpr (DET) {                                     // read-modify-write of this CTA's own slot
+            gp += (size_t)bw0 * p.B * p.I * p.C;
+#pragma unroll
+            for (int d = 0; d < DH; ++d) gp[d] += dv[d] * keep_scale;
+          } else {
 #pragma unroll
           for (int d = 0; d < DH; ++d) atomicAdd(gp + d, dv[d] * keep_scale);
+          }
         }
       };
       auto put_dk = [&](const float (&dk)[DKC]) {
@@ -754,8 +778,14 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
           for (int d = 0; d < DH; ++d) accp_k[d] = fmaf(dk[d], p.scale, accp_k[d]);
         } else {
           float* gp = p.dkp + ((size_t)b * p.I + lane_row) * p.C + head * DH;
+          if constexpr (DET) {
+            gp += (size_t)bw0 * p.B * p.I * p.C;
+#pragma unroll
+            for (int d = 0; d < DH; ++d) gp[d] += dk[d] * p.scale;
+          } else {
 #pragma unroll
           for (int d = 0; d < DH; ++d) atomicAdd(gp + d, dk[d] * p.scale);
+          }
         }
       };
       float dv[DHP], dk[DKC];
@@ -852,7 +882,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
     // a warp's keys share jh = 4 kb + warp, every 4 consecutive lanes share jw, lanes l, l+4, ... share jd.  So after the
     // shuffle reduction the values go to per-(kb, warp) slots with plain stores (the g^T staging buffers are free by
     // now) and are summed when the CTA's result is added to global memory.  Other window shapes keep the atomics.
-    const bool fast = p.ww * p.wd == 32 && p.wd == 4;
+    const bool fast = DET || (p.ww * p.wd == 32 && p.wd == 4);   // (DET: checked by pwa_attn_bwd_det)
     float* slot_w = reinterpret_cast<float*>(smem + L.g);            // [8][ww * ww]
     float* slot_d = slot_w + 8 * p.ww * p.ww;                        // [8][wd * wd]
     const int wq = warp & 3;
@@ -911,6 +941,23 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
     STAMP(154);
     prod_sync();
     STAMP(155);
+    if constexpr (DET) {                                           // this CTA's table slots, summed in slot order
+      const size_t sh = (size_t)bw0 * p.heads + head;
+      for (int i = pt; i < p.wh * p.wh; i += kProd) p.dth[sh * p.wh * p.wh + i] = gth_s[i];
+      for (int i = pt; i < p.ww * p.ww; i += kProd) {
+        float v = 0.f;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) v += slot_w[k * p.ww * p.ww + i];
+        p.dtw[sh * p.ww * p.ww + i] = v;
+      }
+      for (int i = pt; i < p.wd * p.wd; i += kProd) {
+        float v = 0.f;
+#pragma unroll
+        for (int k = 0; k < 8; ++k) v += slot_d[k * 16 + i];
+        p.dtd[sh * p.wd * p.wd + i] = v;
+      }
+      for (int i = pt; i < p.I; i += kProd) p.dtok[sh * p.I + i] = gtok_s[i];
+    } else {
     for (int i = pt; i < p.wh * p.wh; i += kProd) atomicAdd(&p.dth[head * p.wh * p.wh + i], gth_s[i]);
     for (int i = pt; i < p.ww * p.ww; i += kProd) {
       float v = gtw_s[i];
@@ -931,6 +978,7 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
       atomicAdd(&p.dtd[head * p.wd * p.wd + i], v);
     }
     for (int i = pt; i < p.I; i += kProd) atomicAdd(&p.dtok[head * p.I + i], gtok_s[i]);
+    }
   }
   STAMP(151);                                                      // role done
   tc_fence_before();
@@ -940,17 +988,23 @@ __global__ void __launch_bounds__(kThreadsB, 1) attn_bwd_tc_kernel(AttnParams p)
   if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
+// one persistent CTA per SM, a multiple of `heads` (a CTA keeps one head)
+int bwd_grid(const AttnParams& p) {
+  int grid = 148;
+  grid -= grid % p.heads;
+  if (grid < p.heads) grid = p.heads;
+  const int need = p.B * p.P * p.heads;
+  if (grid > need) grid = need;
+  return grid;
+}
+
 template <int DH, typename E>
 int launch_bwd_tc(const AttnParams& p, cudaStream_t st) {
   constexpr int DHP = BCfg<DH>::DHP, KS = BCfg<DH>::KS;
   const int NKT = kN + p.I;
   const BwdSmem L = bwd_layout(KS, DHP, NKT, p.wh, p.ww, p.wd, p.I, p.ids != nullptr);
   const size_t smem = L.total;
-  int grid = 148;
-  grid -= grid % p.heads;
-  if (grid < p.heads) grid = p.heads;
-  const int need = p.B * p.P * p.heads;
-  if (grid > need) grid = need;
+  const int grid = bwd_grid(p);
   auto kern = p.drop_thresh ? (p.ids ? attn_bwd_tc_kernel<DH, true, true, E> : attn_bwd_tc_kernel<DH, false, true, E>)
                             : (p.ids ? attn_bwd_tc_kernel<DH, true, false, E> : attn_bwd_tc_kernel<DH, false, false, E>);
   PWA_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -983,6 +1037,12 @@ static int backward_t(const AttnParams& p, cudaStream_t st) {
 
 int attn_tc_backward(const AttnParams& p, int dtype, cudaStream_t st) {
   return dtype == PWA_F16 ? backward_t<__half>(p, st) : backward_t<__nv_bfloat16>(p, st);
+}
+
+int attn_tc_bwd_slots(const AttnParams& p) { return bwd_grid(p) / p.heads; }
+
+int attn_tc_backward_det(const AttnParams& p, int dtype, cudaStream_t st) {
+  return dtype == PWA_F16 ? backward_t<Det<__half>>(p, st) : backward_t<Det<__nv_bfloat16>>(p, st);
 }
 
 }  // namespace pwa

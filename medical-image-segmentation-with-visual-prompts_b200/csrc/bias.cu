@@ -58,21 +58,37 @@ __global__ void __launch_bounds__(256) bias_tables_fwd_kernel(BiasArgs a) {
   }
 }
 
-// grid = (4, kBwdSplit): every block rebuilds the tiny dper table, then owns a slice of the output elements
+// grid = (4, kBwdSplit): every block rebuilds the tiny dper table, then owns a slice of the output elements.
+// DET: dper[h][r] is summed by one thread over the (i, j) of its distance in index order, without shared atomics (the
+// only cross-thread reduction of this kernel; nothing crosses CTAs).
 constexpr int kBwdSplit = 16;
-__global__ void __launch_bounds__(256) bias_tables_bwd_kernel(BiasArgs a) {
+// (tid: the wrapper's threadIdx.x, which carries the range its launch bounds give it)
+template <bool DET>
+__device__ __forceinline__ void bias_tables_bwd_body(const BiasArgs& a, const int tid) {
   extern __shared__ float sm[];                                  // dper [heads][R] (content) / unused (token)
-  const int ax = blockIdx.x, tid = threadIdx.x;
+  const int ax = blockIdx.x;
   const int gt = blockIdx.y * 256 + tid, gn = kBwdSplit * 256;   // thread id / count across the blockIdx.y slices
   const float scale = rsqrtf((float)a.E);
   if (ax < 3) {
     const int w = a.ws[ax], cap = a.cap[ax], R = 2 * cap - 1;
     const float f = scale / 3.f;
-    for (int o = tid; o < a.heads * R; o += 256) sm[o] = 0.f;
-    __syncthreads();
-    for (int o = tid; o < a.heads * w * w; o += 256) {
-      const int hd = o / (w * w), ij = o - hd * w * w, i = ij / w, j = ij - i * w;
-      atomicAdd(&sm[hd * R + rel_index(i, j, cap)], a.tab[ax][o]);
+    if constexpr (DET) {
+      for (int o = tid; o < a.heads * R; o += 256) {
+        const int hd = o / R, r = o - hd * R;
+        float s = 0.f;
+        for (int ij = 0; ij < w * w; ++ij) {
+          const int i = ij / w, j = ij - i * w;
+          if (rel_index(i, j, cap) == r) s += a.tab[ax][hd * w * w + ij];
+        }
+        sm[o] = s;
+      }
+    } else {
+      for (int o = tid; o < a.heads * R; o += 256) sm[o] = 0.f;
+      __syncthreads();
+      for (int o = tid; o < a.heads * w * w; o += 256) {
+        const int hd = o / (w * w), ij = o - hd * w * w, i = ij / w, j = ij - i * w;
+        atomicAdd(&sm[hd * R + rel_index(i, j, cap)], a.tab[ax][o]);
+      }
     }
     __syncthreads();
     for (int o = gt; o < R * a.E; o += gn) {                     // d enc[r][c] = f * sum_h dper[h][r] * W[h][c]
@@ -103,6 +119,9 @@ __global__ void __launch_bounds__(256) bias_tables_bwd_kernel(BiasArgs a) {
     }
   }
 }
+
+__global__ void __launch_bounds__(256) bias_tables_bwd_kernel(BiasArgs a) { bias_tables_bwd_body<false>(a, threadIdx.x); }
+__global__ void __launch_bounds__(256) bias_tables_bwd_det_kernel(BiasArgs a) { bias_tables_bwd_body<true>(a, threadIdx.x); }
 
 static int check_common(const BiasArgs& a, const char* who) {
   PWA_CHECK_ARG(a.heads > 0 && a.E > 0 && a.I >= 0, "%s: bad heads/E/I", who);
@@ -138,12 +157,11 @@ extern "C" int pwa_bias_tables_fwd(const float* enc_h, const float* enc_w, const
   return PWA_OK;
 }
 
-extern "C" int pwa_bias_tables_bwd(const float* enc_h, const float* enc_w, const float* enc_d, const float* wc_h,
-                                   const float* wc_w, const float* wc_d, const float* enc_tok, const float* w_tok,
-                                   const float* dth, const float* dtw, const float* dtd, const float* dtok,
-                                   float* denc_h, float* denc_w, float* denc_d, float* dwc_h, float* dwc_w, float* dwc_d,
-                                   float* denc_tok, float* dw_tok, int heads, int E, const int32_t ws[3],
-                                   const int32_t cap[3], int I, void* stream) {
+static int bias_tables_bwd(const float* enc_h, const float* enc_w, const float* enc_d, const float* wc_h, const float* wc_w,
+                           const float* wc_d, const float* enc_tok, const float* w_tok, const float* dth, const float* dtw,
+                           const float* dtd, const float* dtok, float* denc_h, float* denc_w, float* denc_d, float* dwc_h,
+                           float* dwc_w, float* dwc_d, float* denc_tok, float* dw_tok, int heads, int E, const int32_t ws[3],
+                           const int32_t cap[3], int I, void* stream, bool det) {
   BiasArgs a = {};
   a.enc[0] = enc_h; a.enc[1] = enc_w; a.enc[2] = enc_d;
   a.wc[0] = wc_h; a.wc[1] = wc_w; a.wc[2] = wc_d;
@@ -161,7 +179,35 @@ extern "C" int pwa_bias_tables_bwd(const float* enc_h, const float* enc_w, const
   if (rc != PWA_OK) return rc;
   for (int x = 0; x < 3; ++x) PWA_CHECK_ARG(a.denc[x] && a.dwc[x], "pwa_bias_tables_bwd: null gradient pointer");
   PWA_CHECK_ARG(I == 0 || (denc_tok && dw_tok), "pwa_bias_tables_bwd: null token gradient pointer");
-  bias_tables_bwd_kernel<<<dim3(4, kBwdSplit), 256, (size_t)heads * maxR * 4, (cudaStream_t)stream>>>(a);
+  (det ? bias_tables_bwd_det_kernel : bias_tables_bwd_kernel)<<<dim3(4, kBwdSplit), 256, (size_t)heads * maxR * 4, (cudaStream_t)stream>>>(a);
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
+}
+
+extern "C" int pwa_bias_tables_bwd(const float* enc_h, const float* enc_w, const float* enc_d, const float* wc_h,
+                                   const float* wc_w, const float* wc_d, const float* enc_tok, const float* w_tok,
+                                   const float* dth, const float* dtw, const float* dtd, const float* dtok,
+                                   float* denc_h, float* denc_w, float* denc_d, float* dwc_h, float* dwc_w, float* dwc_d,
+                                   float* denc_tok, float* dw_tok, int heads, int E, const int32_t ws[3],
+                                   const int32_t cap[3], int I, void* stream) {
+  return bias_tables_bwd(enc_h, enc_w, enc_d, wc_h, wc_w, wc_d, enc_tok, w_tok, dth, dtw, dtd, dtok, denc_h, denc_w, denc_d,
+                         dwc_h, dwc_w, dwc_d, denc_tok, dw_tok, heads, E, ws, cap, I, stream, false);
+}
+
+// Every CTA of this backward computes its outputs alone (no cross-CTA sums): the deterministic form needs no workspace.
+extern "C" int64_t pwa_bias_tables_bwd_det_workspace_size(int heads, int E, const int32_t ws[3], const int32_t cap[3], int I) {
+  if (heads <= 0 || E <= 0 || I < 0 || ws == nullptr || cap == nullptr) return PWA_ERR_ARG;
+  return 0;
+}
+
+extern "C" int pwa_bias_tables_bwd_det(const float* enc_h, const float* enc_w, const float* enc_d, const float* wc_h,
+                                       const float* wc_w, const float* wc_d, const float* enc_tok, const float* w_tok,
+                                       const float* dth, const float* dtw, const float* dtd, const float* dtok,
+                                       float* denc_h, float* denc_w, float* denc_d, float* dwc_h, float* dwc_w, float* dwc_d,
+                                       float* denc_tok, float* dw_tok, int heads, int E, const int32_t ws[3],
+                                       const int32_t cap[3], int I, void* workspace, int64_t workspace_bytes, void* stream) {
+  (void)workspace;
+  PWA_CHECK_ARG(workspace_bytes >= 0, "pwa_bias_tables_bwd_det: workspace_bytes=%lld", (long long)workspace_bytes);
+  return bias_tables_bwd(enc_h, enc_w, enc_d, wc_h, wc_w, wc_d, enc_tok, w_tok, dth, dtw, dtd, dtok, denc_h, denc_w, denc_d,
+                         dwc_h, dwc_w, dwc_d, denc_tok, dw_tok, heads, E, ws, cap, I, stream, true);
 }

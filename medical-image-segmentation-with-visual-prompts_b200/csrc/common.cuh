@@ -49,6 +49,14 @@ template <> __device__ __forceinline__ float from_f32<float>(float v) { return v
 template <> __device__ __forceinline__ __nv_bfloat16 from_f32<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 template <> __device__ __forceinline__ __half from_f32<__half>(float v) { return __float2half_rn(v); }
 
+// Det<T> in place of a kernel's element type T selects the deterministic instantiation of a kernel whose cross-CTA sums are
+// float atomics: it writes fixed-order partial sums to one workspace slot per CTA instead, and the host sums the slots in a
+// fixed order (pwa_colsum_f32).  The default instantiations keep their names and their code; the variant is another
+// instantiation of the same template, never a runtime branch.  Elem<X>::type is the element type, Elem<X>::det the switch.
+template <typename T> struct Det { T v; };
+template <typename X> struct Elem { using type = X; static constexpr bool det = false; };
+template <typename T> struct Elem<Det<T>> { using type = T; static constexpr bool det = true; };
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -171,13 +171,20 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 16 ? 4 : (NV * EPV <=
 // the gradient of `proj(...) + bias`, dres that of `mlp(...) + bias`), which saves two full reduction passes.
 // PLAIN: no residual-path gradient and no column sums (the PatchMerging norm, down.py:44: rows of 384-1536 channels, where
 // the three extra per-column register arrays of the general kernel meant spills and one CTA per SM)
-template <typename T, int G, int NV, int EPV, bool PLAIN = false>
-__global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 8 ? 4 : (NV * EPV <= 16 ? 2 : 1))) ln_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ x,
+// X = Det<T>: dgamma, dbeta, dres_colsum and dx_colsum are slot arrays [gridDim][C]; the warps add their column sums to shared
+// memory one warp after the other and the CTA stores its sums to its own slots (summed in a fixed order by pwa_ln_bwd2_det).
+template <typename X, int G, int NV, int EPV, bool PLAIN = false>
+__global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 8 ? 4 : (NV * EPV <= 16 ? 2 : 1))) ln_bwd_kernel(const X* __restrict__ dyin, const X* __restrict__ xin,
                                                             const float* __restrict__ gamma, const float* __restrict__ mean_in,
-                                                            const float* __restrict__ rstd_in, const T* __restrict__ dres,
-                                                            T* __restrict__ dx, float* __restrict__ dgamma,
+                                                            const float* __restrict__ rstd_in, const X* __restrict__ dresin,
+                                                            X* __restrict__ dxout, float* __restrict__ dgamma,
                                                             float* __restrict__ dbeta, float* __restrict__ dres_colsum,
                                                             float* __restrict__ dx_colsum, long rows, int C) {
+  using T = typename Elem<X>::type;
+  const T* __restrict__ dy = reinterpret_cast<const T*>(dyin);
+  const T* __restrict__ x = reinterpret_cast<const T*>(xin);
+  const T* __restrict__ dres = reinterpret_cast<const T*>(dresin);
+  T* __restrict__ dx = reinterpret_cast<T*>(dxout);
   constexpr int GPB = kLnThreads / G;
   extern __shared__ float red[];                        // [4][C]
   const int gl = threadIdx.x % G, gr = threadIdx.x / G;
@@ -257,6 +264,50 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 8 ? 4 : (NV * EPV <= 
     }
   }
   __syncthreads();
+  if constexpr (Elem<X>::det) {
+    // the same shuffles, then the warps add to shared memory in warp order, then plain stores to this CTA's slots
+#pragma unroll
+    for (int k = 0; k < NV; ++k) {
+#pragma unroll
+      for (int e = 0; e < EPV; ++e) {
+#pragma unroll
+        for (int o = G; o < 32; o <<= 1) {
+          ag[k][e] += __shfl_xor_sync(0xffffffffu, ag[k][e], o);
+          ab[k][e] += __shfl_xor_sync(0xffffffffu, ab[k][e], o);
+          if constexpr (!PLAIN) {
+            if (want_rs) ar[k][e] += __shfl_xor_sync(0xffffffffu, ar[k][e], o);
+            if (want_xs) ax[k][e] += __shfl_xor_sync(0xffffffffu, ax[k][e], o);
+          }
+        }
+      }
+    }
+    for (int w = 0; w < kLnThreads / 32; ++w) {
+      if ((int)(threadIdx.x >> 5) == w && (threadIdx.x & 31) < G) {
+#pragma unroll
+        for (int k = 0; k < NV; ++k) {
+          const int vi = gl + k * G;
+          if (vi >= nvec) continue;
+#pragma unroll
+          for (int e = 0; e < EPV; ++e) {
+            red[vi * EPV + e] += ag[k][e];
+            red[C + vi * EPV + e] += ab[k][e];
+            if constexpr (!PLAIN) {
+              if (want_rs) red[2 * C + vi * EPV + e] += ar[k][e];
+              if (want_xs) red[3 * C + vi * EPV + e] += ax[k][e];
+            }
+          }
+        }
+      }
+      __syncthreads();
+    }
+    const size_t slot = (size_t)blockIdx.x * C;
+    for (int i = threadIdx.x; i < C; i += kLnThreads) {
+      dgamma[slot + i] = red[i];
+      dbeta[slot + i] = red[C + i];
+      if (want_rs) dres_colsum[slot + i] = red[2 * C + i];
+      if (want_xs) dx_colsum[slot + i] = red[3 * C + i];
+    }
+  } else {
   // column sums: first across the 32/G row groups of a warp (lanes with equal gl) by shuffles, then one
   // shared-memory atomic per warp and column (8-way instead of 256/G-way contention), then one global atomic per CTA
 #pragma unroll
@@ -287,6 +338,7 @@ __global__ void __launch_bounds__(kLnThreads, (NV * EPV <= 8 ? 4 : (NV * EPV <= 
     atomicAdd(&dbeta[i], red[C + i]);
     if (want_rs) atomicAdd(&dres_colsum[i], red[2 * C + i]);
     if (want_xs) atomicAdd(&dx_colsum[i], red[3 * C + i]);
+  }
   }
 }
 
@@ -460,13 +512,20 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 4 : 3) ln_fwd_bulk_kernel
   }
 }
 
-template <int G, int R, typename T>
-__global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel(const T* __restrict__ dy, const T* __restrict__ x,
+// X = Det<T>: dgamma, dbeta, dres_colsum and dx_colsum are slot arrays [gridDim][C] that the CTA stores its sums to (the in-CTA
+// order is fixed either way); pwa_ln_bwd2_det sums the slots in a fixed order.
+template <int G, int R, typename X>
+__global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel(const X* __restrict__ dyin, const X* __restrict__ xin,
                                                                     const float* __restrict__ gamma, const float* __restrict__ mean_in,
-                                                                    const float* __restrict__ rstd_in, const T* __restrict__ dres,
-                                                                    T* __restrict__ dx, float* __restrict__ dgamma,
+                                                                    const float* __restrict__ rstd_in, const X* __restrict__ dresin,
+                                                                    X* __restrict__ dxout, float* __restrict__ dgamma,
                                                                     float* __restrict__ dbeta, float* __restrict__ dres_colsum,
                                                                     float* __restrict__ dx_colsum, long rows, int C) {
+  using T = typename Elem<X>::type;
+  const T* __restrict__ dy = reinterpret_cast<const T*>(dyin);
+  const T* __restrict__ x = reinterpret_cast<const T*>(xin);
+  const T* __restrict__ dres = reinterpret_cast<const T*>(dresin);
+  T* __restrict__ dx = reinterpret_cast<T*>(dxout);
   constexpr int GPB = kLnThreads / G, TR = GPB * R, EPV = 8;
   extern __shared__ __align__(128) uint8_t ln_sm[];
   __shared__ __align__(8) uint64_t full[kMaxStages];
@@ -596,10 +655,18 @@ __global__ void __launch_bounds__(kLnThreads, R == 1 ? 3 : 2) ln_bwd_bulk_kernel
       if (want_rs) c += part[(w * 4 + 2) * C + i];
       if (want_xs) d += part[(w * 4 + 3) * C + i];
     }
-    atomicAdd(&dgamma[i], a);
-    atomicAdd(&dbeta[i], b);
-    if (want_rs) atomicAdd(&dres_colsum[i], c);
-    if (want_xs) atomicAdd(&dx_colsum[i], d);
+    if constexpr (Elem<X>::det) {
+      const size_t slot = (size_t)blockIdx.x * C;
+      dgamma[slot + i] = a;
+      dbeta[slot + i] = b;
+      if (want_rs) dres_colsum[slot + i] = c;
+      if (want_xs) dx_colsum[slot + i] = d;
+    } else {
+      atomicAdd(&dgamma[i], a);
+      atomicAdd(&dbeta[i], b);
+      if (want_rs) atomicAdd(&dres_colsum[i], c);
+      if (want_xs) atomicAdd(&dx_colsum[i], d);
+    }
   }
 }
 
@@ -611,12 +678,13 @@ struct LnArgs {
   long rows;
   int C;
   float eps;
+  float* det_ws;       // backward: non-NULL = the deterministic kernels, slot arrays [4][blocks][C] here (see ln_det_slots)
 };
 
-template <typename T, int G, int NV, int EPV>
-static int ln_launch(bool fwd, const LnArgs& a, cudaStream_t st) {
-  constexpr int GPB = kLnThreads / G;
-  long blocks = (a.rows + GPB - 1) / GPB;
+// grid of the register kernels
+static long ln_reg_blocks(bool fwd, long rows, int G) {
+  const int GPB = kLnThreads / G;
+  long blocks = (rows + GPB - 1) / GPB;
   // backward: fewer CTAs -> fewer global atomics; with few rows (the late PatchMerging norms: 7 K rows of 768 channels) every
   // CTA should also run several iterations, or its epilogue (4C shared words zeroed, 2C..4C shared + global atomics)
   // outweighs its share of the rows: 48 -> see tools/bench_ln.py
@@ -627,6 +695,64 @@ static int ln_launch(bool fwd, const LnArgs& a, cudaStream_t st) {
   }
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
+  return blocks;
+}
+
+// Rows per lane group and iteration of the bulk kernels, measured (tools/bench_ln.py): R = 2 is 8-13 % faster in backward,
+// within +-5 % in forward.  At most 4 CTAs per SM forward, 2 backward (the bytes in flight no longer depend on the occupancy).
+constexpr int kBulkRF = 1, kBulkRB = 2;
+static long ln_bulk_blocks(bool fwd, long rows, int G) {
+  const int TR = kLnThreads / G * (fwd ? kBulkRF : kBulkRB);
+  long blocks = (rows + TR - 1) / TR;
+  const long cap = 148L * (fwd ? 4 : 2);
+  if (blocks > cap) blocks = cap;
+  if (blocks < 1) blocks = 1;
+  return blocks;
+}
+
+// Deterministic backward: the kernel writes its column sums to the slot arrays [4][blocks][C] of a.det_ws (dgamma, dbeta,
+// dres_colsum, dx_colsum), which ln_det_reduce then sums over the CTAs in a fixed order into the caller's outputs.
+static LnArgs ln_det_slots(const LnArgs& a, long blocks) {
+  LnArgs d = a;
+  const size_t n = (size_t)blocks * a.C;
+  d.f1 = a.det_ws;
+  d.f2 = a.det_ws + n;
+  d.f3 = a.f3 ? a.det_ws + 2 * n : nullptr;
+  d.f4 = a.f4 ? a.det_ws + 3 * n : nullptr;
+  return d;
+}
+
+static int ln_det_reduce(const LnArgs& a, long blocks, cudaStream_t st) {
+  const size_t n = (size_t)blocks * a.C;
+  float* out[4] = {a.f1, a.f2, a.f3, a.f4};
+  for (int i = 0; i < 4; ++i) {
+    if (out[i] == nullptr) continue;
+    const int rc = pwa_colsum_f32(a.det_ws + i * n, out[i], (int)blocks, a.C, st);
+    if (rc != PWA_OK) return rc;
+  }
+  return PWA_OK;
+}
+
+template <typename T, int G, int NV, int EPV>
+static int ln_launch(bool fwd, const LnArgs& a0, cudaStream_t st) {
+  const long blocks = ln_reg_blocks(fwd, a0.rows, G);
+  const bool det = !fwd && a0.det_ws != nullptr;
+  const LnArgs a = det ? ln_det_slots(a0, blocks) : a0;
+  if (det) {
+    using D = Det<T>;
+    if constexpr (NV >= 2) {
+      if (a.res == nullptr && a.f3 == nullptr && a.f4 == nullptr) {
+        ln_bwd_kernel<D, G, NV, EPV, true><<<(unsigned)blocks, kLnThreads, 4 * a.C * sizeof(float), st>>>(
+            (const D*)a.a, (const D*)a.b, a.gamma, a.bm, a.rstd, nullptr, (D*)a.o1, a.f1, a.f2, nullptr, nullptr, a.rows, a.C);
+        PWA_CUDA_OK(cudaGetLastError());
+        return ln_det_reduce(a0, blocks, st);
+      }
+    }
+    ln_bwd_kernel<D, G, NV, EPV><<<(unsigned)blocks, kLnThreads, 4 * a.C * sizeof(float), st>>>(
+        (const D*)a.a, (const D*)a.b, a.gamma, a.bm, a.rstd, (const D*)a.res, (D*)a.o1, a.f1, a.f2, a.f3, a.f4, a.rows, a.C);
+    PWA_CUDA_OK(cudaGetLastError());
+    return ln_det_reduce(a0, blocks, st);
+  }
   if (fwd) {
     ln_fwd_kernel<T, G, NV, EPV><<<(unsigned)blocks, kLnThreads, 0, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm,
                                                                            (T*)a.o1, (T*)a.o2, a.f1, a.f2, a.rows, a.C, a.eps);
@@ -646,19 +772,24 @@ static int ln_launch(bool fwd, const LnArgs& a, cudaStream_t st) {
   return PWA_OK;
 }
 
-// Rows per lane group and iteration of the bulk kernels, measured (tools/bench_ln.py): R = 2 is 8-13 % faster in backward,
-// within +-5 % in forward.  At most 4 CTAs per SM forward, 2 backward (the bytes in flight no longer depend on the occupancy).
 template <int G, typename T>
-static int ln_launch_bulk(bool fwd, const LnArgs& a, cudaStream_t st) {
-  constexpr int RF = 1, RB = 2;
+static int ln_launch_bulk(bool fwd, const LnArgs& a0, cudaStream_t st) {
+  constexpr int RF = kBulkRF, RB = kBulkRB;
   const int R = fwd ? RF : RB, TR = kLnThreads / G * R;
-  const int nop = fwd ? (a.res ? 2 : 1) : (a.res ? 3 : 2);
+  const int nop = fwd ? (a0.res ? 2 : 1) : (a0.res ? 3 : 2);
   // (backward epilogue: the per-warp column sums, 8 x 4 x C floats, reuse the ring memory: >= 192 * C bytes for every G)
-  const size_t smem = (size_t)(kMaxStages / nop / R) * nop * TR * a.C * 2;
-  long blocks = (a.rows + TR - 1) / TR;
-  const long cap = 148L * (fwd ? 4 : 2);
-  if (blocks > cap) blocks = cap;
-  if (blocks < 1) blocks = 1;
+  const size_t smem = (size_t)(kMaxStages / nop / R) * nop * TR * a0.C * 2;
+  const long blocks = ln_bulk_blocks(fwd, a0.rows, G);
+  if (!fwd && a0.det_ws != nullptr) {
+    using D = Det<T>;
+    const LnArgs a = ln_det_slots(a0, blocks);
+    PWA_CUDA_OK(cudaFuncSetAttribute(ln_bwd_bulk_kernel<G, RB, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ln_bwd_bulk_kernel<G, RB, D><<<(unsigned)blocks, kLnThreads, smem, st>>>((const D*)a.a, (const D*)a.b, a.gamma, a.bm, a.rstd,
+                                                                          (const D*)a.res, (D*)a.o1, a.f1, a.f2, a.f3, a.f4, a.rows, a.C);
+    PWA_CUDA_OK(cudaGetLastError());
+    return ln_det_reduce(a0, blocks, st);
+  }
+  const LnArgs& a = a0;
   if (fwd) {
     PWA_CUDA_OK(cudaFuncSetAttribute(ln_fwd_bulk_kernel<G, RF, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ln_fwd_bulk_kernel<G, RF, T><<<(unsigned)blocks, kLnThreads, smem, st>>>((const T*)a.a, (const T*)a.res, a.gamma, a.bm,
@@ -671,6 +802,9 @@ static int ln_launch_bulk(bool fwd, const LnArgs& a, cudaStream_t st) {
   PWA_CUDA_OK(cudaGetLastError());
   return PWA_OK;
 }
+
+// lane group width of the row kernels for rows of nvec vectors (ln_dispatch_v)
+static int ln_group(int nvec) { return nvec <= 4 ? 4 : (nvec <= 8 ? 8 : (nvec <= 16 ? 16 : 32)); }
 
 template <typename T, int EPV>
 static int ln_dispatch_v(bool fwd, const LnArgs& a, cudaStream_t st) {
@@ -720,7 +854,7 @@ extern "C" int pwa_ln_fwd(const void* x, const void* res, const float* gamma, co
   PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_ln_fwd: bad dtype %d", dtype);
   if (rows == 0) return PWA_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  LnArgs a = {x, nullptr, res, gamma, beta, nullptr, sum_out, y, mean, rstd, nullptr, nullptr, (long)rows, C, eps};
+  LnArgs a = {x, nullptr, res, gamma, beta, nullptr, sum_out, y, mean, rstd, nullptr, nullptr, (long)rows, C, eps, nullptr};
   if (dtype == PWA_F16) return ln_dispatch<__half>(true, a, st);
   return dtype == PWA_F32 ? ln_dispatch<float>(true, a, st) : ln_dispatch<__nv_bfloat16>(true, a, st);
 }
@@ -738,7 +872,45 @@ extern "C" int pwa_ln_bwd2(const void* dy, const void* x, const float* gamma, co
   if (dres_colsum) PWA_CUDA_OK(cudaMemsetAsync(dres_colsum, 0, (size_t)C * 4, st));
   if (dx_colsum) PWA_CUDA_OK(cudaMemsetAsync(dx_colsum, 0, (size_t)C * 4, st));
   if (rows == 0) return PWA_OK;
-  LnArgs a = {dy, x, dres, gamma, mean, rstd, dx, nullptr, dgamma, dbeta, dres_colsum, dx_colsum, (long)rows, C, 0.f};
+  LnArgs a = {dy, x, dres, gamma, mean, rstd, dx, nullptr, dgamma, dbeta, dres_colsum, dx_colsum, (long)rows, C, 0.f, nullptr};
+  if (dtype == PWA_F16) return ln_dispatch<__half>(false, a, st);
+  return dtype == PWA_F32 ? ln_dispatch<float>(false, a, st) : ln_dispatch<__nv_bfloat16>(false, a, st);
+}
+
+// Slots of the deterministic backward: the grid of whichever kernel ln_dispatch picks.  16-bit rows with C % 8 == 0 take the
+// EPV = 8 kernels when the pointers are 16-byte aligned and the EPV = 4 ones otherwise: the size covers both.
+extern "C" int64_t pwa_ln_bwd2_det_workspace_size(int64_t rows, int C, int dtype) {
+  if (rows < 0 || C <= 0 || C % 4 != 0 || C > 2048) return PWA_ERR_ARG;
+  if (dtype != PWA_F32 && dtype != PWA_BF16 && dtype != PWA_F16) return PWA_ERR_ARG;
+  if (rows == 0) return 0;
+  long blocks = ln_reg_blocks(false, (long)rows, ln_group(C / 4));
+  if (dtype != PWA_F32 && C % 8 == 0) {
+    const int nvec = C / 8;
+    const long b8 = nvec <= 32 ? ln_bulk_blocks(false, (long)rows, ln_group(nvec)) : ln_reg_blocks(false, (long)rows, 32);
+    if (b8 > blocks) blocks = b8;
+  }
+  return (int64_t)blocks * 4 * C * 4;
+}
+
+extern "C" int pwa_ln_bwd2_det(const void* dy, const void* x, const float* gamma, const float* mean, const float* rstd,
+                               const void* dres, void* dx, float* dgamma, float* dbeta, float* dres_colsum, float* dx_colsum,
+                               int64_t rows, int C, int dtype, void* workspace, int64_t workspace_bytes, void* stream) {
+  PWA_CHECK_ARG(dy && x && gamma && mean && rstd && dx && dgamma && dbeta, "pwa_ln_bwd2_det: null pointer");
+  PWA_CHECK_ARG(rows >= 0 && C > 0 && C % 4 == 0 && C <= 2048, "pwa_ln_bwd2_det: need C %% 4 == 0, C <= 2048 (C=%d)", C);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_ln_bwd2_det: bad dtype %d", dtype);
+  PWA_CHECK_ARG(dres_colsum == nullptr || dres != nullptr, "pwa_ln_bwd2_det: dres_colsum without dres");
+  const int64_t need = pwa_ln_bwd2_det_workspace_size(rows, C, dtype);
+  PWA_CHECK_ARG(workspace_bytes >= need && (need == 0 || workspace != nullptr),
+                "pwa_ln_bwd2_det: workspace of %lld bytes, %lld needed", (long long)workspace_bytes, (long long)need);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (rows == 0) {
+    PWA_CUDA_OK(cudaMemsetAsync(dgamma, 0, (size_t)C * 4, st));
+    PWA_CUDA_OK(cudaMemsetAsync(dbeta, 0, (size_t)C * 4, st));
+    if (dres_colsum) PWA_CUDA_OK(cudaMemsetAsync(dres_colsum, 0, (size_t)C * 4, st));
+    if (dx_colsum) PWA_CUDA_OK(cudaMemsetAsync(dx_colsum, 0, (size_t)C * 4, st));
+    return PWA_OK;
+  }
+  LnArgs a = {dy, x, dres, gamma, mean, rstd, dx, nullptr, dgamma, dbeta, dres_colsum, dx_colsum, (long)rows, C, 0.f, (float*)workspace};
   if (dtype == PWA_F16) return ln_dispatch<__half>(false, a, st);
   return dtype == PWA_F32 ? ln_dispatch<float>(false, a, st) : ln_dispatch<__nv_bfloat16>(false, a, st);
 }

@@ -38,8 +38,12 @@ __global__ void __launch_bounds__(32 * kRowGroups) colsum_f32_kernel(const float
 // generic reduction needed 36-62 us per call for it (0.5-2.3 TB/s).  blockDim is a multiple of the 16-byte vectors per
 // row, so a thread meets the same columns in every iteration: four independent vector loads in flight per thread,
 // register accumulators, a shared-memory transposition and one global atomic per (CTA, column) at the end.
-template <typename T>
-__global__ void __launch_bounds__(512) colsum_rows_kernel(const T* __restrict__ x, float* __restrict__ dst, long nvec, int C) {
+// X = Det<T>: the CTA's column sums go with plain stores to its own slot dst[blockIdx.x][C] instead, summed over the slots in
+// a fixed order by pwa_colsum_rows_det (the in-CTA order is fixed either way).
+template <typename X>
+__global__ void __launch_bounds__(512) colsum_rows_kernel(const X* __restrict__ xin, float* __restrict__ dst, long nvec, int C) {
+  using T = typename Elem<X>::type;
+  const T* __restrict__ x = reinterpret_cast<const T*>(xin);
   constexpr int E = 16 / (int)sizeof(T);
   extern __shared__ float part_s[];                       // [blockDim][E] partial sums
   float acc[E];
@@ -69,7 +73,8 @@ __global__ void __launch_bounds__(512) colsum_rows_kernel(const T* __restrict__ 
     const int cg = c / E, e = c - cg * E;
     float t = 0.f;
     for (int r = 0; r < reps; ++r) t += part_s[(r * vpr + cg) * E + e];
-    atomicAdd(&dst[c], t);
+    if constexpr (Elem<X>::det) dst[(size_t)blockIdx.x * C + c] = t;
+    else atomicAdd(&dst[c], t);
   }
 }
 
@@ -88,26 +93,83 @@ extern "C" int pwa_colsum_f32(const float* src, float* dst, int S, int64_t n, vo
   return PWA_OK;
 }
 
-extern "C" int pwa_colsum_rows(const void* x, float* dst, int64_t rows, int C, int dtype, void* stream) {
-  PWA_CHECK_ARG(x != nullptr && dst != nullptr, "pwa_colsum_rows: null pointer");
-  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "pwa_colsum_rows: bad dtype %d", dtype);
+struct ColsumRowsGrid {
+  int threads;
+  long nvec, blocks;
+};
+
+static ColsumRowsGrid colsum_rows_grid(int64_t rows, int C, int dtype) {
   const int E = dtype == PWA_F32 ? 4 : 8;
-  PWA_CHECK_ARG(rows >= 0 && C >= E && C % E == 0 && C / E <= 512, "pwa_colsum_rows: rows=%lld C=%d (need C %% %d == 0, C <= %d)",
+  const int vpr = C / E;
+  ColsumRowsGrid g;
+  g.threads = 512 / vpr * vpr;                          // a multiple of the vectors per row: fixed columns per thread
+  g.nvec = (long)rows * vpr;
+  g.blocks = (g.nvec + (long)g.threads * 4 - 1) / ((long)g.threads * 4);
+  if (g.blocks > 148 * 2) g.blocks = 148 * 2;
+  if (g.blocks < 1) g.blocks = 1;
+  return g;
+}
+
+static int colsum_rows_check(const void* x, const float* dst, int64_t rows, int C, int dtype, const char* who) {
+  PWA_CHECK_ARG(x != nullptr && dst != nullptr, "%s: null pointer", who);
+  PWA_CHECK_ARG(dtype == PWA_F32 || dtype == PWA_BF16 || dtype == PWA_F16, "%s: bad dtype %d", who, dtype);
+  const int E = dtype == PWA_F32 ? 4 : 8;
+  PWA_CHECK_ARG(rows >= 0 && C >= E && C % E == 0 && C / E <= 512, "%s: rows=%lld C=%d (need C %% %d == 0, C <= %d)", who,
                 (long long)rows, C, E, 512 * E);
-  PWA_CHECK_ARG(((uintptr_t)x & 15) == 0, "pwa_colsum_rows: x must be 16-byte aligned");
+  PWA_CHECK_ARG(((uintptr_t)x & 15) == 0, "%s: x must be 16-byte aligned", who);
+  return PWA_OK;
+}
+
+template <bool DET>
+static int colsum_rows_launch(const void* x, float* dst, int64_t rows, int C, int dtype, cudaStream_t st) {
+  const ColsumRowsGrid g = colsum_rows_grid(rows, C, dtype);
+  const size_t smem = (size_t)g.threads * 16;
+  const unsigned nb = (unsigned)g.blocks;
+  using B = __nv_bfloat16;
+  using H = __half;
+  if (dtype == PWA_BF16) {
+    if (DET) colsum_rows_kernel<Det<B>><<<nb, g.threads, smem * 2, st>>>((const Det<B>*)x, dst, g.nvec, C);
+    else colsum_rows_kernel<B><<<nb, g.threads, smem * 2, st>>>((const B*)x, dst, g.nvec, C);
+  } else if (dtype == PWA_F16) {
+    if (DET) colsum_rows_kernel<Det<H>><<<nb, g.threads, smem * 2, st>>>((const Det<H>*)x, dst, g.nvec, C);
+    else colsum_rows_kernel<H><<<nb, g.threads, smem * 2, st>>>((const H*)x, dst, g.nvec, C);
+  } else {
+    if (DET) colsum_rows_kernel<Det<float>><<<nb, g.threads, smem, st>>>((const Det<float>*)x, dst, g.nvec, C);
+    else colsum_rows_kernel<float><<<nb, g.threads, smem, st>>>((const float*)x, dst, g.nvec, C);
+  }
+  PWA_CUDA_OK(cudaGetLastError());
+  return PWA_OK;
+}
+
+extern "C" int pwa_colsum_rows(const void* x, float* dst, int64_t rows, int C, int dtype, void* stream) {
+  int rc = colsum_rows_check(x, dst, rows, C, dtype, "pwa_colsum_rows");
+  if (rc != PWA_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   PWA_CUDA_OK(cudaMemsetAsync(dst, 0, (size_t)C * 4, st));
   if (rows == 0) return PWA_OK;
-  const int vpr = C / E;
-  const int threads = 512 / vpr * vpr;                  // a multiple of the vectors per row: fixed columns per thread
-  const long nvec = (long)rows * vpr;
-  long blocks = (nvec + (long)threads * 4 - 1) / ((long)threads * 4);
-  if (blocks > 148 * 2) blocks = 148 * 2;
-  if (blocks < 1) blocks = 1;
-  const size_t smem = (size_t)threads * 16;
-  if (dtype == PWA_BF16) colsum_rows_kernel<__nv_bfloat16><<<(unsigned)blocks, threads, smem * 2, st>>>((const __nv_bfloat16*)x, dst, nvec, C);
-  else if (dtype == PWA_F16) colsum_rows_kernel<__half><<<(unsigned)blocks, threads, smem * 2, st>>>((const __half*)x, dst, nvec, C);
-  else colsum_rows_kernel<float><<<(unsigned)blocks, threads, smem, st>>>((const float*)x, dst, nvec, C);
-  PWA_CUDA_OK(cudaGetLastError());
-  return PWA_OK;
+  return colsum_rows_launch<false>(x, dst, rows, C, dtype, st);
+}
+
+extern "C" int64_t pwa_colsum_rows_det_workspace_size(int64_t rows, int C, int dtype) {
+  const int E = dtype == PWA_F32 ? 4 : 8;
+  if (rows < 0 || C < E || C % E != 0 || C / E > 512) return PWA_ERR_ARG;
+  return rows == 0 ? 0 : colsum_rows_grid(rows, C, dtype).blocks * C * 4;
+}
+
+extern "C" int pwa_colsum_rows_det(const void* x, float* dst, int64_t rows, int C, int dtype, void* workspace,
+                                   int64_t workspace_bytes, void* stream) {
+  int rc = colsum_rows_check(x, dst, rows, C, dtype, "pwa_colsum_rows_det");
+  if (rc != PWA_OK) return rc;
+  const int64_t need = pwa_colsum_rows_det_workspace_size(rows, C, dtype);
+  PWA_CHECK_ARG(workspace_bytes >= need && (need == 0 || workspace != nullptr),
+                "pwa_colsum_rows_det: workspace of %lld bytes, %lld needed", (long long)workspace_bytes, (long long)need);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (rows == 0) {
+    PWA_CUDA_OK(cudaMemsetAsync(dst, 0, (size_t)C * 4, st));
+    return PWA_OK;
+  }
+  float* slots = (float*)workspace;
+  rc = colsum_rows_launch<true>(x, slots, rows, C, dtype, st);
+  if (rc != PWA_OK) return rc;
+  return pwa_colsum_f32(slots, dst, (int)colsum_rows_grid(rows, C, dtype).blocks, C, stream);
 }

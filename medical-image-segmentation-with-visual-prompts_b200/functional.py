@@ -6,6 +6,7 @@ import ctypes as C
 from typing import Optional, Sequence
 
 import functools
+import warnings
 
 import torch
 
@@ -76,6 +77,30 @@ def _stream(t: torch.Tensor):
 
 def _ptr(t: Optional[torch.Tensor]):
     return C.c_void_p(0 if t is None else t.data_ptr())
+
+
+# ------------------------------------------------------------------------------------------------
+# deterministic mode: torch.use_deterministic_algorithms(True) switches every backward with cross-CTA float sums to the
+# `_det` sibling of its entry point (include/pwa.h).  The flag is read when the backward runs, as torch does for its own ops.
+# ------------------------------------------------------------------------------------------------
+def _det_workspace(nbytes: int, what: str, device) -> torch.Tensor:
+    """Device scratch of a deterministic sibling, `nbytes` as its size query returned (negative = error code).  It comes from
+    the caching allocator, so it is valid under CUDA-graph capture."""
+    _lib.check(min(int(nbytes), 0), what)
+    return torch.empty(max(int(nbytes), 1), dtype=torch.uint8, device=device)
+
+
+def _no_deterministic_form(op: str, how: str):
+    """What torch does for an op without a deterministic implementation: raise under use_deterministic_algorithms(True), warn
+    under warn_only=True (and then run)."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = (f"{op} does not have a deterministic implementation, but you set 'torch.use_deterministic_algorithms(True)'. "
+           f"{how}")
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg, stacklevel=3)
+    else:
+        raise RuntimeError(msg)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -290,6 +315,25 @@ def _check_attn_side_inputs(B, P, N, Cc, dtype, kp, vp, kp_width, th, tw, td, to
         raise ValueError(f"region ids must be uint8 [{P},{N}], got {ids.dtype} {tuple(ids.shape)}")
 
 
+_ATTN_DET_HOW = ("The deterministic attention backward is the tcgen05 kernel's: bf16 or fp16 tensors (or torch.autocast), impl "
+                 "AUTO or TC, and a shape inside pwa_attn_tc_supported (256-token windows with wd <= 4 and wh + ww <= 16, head "
+                 "dim 3, 6, 12, 24 or 48, 0 to 128 prompt tokens in steps of 32).")
+
+
+def _attn_bwd(ptrs, s, dtype, impl, device, stream):
+    """pwa_attn_bwd, or pwa_attn_bwd_det under torch.use_deterministic_algorithms(True) (tcgen05 shapes only; the fp32-math
+    backward has no deterministic form)."""
+    code = _DT[dtype]
+    if torch.are_deterministic_algorithms_enabled():
+        if dtype in _LOWP and impl != IMPL_F32 and _lib.lib.pwa_attn_tc_supported(C.byref(s), code):
+            ws = _det_workspace(_lib.lib.pwa_attn_bwd_det_workspace_size(C.byref(s), code), "pwa_attn_bwd_det", device)
+            rc = _lib.lib.pwa_attn_bwd_det(*ptrs, _ptr(ws), ws.numel(), C.byref(s), code, stream)
+            _lib.check(rc, "pwa_attn_bwd_det")
+            return
+        _no_deterministic_form("prompted window attention backward (fp32-math kernel)", _ATTN_DET_HOW)
+    _lib.check(_lib.lib.pwa_attn_bwd(*ptrs, C.byref(s), code, impl, stream), "pwa_attn_bwd")
+
+
 class _WindowAttention(torch.autograd.Function):
     @staticmethod
     def forward(ctx, q, k, v, kp, vp, th, tw, td, tok, ids, heads, ws, scale, impl, p_drop=0.0, seed=None):
@@ -329,11 +373,9 @@ class _WindowAttention(torch.autograd.Function):
         s = _shape_struct(B, P, Cc, heads, I, ws, scale, p_drop=p_drop, seed_dev=seed,
                           sel=sel_table_for(ids) if q.dtype in _LOWP and impl != IMPL_F32 else None)
         with torch.cuda.device(q.device), _timed("attn_bwd", 2, 8.0 * B * P * N * (N + I) * Cc, q):
-            rc = _lib.lib.pwa_attn_bwd(_ptr(q), _ptr(k), _ptr(v), _ptr(kp), _ptr(vp), _ptr(th), _ptr(tw), _ptr(td),
-                                       _ptr(tok), _ptr(ids), _ptr(out), _ptr(lse), _ptr(dout), _ptr(dq), _ptr(dk),
-                                       _ptr(dv), _ptr(dkp), _ptr(dvp), _ptr(dth), _ptr(dtw), _ptr(dtd), _ptr(dtok),
-                                       _ptr(delta), C.byref(s), _dtype_code(q), impl, _stream(q))
-        _lib.check(rc, "pwa_attn_bwd")
+            _attn_bwd([_ptr(q), _ptr(k), _ptr(v), _ptr(kp), _ptr(vp), _ptr(th), _ptr(tw), _ptr(td), _ptr(tok), _ptr(ids),
+                       _ptr(out), _ptr(lse), _ptr(dout), _ptr(dq), _ptr(dk), _ptr(dv), _ptr(dkp), _ptr(dvp), _ptr(dth),
+                       _ptr(dtw), _ptr(dtd), _ptr(dtok), _ptr(delta)], s, q.dtype, impl, q.device, _stream(q))
         if I:
             dkp, dvp = dkp.to(q.dtype), dvp.to(q.dtype)
         return dq, dk, dv, dkp, dvp, dth, dtw, dtd, dtok, None, None, None, None, None, None, None
@@ -395,6 +437,8 @@ class _DenseWindowAttention(torch.autograd.Function):
         dout = dout.contiguous()
         dq, dk, dv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
         want_db = bias5 is not None and ctx.needs_input_grad[3]
+        _no_deterministic_form("dense_window_attention backward (float atomics across queries and windows)",
+                               "Use prompted_window_attention (compact bias tables) in bf16 or fp16 for a deterministic backward.")
         dbias = torch.zeros_like(bias5) if want_db else None
         delta = torch.empty_like(lse)
         with torch.cuda.device(q.device):
@@ -444,6 +488,17 @@ def prompted_window_attention(q, k, v, kp, vp, th, tw, td, tok, ids, heads: int,
 # ------------------------------------------------------------------------------------------------
 # LayerNorm over channels (+ fused residual add)
 # ------------------------------------------------------------------------------------------------
+def _ln_bwd2(dy, x, g32, mean, rstd, dres, dx, dg, db, dbr, dbx, rows, Cc):
+    """pwa_ln_bwd2, or pwa_ln_bwd2_det under torch.use_deterministic_algorithms(True)."""
+    args = [_ptr(dy), _ptr(x), _ptr(g32), _ptr(mean), _ptr(rstd), _ptr(dres), _ptr(dx), _ptr(dg), _ptr(db), _ptr(dbr), _ptr(dbx),
+            rows, Cc, _dtype_code(x)]
+    if torch.are_deterministic_algorithms_enabled():
+        ws = _det_workspace(_lib.lib.pwa_ln_bwd2_det_workspace_size(rows, Cc, _dtype_code(x)), "pwa_ln_bwd2_det", x.device)
+        _lib.check(_lib.lib.pwa_ln_bwd2_det(*args, _ptr(ws), ws.numel(), _stream(x)), "pwa_ln_bwd2_det")
+    else:
+        _lib.check(_lib.lib.pwa_ln_bwd2(*args, _stream(x)), "pwa_ln_bwd")
+
+
 class _AddLayerNorm(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, res, gamma, beta, eps, bias_of_x=None, bias_of_res=None):
@@ -492,9 +547,7 @@ class _AddLayerNorm(torch.autograd.Function):
         dbr = torch.empty(Cc, dtype=torch.float32, device=normed.device) if br_dt is not None and ds is not None else None
         nbytes = (3 if ds is None else 4) * normed.numel() * normed.element_size()
         with torch.cuda.device(normed.device), _timed("ln_bwd", 1, float(nbytes), normed):
-            rc = _lib.lib.pwa_ln_bwd2(_ptr(dy), _ptr(normed), _ptr(g32), _ptr(mean), _ptr(rstd), _ptr(ds), _ptr(dx), _ptr(dg),
-                                      _ptr(db), _ptr(dbr), _ptr(dbx), rows, Cc, _dtype_code(normed), _stream(normed))
-        _lib.check(rc, "pwa_ln_bwd")
+            _ln_bwd2(dy, normed, g32, mean, rstd, ds, dx, dg, db, dbr, dbx, rows, Cc)
         gd, bd = ctx.param_dtypes
         return (dx, (dx if ctx.has_res else None), dg.to(gd), db.to(bd), None,
                 None if dbx is None else dbx.to(bx_dt), None if dbr is None else dbr.to(br_dt))
@@ -536,9 +589,7 @@ class _LayerNormPass(torch.autograd.Function):
         db = torch.empty(Cc, dtype=torch.float32, device=x.device)
         nbytes = (3 if dalias is None else 4) * x.numel() * x.element_size()
         with torch.cuda.device(x.device), _timed("ln_bwd", 1, float(nbytes), x):
-            rc = _lib.lib.pwa_ln_bwd2(_ptr(dy), _ptr(x), _ptr(g32), _ptr(mean), _ptr(rstd), _ptr(dalias), _ptr(dx), _ptr(dg), _ptr(db),
-                                      None, None, rows, Cc, _dtype_code(x), _stream(x))
-        _lib.check(rc, "pwa_ln_bwd")
+            _ln_bwd2(dy, x, g32, mean, rstd, dalias, dx, dg, db, None, None, rows, Cc)
         gd, bd = ctx.param_dtypes
         return dx, dg.to(gd), db.to(bd), None
 
@@ -616,11 +667,15 @@ class _BiasTables(torch.autograd.Function):
         dtk = [torch.empty_like(t) for t in tk] if has_tok else [None, None]
         a3 = C.c_int32 * 3
         cap = a3(*[(t.shape[0] + 1) // 2 for t in ten[:3]])
+        args = [*[_ptr(t) for t in ten], _ptr(tk[0]), _ptr(tk[1]), _ptr(grads[0]), _ptr(grads[1]), _ptr(grads[2]), _ptr(dtok),
+                *[_ptr(t) for t in outs], _ptr(dtk[0]), _ptr(dtk[1]), heads, E, a3(*ws), cap, I]
         with torch.cuda.device(ten[0].device), _timed("bias_tables_bwd", 1, 0.0, ten[0]):
-            rc = _lib.lib.pwa_bias_tables_bwd(*[_ptr(t) for t in ten], _ptr(tk[0]), _ptr(tk[1]), _ptr(grads[0]),
-                                              _ptr(grads[1]), _ptr(grads[2]), _ptr(dtok), *[_ptr(t) for t in outs],
-                                              _ptr(dtk[0]), _ptr(dtk[1]), heads, E, a3(*ws), cap, I, _stream(ten[0]))
-        _lib.check(rc, "pwa_bias_tables_bwd")
+            if torch.are_deterministic_algorithms_enabled():
+                wsb = _det_workspace(_lib.lib.pwa_bias_tables_bwd_det_workspace_size(heads, E, a3(*ws), cap, I),
+                                     "pwa_bias_tables_bwd_det", ten[0].device)
+                _lib.check(_lib.lib.pwa_bias_tables_bwd_det(*args, _ptr(wsb), wsb.numel(), _stream(ten[0])), "pwa_bias_tables_bwd_det")
+            else:
+                _lib.check(_lib.lib.pwa_bias_tables_bwd(*args, _stream(ten[0])), "pwa_bias_tables_bwd")
         outs = [o.to(d) for o, d in zip(outs, dts)]
         return (*outs, dtk[0], dtk[1], None)
 
@@ -683,13 +738,11 @@ class _WindowAttentionPacked(torch.autograd.Function):
         p0 = 0 if kvp is None else kvp.data_ptr()
         vpp = C.c_void_p
         with torch.cuda.device(qkv.device), _timed("attn_bwd", 2, 8.0 * B * P * N * (N + I) * Cc, qkv):
-            rc = _lib.lib.pwa_attn_bwd(vpp(q0), vpp(q0 + Cc * es), vpp(q0 + 2 * Cc * es), vpp(p0), vpp(p0 + Cc * es if p0 else 0),
-                                       _ptr(th), _ptr(tw), _ptr(td), _ptr(tok), _ptr(ids), _ptr(out), _ptr(lse), _ptr(dout),
-                                       vpp(d0), vpp(d0 + Cc * es), vpp(d0 + 2 * Cc * es),
-                                       _ptr(dkvp32[0] if I else None), _ptr(dkvp32[1] if I else None),
-                                       _ptr(dth), _ptr(dtw), _ptr(dtd), _ptr(dtok), _ptr(delta), C.byref(s),
-                                       _dtype_code(qkv), impl, _stream(qkv))
-        _lib.check(rc, "pwa_attn_bwd")
+            _attn_bwd([vpp(q0), vpp(q0 + Cc * es), vpp(q0 + 2 * Cc * es), vpp(p0), vpp(p0 + Cc * es if p0 else 0),
+                       _ptr(th), _ptr(tw), _ptr(td), _ptr(tok), _ptr(ids), _ptr(out), _ptr(lse), _ptr(dout),
+                       vpp(d0), vpp(d0 + Cc * es), vpp(d0 + 2 * Cc * es),
+                       _ptr(dkvp32[0] if I else None), _ptr(dkvp32[1] if I else None),
+                       _ptr(dth), _ptr(dtw), _ptr(dtd), _ptr(dtok), _ptr(delta)], s, qkv.dtype, impl, qkv.device, _stream(qkv))
         dkvp = None
         if I:
             dkvp = torch.cat([dkvp32[0], dkvp32[1]], dim=-1).to(qkv.dtype)          # [B,I,2C]
@@ -700,6 +753,18 @@ def new_dropout_seed(device, words: int = 2) -> torch.Tensor:
     """32-bit seed words ON THE DEVICE (two per dropout site: forward and backward share them).  Drawn with a CUDA RNG op,
     so torch.manual_seed governs it and a captured CUDA graph gets fresh words on every replay."""
     return torch.randint(0, 2 ** 31 - 1, (words,), dtype=torch.int32, device=device)
+
+
+def _dropout_colsum(x, y, Cc, p_drop, seed, colsum):
+    """pwa_dropout_colsum, or pwa_dropout_colsum_det under torch.use_deterministic_algorithms(True)."""
+    rows = x.numel() // Cc
+    args = [_ptr(x), _ptr(y), rows, Cc, float(p_drop), _ptr(seed), _ptr(colsum), _dtype_code(x)]
+    if torch.are_deterministic_algorithms_enabled():
+        ws = _det_workspace(_lib.lib.pwa_dropout_colsum_det_workspace_size(rows, Cc, _dtype_code(x)), "pwa_dropout_colsum_det",
+                            x.device)
+        _lib.check(_lib.lib.pwa_dropout_colsum_det(*args, _ptr(ws), ws.numel(), _stream(x)), "pwa_dropout_colsum_det")
+    else:
+        _lib.check(_lib.lib.pwa_dropout_colsum(*args, _stream(x)), "pwa_dropout")
 
 
 class _SeededDropout(torch.autograd.Function):
@@ -727,11 +792,10 @@ class _SeededDropout(torch.autograd.Function):
         with torch.cuda.device(dy.device), _timed("dropout", 1, 2.0 * dy.numel() * dy.element_size(), dy):
             if ctx.bias_dtype is not None:
                 db = torch.empty(Cc, dtype=torch.float32, device=dy.device)
-                rc = _lib.lib.pwa_dropout_colsum(_ptr(dy), _ptr(dx), dy.numel() // Cc, Cc, ctx.p_drop, _ptr(seed), _ptr(db),
-                                                 _dtype_code(dy), _stream(dy))
+                _dropout_colsum(dy, dx, Cc, ctx.p_drop, seed, db)
             else:
-                rc = _lib.lib.pwa_dropout(_ptr(dy), _ptr(dx), dy.numel(), ctx.p_drop, _ptr(seed), _dtype_code(dy), _stream(dy))
-        _lib.check(rc, "pwa_dropout")
+                _lib.check(_lib.lib.pwa_dropout(_ptr(dy), _ptr(dx), dy.numel(), ctx.p_drop, _ptr(seed), _dtype_code(dy), _stream(dy)),
+                           "pwa_dropout")
         return dx, None, None, (None if db is None else db.to(ctx.bias_dtype))
 
 
@@ -816,7 +880,11 @@ def colsum_rows(x2):
         return torch.zeros(Cc, dtype=torch.float32, device=x2.device)
     out = torch.empty(Cc, dtype=torch.float32, device=x2.device)
     with torch.cuda.device(x2.device), _timed("colsum_rows", 1, float(x2.numel() * x2.element_size()), x2):
-        rc = _lib.lib.pwa_colsum_rows(_ptr(x2), _ptr(out), T, Cc, _dtype_code(x2), _stream(x2))
+        if torch.are_deterministic_algorithms_enabled():
+            ws = _det_workspace(_lib.lib.pwa_colsum_rows_det_workspace_size(T, Cc, _dtype_code(x2)), "pwa_colsum_rows_det", x2.device)
+            rc = _lib.lib.pwa_colsum_rows_det(_ptr(x2), _ptr(out), T, Cc, _dtype_code(x2), _ptr(ws), ws.numel(), _stream(x2))
+        else:
+            rc = _lib.lib.pwa_colsum_rows(_ptr(x2), _ptr(out), T, Cc, _dtype_code(x2), _stream(x2))
     _lib.check(rc, "pwa_colsum_rows")
     return out
 
@@ -928,9 +996,7 @@ def _ln_backward_raw(dy, x, g32, mean, rstd, dres, want_res_colsum, want_x_colsu
     dbx = torch.empty(Cc, **f32) if want_x_colsum else None
     nbytes = (3 if dres is None else 4) * x.numel() * x.element_size()
     with torch.cuda.device(x.device), _timed("ln_bwd", 1, float(nbytes), x):
-        rc = _lib.lib.pwa_ln_bwd2(_ptr(dy), _ptr(x), _ptr(g32), _ptr(mean), _ptr(rstd), _ptr(dres), _ptr(dx), _ptr(dg), _ptr(db),
-                                  _ptr(dbr), _ptr(dbx), rows, Cc, _dtype_code(x), _stream(x))
-    _lib.check(rc, "pwa_ln_bwd")
+        _ln_bwd2(dy, x, g32, mean, rstd, dres, dx, dg, db, dbr, dbx, rows, Cc)
     return dx, dg, db, dbr, dbx
 
 
@@ -1012,11 +1078,10 @@ class _DropAddLnLinear(torch.autograd.Function):
             with torch.cuda.device(dx.device), _timed("dropout", 1, 2.0 * dx.numel() * dx.element_size(), dx):
                 if want_ba and dropout_colsum_supported(Cc):
                     dba = torch.empty(Cc, dtype=torch.float32, device=dx.device)
-                    rc = _lib.lib.pwa_dropout_colsum(_ptr(dx), _ptr(da), dx.numel() // Cc, Cc, p_drop, _ptr(seed), _ptr(dba),
-                                                     _dtype_code(dx), _stream(dx))
+                    _dropout_colsum(dx, da, Cc, p_drop, seed, dba)
                 else:
-                    rc = _lib.lib.pwa_dropout(_ptr(dx), _ptr(da), dx.numel(), p_drop, _ptr(seed), _dtype_code(dx), _stream(dx))
-            _lib.check(rc, "pwa_dropout")
+                    _lib.check(_lib.lib.pwa_dropout(_ptr(dx), _ptr(da), dx.numel(), p_drop, _ptr(seed), _dtype_code(dx), _stream(dx)),
+                               "pwa_dropout")
             if want_ba and dba is None:
                 dba = colsum_rows(da)
         else:

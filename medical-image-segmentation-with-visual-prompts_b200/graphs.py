@@ -26,6 +26,8 @@ class GraphedStep:
         """step_fn(*inputs) must run forward AND backward and return a (scalar) loss tensor; it is called `warmup`
         times eagerly on a side stream (lazy initialisation: cuBLAS handles, kernel attributes, cached index maps),
         then once more under capture.  Inputs that require grad get a static .grad too (`input_grads`).
+        The graph replays the kernels the capture recorded: under torch.use_deterministic_algorithms(True) at capture time
+        every replay runs the deterministic backward kernels (see INTEGRATION.md), whatever the flag says at replay time.
         flat_grads=True makes every parameter's .grad a view into ONE flat fp32 buffer (`flat_grad`), so that the
         data-parallel exchange is a single in-place all-reduce of that buffer (`allreduce_flat`).  Inside the graph the
         backward produces its gradients as usual (autograd hands the freshly computed tensors over without a kernel) and
