@@ -329,6 +329,55 @@ int pwa_bias_tables_bwd_det(const float* enc_h, const float* enc_w, const float*
                             float* denc_tok, float* dw_tok, int heads, int E, const int32_t ws[3],
                             const int32_t cap[3], int I, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- whole-volume sliding-window inference ----------------------------------------------------------------------------- */
+
+/* The reference scores the downstream model on whole volumes by cutting them into roi-sized patches, running the model on
+ * sub-batches of patches and adding the predictions back with overlap weights (SegmentationTrainer.test, SURVEY.md §3(4)).
+ * These entry points are the GPU side of that loop (pwa_b200.inference builds the tiling on the host):
+ *   - origins: int32 [n_total][4] table (b, x0, y0, z0) on the DEVICE, 16-byte aligned, in patch order (sample, then raster
+ *     order over x, y, z).  Origins are >= 0; a patch may reach past the volume (an axis shorter than the roi).
+ *   - cursor: int32 {first, count} on the DEVICE.  A call works on patches [first, first + count) of the table (count is
+ *     clamped to [0, sw] and to the table).  pwa_tile_advance moves the cursor to the next sub-batch, so a captured CUDA
+ *     graph of gather -> predictor -> stitch -> advance walks the whole table by replaying, with no host scalar in it.
+ *   - dims = (X, Y, Z) of the volume, roi = (r0, r1, r2), 1 <= sw <= PWA_TILE_MAX_SW patches per sub-batch.
+ *   - arguments are checked before any CUDA call (PWA_ERR_ARG without a GPU); nothing allocates or synchronises. */
+#define PWA_TILE_MAX_SW 1024
+/* Element types of label maps and target volumes. */
+enum { PWA_LABEL_U8 = 0, PWA_LABEL_I32 = 1, PWA_LABEL_I64 = 2 };
+
+/* patches [sw][Cin][r0][r1][r2] (dtype_out) <- image [B][Cin][X][Y][Z] (dtype_in): slot s < count holds the patch at
+ * origins[first + s], voxels outside the volume read `cval` (rounded to dtype_in first, as F.pad does); slots >= count are all
+ * `cval`.  Bit-exact against slicing + F.pad + .to(dtype_out).  16-byte vectors along z where roi[2] % 8 == 0 and the row is
+ * aligned, elements otherwise. */
+int pwa_tile_gather(const void* image, int dtype_in, int B, int Cin, const int32_t dims[3], const int32_t* origins,
+                    int64_t n_total, const int32_t* cursor, const int32_t roi[3], int sw, float cval, void* patches,
+                    int dtype_out, void* stream);
+
+/* acc fp32 [B][K][X][Y][Z] += weight * pred and wsum fp32 [B][X][Y][Z] += weight for the `count` patches of this call, with
+ * pred [sw][K][r0][r1][r2] (fp32, bf16 or fp16) and the importance map weight fp32 [r0][r1][r2].  No float atomics: each
+ * covered voxel is read once, gets the terms of the covering patches added one after the other in patch order (fused
+ * multiply-add, fp32) and is written once, so the sums are bitwise independent of sw and reproducible from run to run. */
+int pwa_tile_stitch(const void* pred, int dtype_pred, const float* weight, int B, int K, const int32_t dims[3],
+                    const int32_t* origins, int64_t n_total, const int32_t* cursor, const int32_t roi[3], int sw,
+                    float* acc, float* wsum, void* stream);
+
+/* cursor {first, count} <- {first + count, min(sw, n_total - first - count)}: one single-thread kernel. */
+int pwa_tile_advance(int32_t* cursor, int sw, int64_t n_total, void* stream);
+
+/* One pass over acc [B][K][X][Y][Z] and wsum [B][X][Y][Z]; each output is optional (NULL = skip):
+ *   - out [B][K][X][Y][Z] = acc / wsum in dtype_out (fp32 division, rounded once);
+ *   - labels [B][X][Y][Z] = argmax over K of the fp32 acc / wsum, the lowest class on ties (torch.argmax), uint8 for K <= 256
+ *     and int32 otherwise;
+ *   - tp, fp, fn int64 [B][K] (zeroed by the call, exact integer atomics) against target [B][X][Y][Z] of type target_dtype
+ *     (PWA_LABEL_*); voxels whose target is outside [0, K) are not counted.  Counting needs K <= 1024. */
+int pwa_tile_finalize(const float* acc, const float* wsum, int B, int K, const int32_t dims[3], void* out, int dtype_out,
+                      void* labels, const void* target, int target_dtype, int64_t* tp, int64_t* fp, int64_t* fn, void* stream);
+
+/* tp, fp, fn int64 [B][K] (zeroed by the call) of a label map against a target, both [B][nvox] of types PWA_LABEL_*; voxels
+ * whose label or target is outside [0, K) are not counted.  K <= 1024. */
+int pwa_seg_counts(const void* labels, int label_dtype, const void* target, int target_dtype, int B, int64_t nvox, int K,
+                   int64_t* tp, int64_t* fp, int64_t* fn, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

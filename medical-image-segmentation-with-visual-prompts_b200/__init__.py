@@ -10,9 +10,12 @@ from . import functional
 from . import graphs
 from . import trainer
 from .graphs import GraphedStep
+from . import inference
+from .inference import sliding_window_inference, segmentation_counts, dice_iou
 from .modules import (ConsecutiveSwinBlocks, SwinTransformerBlock, PatchMerging, WindowAttention, RelativePE,
                       BiasTables, window_partition, window_reverse, get_attn_mask, SwinUnetR, SwinUnetRConfig, SwinUpBlock)
 
 __all__ = ['ConsecutiveSwinBlocks', 'SwinTransformerBlock', 'PatchMerging', 'WindowAttention', 'RelativePE',
            'BiasTables', 'window_partition', 'window_reverse', 'get_attn_mask', 'Geometry', 'get_geometry',
-           'functional', 'graphs', 'trainer', 'GraphedStep', 'SwinUnetR', 'SwinUnetRConfig', 'SwinUpBlock']
+           'functional', 'graphs', 'trainer', 'GraphedStep', 'inference', 'sliding_window_inference',
+           'segmentation_counts', 'dice_iou', 'SwinUnetR', 'SwinUnetRConfig', 'SwinUpBlock']

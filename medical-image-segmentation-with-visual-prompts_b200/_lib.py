@@ -112,6 +112,15 @@ def _load():
     lib.pwa_bias_tables_bwd_det_workspace_size.argtypes = [i32, i32, i32p, i32p, i32]
     for name in DETERMINISTIC_SYMBOLS:
         getattr(lib, name).restype = i64 if name.endswith("_workspace_size") else i32
+    # whole-volume sliding-window inference (pwa_b200.inference)
+    a3 = C.POINTER(i32)
+    lib.pwa_tile_gather.argtypes = [vp, i32, i32, i32, a3, vp, i64, vp, a3, i32, f32, vp, i32, vp]
+    lib.pwa_tile_stitch.argtypes = [vp, i32, f32p, i32, i32, a3, vp, i64, vp, a3, i32, f32p, f32p, vp]
+    lib.pwa_tile_advance.argtypes = [vp, i32, i64, vp]
+    lib.pwa_tile_finalize.argtypes = [f32p, f32p, i32, i32, a3, vp, i32, vp, vp, i32, vp, vp, vp, vp]
+    lib.pwa_seg_counts.argtypes = [vp, i32, vp, i32, i32, i64, i32, vp, vp, vp, vp]
+    for name in TILE_SYMBOLS:
+        getattr(lib, name).restype = i32
     for name in ("pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_partition", "pwa_reverse",
                  "pwa_attn_tc_supported", "pwa_attn_fwd", "pwa_attn_bwd"):
         getattr(lib, name).restype = i32
@@ -122,9 +131,13 @@ DETERMINISTIC_SYMBOLS = ("pwa_attn_bwd_det", "pwa_attn_bwd_det_workspace_size", 
                          "pwa_dropout_colsum_det", "pwa_dropout_colsum_det_workspace_size", "pwa_colsum_rows_det",
                          "pwa_colsum_rows_det_workspace_size", "pwa_bias_tables_bwd_det", "pwa_bias_tables_bwd_det_workspace_size")
 
+TILE_SYMBOLS = ("pwa_tile_gather", "pwa_tile_stitch", "pwa_tile_advance", "pwa_tile_finalize", "pwa_seg_counts")
+PWA_LABEL_U8, PWA_LABEL_I32, PWA_LABEL_I64 = 0, 1, 2
+PWA_TILE_MAX_SW = 1024
+
 lib = _load()
 
-EXPORTED_SYMBOLS = DETERMINISTIC_SYMBOLS + ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
+EXPORTED_SYMBOLS = DETERMINISTIC_SYMBOLS + TILE_SYMBOLS + ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
                     "pwa_partition", "pwa_reverse", "pwa_reverse_add", "pwa_gather_rows", "pwa_colsum_f32", "pwa_colsum_rows", "pwa_dropout", "pwa_dropout_colsum", "pwa_token_gemm_supported", "pwa_token_gemm_fwd", "pwa_token_gemm_fwd_dt", "pwa_attn_fwd", "pwa_attn_bwd", "pwa_attn_tc_supported", "pwa_attn_dense_fwd", "pwa_attn_dense_bwd",
                     "pwa_ln_fwd", "pwa_ln_bwd", "pwa_ln_bwd2", "pwa_bias_tables_fwd", "pwa_bias_tables_bwd")
 
