@@ -378,6 +378,39 @@ int pwa_tile_finalize(const float* acc, const float* wsum, int B, int K, const i
 int pwa_seg_counts(const void* labels, int label_dtype, const void* target, int target_dtype, int B, int64_t nvox, int K,
                    int64_t* tp, int64_t* fp, int64_t* fn, void* stream);
 
+/* ---- segmentation losses ----------------------------------------------------------------------------------------------- */
+
+/* The per-(sample, class) sums behind MONAI's DiceLoss / FocalLoss / DiceFocalLoss with integer label maps (pwa_b200.trainer
+ * builds the losses from them).  logits and dlogits: contiguous [B][K][nvox] (PWA_F32 / PWA_BF16 / PWA_F16); labels: [B][nvox]
+ * of type PWA_LABEL_*; one-hot y_k = [label == k], a label outside [0, K) is an all-zero row.  Per voxel:
+ *   p_k = x_k (PWA_ACT_NONE), sigmoid(x_k) (PWA_ACT_SIGMOID) or softmax over the K channels (PWA_ACT_SOFTMAX);
+ *   sums [4][B][K] fp32: I = sum p_k y_k, P = sum p_k (p_k^2 with squared_pred), G = sum y_k, F = sum focal_k;
+ *   focal_k, PWA_FOCAL_SIGMOID: (x - x y - log sigmoid(x)) exp(gamma log sigmoid(-x (2y - 1))), times (alpha y + (1 - alpha)(1 - y));
+ *   focal_k, PWA_FOCAL_SOFTMAX: -(1 - q_k)^gamma log(q_k) y_k, q = softmax over channels c0 .. K-1 (c0 = focal_skip_bg), 0 for
+ *     k < c0, times (1 - alpha) for k = 0 and alpha otherwise;  F = 0 with PWA_FOCAL_OFF.
+ *   alpha = NaN: no alpha factor.  focal_skip_bg needs PWA_FOCAL_SOFTMAX; alpha needs a focal form and focal_skip_bg = 0.
+ * pwa_segloss_bwd: dlogits = d(sum_{q,b,k} dsums[q][b][k] sums[q][b][k]) / dlogits (the G row has no gradient), computed in
+ * fp32 and rounded once to the logits' dtype.
+ * The forward's CTAs store their partial sums to their own slots of the DEVICE workspace (pwa_segloss_workspace_size bytes, a
+ * function of B, K and nvox; needs no GPU) and pwa_colsum_f32 sums the slots in index order: no float atomics, the sums are
+ * bitwise reproducible for a given GPU model, build and shape.  Arguments are checked before any CUDA call (PWA_ERR_ARG
+ * without a GPU); nothing allocates or synchronises, everything runs on `stream`. */
+#define PWA_SEGLOSS_MAX_K 32
+enum { PWA_ACT_NONE = 0, PWA_ACT_SIGMOID = 1, PWA_ACT_SOFTMAX = 2 };
+enum { PWA_FOCAL_OFF = 0, PWA_FOCAL_SIGMOID = 1, PWA_FOCAL_SOFTMAX = 2 };
+typedef struct pwa_segloss {
+  int32_t B, K;              /* 1 <= B <= 65535, 2 <= K <= PWA_SEGLOSS_MAX_K */
+  int64_t nvox;              /* voxels per sample and class, >= 1 */
+  int32_t act, squared_pred, focal, focal_skip_bg;
+  float gamma, alpha;        /* gamma >= 0; alpha NaN = none */
+} pwa_segloss;
+
+int64_t pwa_segloss_workspace_size(const pwa_segloss* s);
+int pwa_segloss_fwd(const void* logits, int dtype, const void* labels, int label_dtype, const pwa_segloss* s, float* sums,
+                    void* workspace, int64_t workspace_bytes, void* stream);
+int pwa_segloss_bwd(const void* logits, int dtype, const void* labels, int label_dtype, const pwa_segloss* s,
+                    const float* dsums, void* dlogits, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

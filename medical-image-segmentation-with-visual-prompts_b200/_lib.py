@@ -40,6 +40,13 @@ class PwaDenseAttn(C.Structure):                     # struct pwa_dense_attn
     ]
 
 
+class PwaSegLoss(C.Structure):                       # struct pwa_segloss
+    _fields_ = [
+        ("B", C.c_int32), ("K", C.c_int32), ("nvox", C.c_int64), ("act", C.c_int32), ("squared_pred", C.c_int32),
+        ("focal", C.c_int32), ("focal_skip_bg", C.c_int32), ("gamma", C.c_float), ("alpha", C.c_float),
+    ]
+
+
 class PwaError(RuntimeError):
     pass
 
@@ -121,6 +128,13 @@ def _load():
     lib.pwa_seg_counts.argtypes = [vp, i32, vp, i32, i32, i64, i32, vp, vp, vp, vp]
     for name in TILE_SYMBOLS:
         getattr(lib, name).restype = i32
+    # segmentation losses (pwa_b200.trainer.seg_losses)
+    slp = C.POINTER(PwaSegLoss)
+    lib.pwa_segloss_workspace_size.argtypes = [slp]
+    lib.pwa_segloss_workspace_size.restype = i64
+    lib.pwa_segloss_fwd.argtypes = [vp, i32, vp, i32, slp, f32p, vp, i64, vp]
+    lib.pwa_segloss_bwd.argtypes = [vp, i32, vp, i32, slp, f32p, vp, vp]
+    lib.pwa_segloss_fwd.restype = lib.pwa_segloss_bwd.restype = i32
     for name in ("pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_partition", "pwa_reverse",
                  "pwa_attn_tc_supported", "pwa_attn_fwd", "pwa_attn_bwd"):
         getattr(lib, name).restype = i32
@@ -134,10 +148,14 @@ DETERMINISTIC_SYMBOLS = ("pwa_attn_bwd_det", "pwa_attn_bwd_det_workspace_size", 
 TILE_SYMBOLS = ("pwa_tile_gather", "pwa_tile_stitch", "pwa_tile_advance", "pwa_tile_finalize", "pwa_seg_counts")
 PWA_LABEL_U8, PWA_LABEL_I32, PWA_LABEL_I64 = 0, 1, 2
 PWA_TILE_MAX_SW = 1024
+SEGLOSS_SYMBOLS = ("pwa_segloss_workspace_size", "pwa_segloss_fwd", "pwa_segloss_bwd")
+PWA_SEGLOSS_MAX_K = 32
+PWA_ACT_NONE, PWA_ACT_SIGMOID, PWA_ACT_SOFTMAX = 0, 1, 2
+PWA_FOCAL_OFF, PWA_FOCAL_SIGMOID, PWA_FOCAL_SOFTMAX = 0, 1, 2
 
 lib = _load()
 
-EXPORTED_SYMBOLS = DETERMINISTIC_SYMBOLS + TILE_SYMBOLS + ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
+EXPORTED_SYMBOLS = DETERMINISTIC_SYMBOLS + TILE_SYMBOLS + SEGLOSS_SYMBOLS + ("pwa_version", "pwa_last_error", "pwa_geometry", "pwa_region_ids", "pwa_index_map", "pwa_attn_sel_table",
                     "pwa_partition", "pwa_reverse", "pwa_reverse_add", "pwa_gather_rows", "pwa_colsum_f32", "pwa_colsum_rows", "pwa_dropout", "pwa_dropout_colsum", "pwa_token_gemm_supported", "pwa_token_gemm_fwd", "pwa_token_gemm_fwd_dt", "pwa_attn_fwd", "pwa_attn_bwd", "pwa_attn_tc_supported", "pwa_attn_dense_fwd", "pwa_attn_dense_bwd",
                     "pwa_ln_fwd", "pwa_ln_bwd", "pwa_ln_bwd2", "pwa_bias_tables_fwd", "pwa_bias_tables_bwd")
 
