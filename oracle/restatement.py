@@ -316,6 +316,50 @@ def elementwise_dropout_keep_factor(seed_words, n, p_drop):
     return torch.from_numpy((byte >= u(t)).astype(np.float64) * (256.0 / (256 - t)))
 
 
+def elementwise_dropout_keep_factor_torch(seed_words, n0, n, p_drop, device="cpu"):
+    """elementwise_dropout_keep_factor for the elements n0 .. n0+n-1 only, as torch int64 arithmetic on `device`:
+    float64 [n].  Same hash, same byte selection (tests/test_oracle_dropout_cpu.py compares the two); a whole-stage mask
+    (tens of millions of elements) is then a few device passes instead of a host loop."""
+    M = 0xFFFFFFFF
+
+    def mix(x):
+        x = x & M
+        x = x ^ (x >> 16); x = (x * 0x21f0aaad) & M
+        x = x ^ (x >> 15); x = (x * 0x735a2d97) & M
+        x = x ^ (x >> 15)
+        return x
+
+    t = _drop_threshold(p_drop)
+    s0, s1 = (int(w) & M for w in seed_words)
+    i = torch.arange(n, dtype=torch.int64, device=device) + int(n0)
+    q = i >> 2
+    h = mix(s0 + (((q & M) * 0x9E3779B1) & M) + (((q >> 32) * 0x85EBCA77) & M)) ^ s1
+    byte = (mix(h) >> (8 * (i & 3))) & 0xFF
+    return (byte >= t).to(torch.float64) * (256.0 / (256 - t))
+
+
+def block_keep_factors(seed_words, x_shape, ws, num_heads, num_prompt_tokens, attn_drop, proj_drop, device="cpu"):
+    """The two dropout masks one block of the B200 kernels applies, from the block's four seed words (what
+    SwinTransformerBlock draws per forward): words 0-1 seed the attention mask, float64 [B,P,h,N,N+I] over the
+    (sample * window) index b*P + p; words 2-3 seed the projection mask, float64 [B,P,N,C] over the block's window-token
+    tensor in row-major order (the element index of pwa_dropout and of the fused dropout + residual + LayerNorm GEMM).
+    x_shape: the block input [B,C,H,W,D].  A site with rate 0 gets None.  Returns (attn_keep, proj_keep) for
+    block_forward."""
+    B, C = x_shape[:2]
+    ws = tuple(ws)
+    sp = padded_dims(tuple(x_shape[2:]), pad_amounts(tuple(x_shape[2:]), ws))
+    P = math.prod(s // w for s, w in zip(sp, ws))
+    N = math.prod(ws)
+    w = [int(v) for v in seed_words]
+    attn = proj = None
+    if attn_drop > 0:
+        attn = dropout_keep_factor_torch(w[0:2], 0, B * P, num_heads, N, N + num_prompt_tokens, attn_drop, device)
+        attn = attn.reshape(B, P, num_heads, N, N + num_prompt_tokens)
+    if proj_drop > 0:
+        proj = elementwise_dropout_keep_factor_torch(w[2:4], 0, B * P * N * C, proj_drop, device).reshape(B, P, N, C)
+    return attn, proj
+
+
 def prompted_window_attention(q, k, v, kp, vp, bias, ids, scale, num_heads, drop=None):
     """q,k,v [B,P,N,C]; kp,vp [B,I,C] or None; bias [h,N,N+I]; ids int [P,N] or None.
     window_attention.py:45-59: logits = (q.k^T*scale + bias) * mask, softmax over keys, [dropout,] @ v.
@@ -382,10 +426,14 @@ def split_block_params(sd: Dict[str, torch.Tensor]):
 
 
 def block_forward(sd: Dict[str, torch.Tensor], x: torch.Tensor, p: Optional[torch.Tensor],
-                  ws, shift_cfg, num_heads: int, attn_drop: float = 0.0, proj_drop: float = 0.0) -> torch.Tensor:
+                  ws, shift_cfg, num_heads: int, attn_drop: float = 0.0, proj_drop: float = 0.0,
+                  attn_keep: Optional[torch.Tensor] = None, proj_keep: Optional[torch.Tensor] = None) -> torch.Tensor:
     """One SwinTransformerBlock.forward_attn_mlp (swin_block.py:145-255) from a state dict
     with the reference's key names.  attn_drop / proj_drop > 0: torch's own dropout on the attention probabilities and
-    on the projection output, as the reference applies it (window_attention.py:57,60) -- used by the CPU timing arm."""
+    on the projection output, as the reference applies it (window_attention.py:57,60) -- used by the CPU timing arm.
+    attn_keep [B,P,h,N,N+I] / proj_keep [B,P,N,C]: explicit keep factors (0 or 1/keep_rate, see block_keep_factors) that
+    take the place of the dropout at that site whatever its rate: attn_keep multiplies the attention probabilities,
+    proj_keep the projection output o @ Wproj^T + bproj before the residual add."""
     ws = tuple(ws)
     dims = tuple(x.shape[2:])
     C = x.shape[1]
@@ -410,13 +458,15 @@ def block_forward(sd: Dict[str, torch.Tensor], x: torch.Tensor, p: Optional[torc
         kp = lp @ sd["attn.to_k.weight"].t()
         vp = lp @ sd["attn.to_v.weight"].t()
     dh = C // num_heads
-    drop = None
-    if attn_drop > 0:
+    drop = attn_keep
+    if attn_drop > 0 and attn_keep is None:
         B_, P_, N_ = q.shape[:3]
         drop = F.dropout(torch.ones(B_, P_, num_heads, N_, N_ + I, dtype=q.dtype, device=q.device), attn_drop, True)
     o = prompted_window_attention(q, k, v, kp, vp, bias, ids, dh ** -0.5, num_heads, drop=drop)
     a = o @ sd["attn.proj.weight"].t() + sd["attn.proj.bias"]                  # :60
-    if proj_drop > 0:
+    if proj_keep is not None:
+        a = a * proj_keep.to(a.dtype)
+    elif proj_drop > 0:
         a = F.dropout(a, proj_drop, True)
     y = a + xw                                                                  # :222
     z = F.layer_norm(y, (C,), sd["mlp_norm.weight"], sd["mlp_norm.bias"], 1e-6)
@@ -448,14 +498,16 @@ def patch_merging_forward(sd: Dict[str, torch.Tensor], x: torch.Tensor, merge_la
 
 
 def pair_forward(sd: Dict[str, torch.Tensor], x, p_pair, ws, num_heads, down: bool, merge_last_dim: bool = True,
-                 attn_drop: float = 0.0, proj_drop: float = 0.0):
+                 attn_drop: float = 0.0, proj_drop: float = 0.0, keep=None):
     """ConsecutiveSwinBlocks.forward (swin_block.py:66-71): unshifted block, then block
-    shifted by ws//2, then optional PatchMerging."""
+    shifted by ws//2, then optional PatchMerging.  keep: None, or per block the (attn_keep, proj_keep) pair of
+    block_forward (block_keep_factors of that block's seed words)."""
     ws = tuple(ws)
     shift = tuple(w // 2 for w in ws)
     for i, sh in enumerate(((0, 0, 0), shift)):
         sub = {k[len(f"swin_blocks.{i}."):]: v for k, v in sd.items() if k.startswith(f"swin_blocks.{i}.")}
-        x = block_forward(sub, x, p_pair[i], ws, sh, num_heads, attn_drop, proj_drop)
+        ak, pk = (None, None) if keep is None else keep[i]
+        x = block_forward(sub, x, p_pair[i], ws, sh, num_heads, attn_drop, proj_drop, attn_keep=ak, proj_keep=pk)
     if down:
         sub = {k[len("merge."):]: v for k, v in sd.items() if k.startswith("merge.")}
         x = patch_merging_forward(sub, x, merge_last_dim)
